@@ -19,6 +19,10 @@ picture with N x the pixels, one ~1080p row strip per GPU).  ONE JSON line on ra
              over its ms at N is the strip-parallel speed-up), c3 = the reference's dungeon with atmosphere, c5 = Reference{depth:1}
              1024 spp sample-parallel + reduce, small = 640x480 (the size the reference's demo renders; launch-bound).
   strip_parity_ok  (N > 1) the gathered strip-parallel frame is bit-identical to a single-GPU render of the same frame on rank 0.
+
+--dump-outputs DIR writes the composed RGBA32F frame of the last timed step as DIR/output.npy (above 64 MB a fixed seeded sample of its
+pixels, with their indices in DIR/output_pixels.npy), so that two builds run with the same arguments (same scene, seeds and frame ids)
+can be compared output for output.
 """
 import argparse
 import json
@@ -49,7 +53,42 @@ def parse():
     p.add_argument("--no-cpu-baseline", action="store_true")
     p.add_argument("--no-extras", action="store_true", help="skip the c3 / c4 / c5 / small blocks")
     p.add_argument("--c5-spp", type=int, default=1024)
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", help="write the frame of the last timed step to DIR/*.npy")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    return args
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_frame(rows, y0, w, h, dist=None):
+    """--dump-outputs: the composed RGBA32F frame (h, w, 4) of the last timed step, assembled on rank 0 from every rank's `rows`
+    (its strip, starting at row y0).  Whole when it fits in DUMP_BYTES; otherwise the same seeded sample of pixels in every run:
+    "output" (n, 4) and "output_pixels", their row-major pixel indices (float64, exact)."""
+    import numpy as np
+    idx = None
+    part = rows
+    if h * w * 16 > DUMP_BYTES:
+        idx = np.sort(np.random.RandomState(0).choice(h * w, DUMP_BYTES // 32, replace=False))   # 16 B of colour + 8 B of index per pixel
+        lo, hi = y0 * w, (y0 + len(rows)) * w
+        part = rows.reshape(-1, 4)[idx[(idx >= lo) & (idx < hi)] - lo]
+    if dist:
+        parts = [None] * dist.get_world_size()
+        dist.all_gather_object(parts, part)
+        part = np.concatenate(parts)
+    out = {"output": part}
+    if idx is not None:
+        out["output_pixels"] = idx.astype(np.float64)
+    return out
+
+
+def write_dump(path, arrays):
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 class ClockSampler:
@@ -125,8 +164,8 @@ def workload_name(args):
     return f"{SCENE_LABEL[args.scene]} {w}x{h}, ReSTIR DI+GI + SVGF (Image{{denoise:true}}), static camera"
 
 
-def run_cpu(args, frames, warm=0):
-    """Times the CPU restatement (oracle/) on all host cores: `frames` full frames of the workload."""
+def run_cpu(args, frames, warm=0, dump=None):
+    """Times the CPU restatement (oracle/) on all host cores: `frames` full frames of the workload; `dump`: --dump-outputs DIR."""
     from oracle import pyoracle
     from strolle_b200 import scenes
     global CPU_THREADS
@@ -142,6 +181,8 @@ def run_cpu(args, frames, warm=0):
         e.tick(); e.render_camera(cam)
     dt = time.perf_counter() - t0
     rays = pyoracle.ray_count(reset=True)
+    if dump:
+        write_dump(dump, dump_frame(e.read_buffer(cam, "output").reshape(h, w, 4), 0, w, h))
     return frames / dt, dt, rays
 
 
@@ -152,7 +193,7 @@ def reference_arm(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    fps, dt, rays = run_cpu(args, args.steps, warm=args.warmup)
+    fps, dt, rays = run_cpu(args, args.steps, warm=args.warmup, dump=args.dump_outputs)
     mrays = rays / dt / 1e6
     w, h = frame_size(args)
     cores = CPU_THREADS
@@ -249,9 +290,10 @@ class Ctx:
             self.dist.destroy_process_group()
 
 
-def measure(ctx, scene, steps, warmup, detail=False, e2e=False, clocks=None):
+def measure(ctx, scene, steps, warmup, detail=False, e2e=False, clocks=None, dump=False):
     """One configuration: `warmup` untimed frames, then `steps` frames timed with CUDA events (max over ranks); optionally the
-    instrumented replay (per-pass events + ray counter over the same frame ids), the strict-arithmetic timing and the end-to-end region."""
+    instrumented replay (per-pass events + ray counter over the same frame ids), the strict-arithmetic timing and the end-to-end region.
+    `dump`: out["dump"] = dump_frame of the last timed frame (complete on rank 0)."""
     import numpy as np
     import strolle_b200
     from strolle_b200 import scenes
@@ -276,6 +318,8 @@ def measure(ctx, scene, steps, warmup, detail=False, e2e=False, clocks=None):
     dev_ms = eng.mark_end()
     ctx.barrier(eng)
     wall_ms = (time.perf_counter() - t0) * 1000.0
+    # read before the replay below renders over the last timed frame
+    dumped = dump_frame(eng.read_buffer(cam, "output").reshape(H, W, 4)[runner.y0:runner.y1], runner.y0, W, H, ctx.dist) if dump else None
     # the ray counter and per-pass events over a replay of exactly the same frame ids
     eng.enable_timing(True); eng.pass_times(reset=True); eng.wavelet_times(reset=True)
     eng.count_rays(True); eng.ray_count(reset=True)
@@ -297,7 +341,7 @@ def measure(ctx, scene, steps, warmup, detail=False, e2e=False, clocks=None):
     rays, total_launches = ctx.reduce([float(rays), float(launches.sum())], "sum")
     out = {"w": W, "h": H, "rows": runner.y1 - runner.y0, "ms_per_step": dev_ms / steps, "fps": 1000.0 * steps / dev_ms, "wall_ms_per_step": wall_ms / steps,
            "rays_per_frame": rays / steps, "mrays": rays / (dev_ms / 1000.0) / 1e6, "launches": int(total_launches), "pass_ms": pass_ms, "pass_launches": launches,
-           "wav_ms": wav_ms, "wav_launches": wav_launches, "halo_bytes": runner.halo_bytes_last_frame, "transport": runner.transport_name(), "per_rank": per_rank}
+           "wav_ms": wav_ms, "wav_launches": wav_launches, "halo_bytes": runner.halo_bytes_last_frame, "transport": runner.transport_name(), "per_rank": per_rank, "dump": dumped}
     if detail:   # every kernel strict IEEE, one launch per reference dispatch: the configuration that is bit-identical to the oracle
         for opt in (OPT_SVGF_FAST_MATH, OPT_SHADING_FAST_MATH, OPT_FUSED_PASSES):
             eng.set_option(opt, 0)
@@ -412,8 +456,10 @@ def main():
     rank, world = ctx.rank, ctx.world
     W, H = frame_size(args)
     clocks = ClockSampler(ctx.local)
-    main_m = measure(ctx, build_scene(args.scene, W, H), args.steps, args.warmup, detail=True, e2e=True, clocks=clocks)
+    main_m = measure(ctx, build_scene(args.scene, W, H), args.steps, args.warmup, detail=True, e2e=True, clocks=clocks, dump=bool(args.dump_outputs))
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        write_dump(args.dump_outputs, main_m.pop("dump"))
     eng = main_m["engine"]
     if world > 1:
         main_m["strip_parity_ok"], perr = strip_parity(ctx, build_scene(args.scene, W, H))
@@ -440,7 +486,7 @@ def main():
     # ---- the other BASELINE configurations at this N -----------------------------------------------------------------------------
     extras = {}
     if not args.no_extras:
-        k, wu = min(args.steps, 24), 6
+        k, wu = args.steps, 6
         m = measure(ctx, scenes.cornell(3840, 2160), k, wu)
         extras["c4"] = {"workload": f"Cornell 3840x2160 (fixed size, strong scaling), {world} row strip(s) of {m['rows']} rows", "ms_per_step": m["ms_per_step"], "fps": m["fps"],
                         "mrays_per_s": m["mrays"], "steps": k, "halo_bytes_per_frame_rank0": m["halo_bytes"]}
@@ -452,9 +498,9 @@ def main():
         m["engine"].close()
         extras["c5"] = c5_reference_mode(ctx, args.c5_spp)
         if world == 1:
-            m = measure(ctx, scenes.cornell(640, 480), 60, 12)
+            m = measure(ctx, scenes.cornell(640, 480), k, 12)
             extras["small"] = {"workload": "Cornell 640x480 (bevy-strolle/examples/demo.rs:24-25 viewport)", "ms_per_step": m["ms_per_step"], "wall_ms_per_step": m["wall_ms_per_step"],
-                               "fps": m["fps"], "launches_per_frame": m["launches"] / 60.0}
+                               "fps": m["fps"], "launches_per_frame": m["launches"] / k, "steps": k}
             m["engine"].close()
 
     if rank != 0:

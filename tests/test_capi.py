@@ -102,3 +102,63 @@ def test_bench_reference_arm_prints_the_contract_line():
     assert d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["cores"] >= 1 and d["cpu_baseline"]["value"] == d["value"]
     assert d["e2e"]["value"] == d["value"] and d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0
     assert d["value"] > 0 and "160x90" in d["config"]["workload"]
+
+
+def run_bench_dump(args, out_dir):
+    """Runs bench.py with --dump-outputs out_dir; returns its JSON line and the arrays it wrote."""
+    import json
+    import subprocess
+    import sys
+    import numpy as np
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + args + ["--dump-outputs", str(out_dir)],
+                       stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=600, cwd=ROOT)
+    assert p.returncode == 0, p.stderr[-3000:]
+    lines = [l for l in p.stdout.splitlines() if l.startswith("{")]
+    assert len(lines) == 1
+    return json.loads(lines[0]), {f[:-4]: np.load(os.path.join(out_dir, f)) for f in sorted(os.listdir(out_dir))}
+
+
+def test_bench_reference_arm_dumps_identical_outputs(tmp_path):
+    """`--dump-outputs DIR` writes the frame of the last timed step; the same arguments give the same inputs, so two runs write the same bits."""
+    import numpy as np
+    args = ["--impl", "reference", "--steps", "3", "--warmup", "1", "--width", "96", "--height", "54"]
+    d, a = run_bench_dump(args, tmp_path / "a")
+    _, b = run_bench_dump(args, tmp_path / "b")
+    assert d["steps"] == 3 and list(a) == ["output"] and list(b) == ["output"]
+    assert a["output"].shape == (54, 96, 4) and a["output"].dtype == np.float32
+    assert np.isfinite(a["output"]).all() and a["output"][..., :3].mean() > 0.01
+    assert (a["output"].view(np.uint32) == b["output"].view(np.uint32)).all()
+
+
+def test_bench_dump_samples_large_frames(monkeypatch):
+    """A frame larger than the dump budget is written as a fixed seeded sample of pixels with their indices; row strips (one per
+    rank, gathered in rank order) give the same sample as the whole frame."""
+    import numpy as np
+    import bench
+    monkeypatch.setattr(bench, "DUMP_BYTES", 32 * 500)
+    h, w = 40, 30
+    frame = np.random.RandomState(1).rand(h, w, 4).astype(np.float32)
+    whole = bench.dump_frame(frame, 0, w, h)
+    idx = whole["output_pixels"]
+    assert idx.dtype == np.float64 and len(idx) == 500 and (np.diff(idx) > 0).all()
+    assert (whole["output"] == frame.reshape(-1, 4)[idx.astype(np.int64)]).all()
+    strips = [bench.dump_frame(frame[y0:y1], y0, w, h) for y0, y1 in [(0, 7), (7, 25), (25, 40)]]
+    assert (np.concatenate([s["output"] for s in strips]) == whole["output"]).all()
+    assert all((s["output_pixels"] == idx).all() for s in strips)
+    monkeypatch.setattr(bench, "DUMP_BYTES", h * w * 16)
+    assert list(bench.dump_frame(frame, 0, w, h)) == ["output"]
+
+
+@pytest.mark.gpu
+def test_bench_cuda_arm_dumps_identical_outputs(tmp_path):
+    """The CUDA arm: the dumped frame is deterministic across runs with the same arguments and close to the strict CPU oracle's frame of
+    the same frame id (the product default shades with FMA / SFU approximations)."""
+    import numpy as np
+    args = ["--steps", "4", "--warmup", "3", "--width", "96", "--height", "54", "--no-extras", "--no-cpu-baseline"]
+    d, a = run_bench_dump(args, tmp_path / "a")
+    _, b = run_bench_dump(args, tmp_path / "b")
+    _, ref = run_bench_dump(["--impl", "reference"] + args[:8], tmp_path / "ref")
+    assert d["steps"] == 4 and a["output"].shape == (54, 96, 4)
+    assert (a["output"].view(np.uint32) == b["output"].view(np.uint32)).all()
+    x, y = a["output"][..., :3].astype(np.float64), ref["output"][..., :3].astype(np.float64)
+    assert np.sqrt(((x - y) ** 2).sum() / (y ** 2).sum()) <= 1e-2
