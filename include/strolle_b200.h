@@ -78,8 +78,11 @@ typedef struct st_camera {
 } st_camera;
 
 /* Output pixel formats for st_render_camera (the reference composes into the caller's
- * TextureView of CameraViewport::format, strolle/src/camera.rs:170-185). */
-enum { ST_FORMAT_RGBA32F = 0, ST_FORMAT_RGBA8_SRGB = 1 };
+ * TextureView of CameraViewport::format, strolle/src/camera.rs:170-185).  RGBA32F: 16 B/px, the composed
+ * frame as is.  RGBA8_SRGB: 4 B/px, Rgba8UnormSrgb (clamp, sRGB OETF, round to nearest), alpha 255.  RGBA16F:
+ * 8 B/px, IEEE binary16 per channel with round-to-nearest-even (what a render-target store to Rgba16Float does:
+ * above 65504 becomes inf, NaN stays NaN), alpha 1.0 (0x3C00); the format of Bevy's HDR view target. */
+enum { ST_FORMAT_RGBA32F = 0, ST_FORMAT_RGBA8_SRGB = 1, ST_FORMAT_RGBA16F = 2 };
 
 const char* st_last_error(void);
 
@@ -131,6 +134,17 @@ int st_render_camera(st_engine* e, st_camera_handle camera, void* host_out, int 
 /* Converts the camera's composed frame to `format` and copies it to host memory (what
  * st_render_camera does when host_out != NULL), without re-running the passes. */
 int st_copy_output(st_engine* e, st_camera_handle camera, void* host_out, int format);
+/* Engine::render_camera into a caller-owned surface (frame_composition.rs pass: scissor at viewport.position, LoadOp::Load,
+ * strolle/src/camera_controller/passes/frame_composition.rs:108-131).
+ * `dst` = address of the camera's pixel (0,0) inside the surface; `pitch_bytes` = bytes between rows (0 = width * bytes per pixel).
+ * dst may be device memory (this engine's device, or a device it can reach by peer access, or managed memory) or host memory
+ * (pinned or pageable); the kind is found with cudaPointerGetAttributes.  Only the width x height rectangle is written.
+ * Device memory: one kernel on the engine's stream stores straight into dst (no staging, no host round trip); the call returns
+ * once enqueued (order with st_synchronize or st_set_stream).  Host memory: as st_render_camera with host_out (blocking unless
+ * ST_OPT_ASYNC_OUTPUT).  ST_ERR_INVALID, before any pass runs and with nothing written, for a NULL dst, an unknown format, a
+ * nonzero pitch below width * bytes per pixel, a dst or pitch that is not a multiple of the bytes per pixel (16 / 8 / 4), or device
+ * memory this engine's device cannot reach. */
+int st_render_camera_to(st_engine* e, st_camera_handle camera, void* dst, size_t pitch_bytes, int format);
 int st_synchronize(st_engine* e);
 
 /* ---- hooks that the reference does not have (SURVEY §8b) -------------------------------- */
@@ -332,6 +346,10 @@ int st_multi_delete_camera(st_multi* m, st_camera_handle camera);
 int st_multi_tick(st_multi* m);
 /* host_out: the full frame (width*height pixels of `format`); every member fills its own rows.  NULL = enqueue only. */
 int st_multi_render_camera(st_multi* m, st_camera_handle camera, void* host_out, int format);
+/* st_render_camera_to for the group: every member stores its own rows [y0, y1) at dst + y0 * pitch_bytes, a kernel of its own for a
+ * device surface (a peer store when the surface lives on another member's device), a 2-D copy for a host surface.  A device surface
+ * on a device some member cannot reach is refused.  st_multi_render_camera is the tightly packed host case. */
+int st_multi_render_camera_to(st_multi* m, st_camera_handle camera, void* dst, size_t pitch_bytes, int format);
 int st_multi_synchronize(st_multi* m);
 int st_multi_set_option(st_multi* m, int option, int value);
 int st_multi_set_seed_base(st_multi* m, uint32_t base);

@@ -3,7 +3,9 @@
 //! Same shape as the reference plugin (`/bevy-strolle/src/lib.rs:29-84`, `stages.rs`, `rendering_node.rs`): the main world's meshes,
 //! materials, images, instances, lights, sun and cameras are mirrored into the engine once per frame (extract in `ExtractSchedule`, apply
 //! in `Render::Prepare`), and a render-graph node on the camera's view renders through the engine.  The CUDA engine composes into host
-//! memory, so the node ends with one `write_texture` into the view's main texture where the reference records compute passes.
+//! memory in the view's own format (`Rgba16Float`, the HDR main texture the reference requires), so the node ends with one
+//! `write_texture` into that texture at the viewport's position where the reference records compute passes; FXAA, tonemapping and
+//! upscaling follow as in the reference's graph.
 //!
 //! `STROLLE_B200_DEVICES=0,1,2,3` selects the GPUs (default `0`); several devices = row strips of every camera's frame.
 pub mod prelude {
@@ -12,6 +14,9 @@ pub mod prelude {
 
 mod sync;
 
+use bevy::core_pipeline::fxaa::FxaaNode;
+use bevy::core_pipeline::tonemapping::TonemappingNode;
+use bevy::core_pipeline::upscaling::UpscalingNode;
 use bevy::prelude::*;
 use bevy::render::render_graph::{NodeRunError, RenderGraphApp, RenderGraphContext, ViewNode, ViewNodeRunner};
 use bevy::render::renderer::{RenderContext, RenderQueue};
@@ -24,6 +29,8 @@ pub mod graph {
     pub const NAME: &str = "strolle";
     pub mod node {
         pub const RENDERING: &str = "strolle_rendering";
+        pub const TONEMAPPING: &str = "strolle_tonemapping";
+        pub const FXAA: &str = "strolle_fxaa";
         pub const UPSCALING: &str = "strolle_upscaling";
     }
 }
@@ -62,11 +69,14 @@ impl Plugin for StrollePlugin {
         let Ok(render_app) = app.get_sub_app_mut(RenderApp) else { return };
         render_app.insert_resource(sync::Synced::default());
         sync::setup(render_app);
+        // the reference's graph (`/bevy-strolle/src/graph.rs`): the HDR frame is anti-aliased and tonemapped by Bevy's own nodes
         render_app
             .add_render_sub_graph(graph::NAME)
             .add_render_graph_node::<ViewNodeRunner<RenderingNode>>(graph::NAME, graph::node::RENDERING)
-            .add_render_graph_node::<ViewNodeRunner<bevy::core_pipeline::upscaling::UpscalingNode>>(graph::NAME, graph::node::UPSCALING)
-            .add_render_graph_edges(graph::NAME, &[graph::node::RENDERING, graph::node::UPSCALING]);
+            .add_render_graph_node::<ViewNodeRunner<TonemappingNode>>(graph::NAME, graph::node::TONEMAPPING)
+            .add_render_graph_node::<ViewNodeRunner<UpscalingNode>>(graph::NAME, graph::node::UPSCALING)
+            .add_render_graph_node::<ViewNodeRunner<FxaaNode>>(graph::NAME, graph::node::FXAA)
+            .add_render_graph_edges(graph::NAME, &[graph::node::RENDERING, graph::node::FXAA, graph::node::TONEMAPPING, graph::node::UPSCALING]);
     }
 
     fn finish(&self, app: &mut App) {

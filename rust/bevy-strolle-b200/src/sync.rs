@@ -7,8 +7,8 @@ use std::sync::Mutex;
 use bevy::prelude::*;
 use bevy::render::camera::{CameraProjection, CameraRenderGraph, ExtractedCamera};
 use bevy::render::mesh::VertexAttributeValues;
-use bevy::render::render_resource::PrimitiveTopology;
-use bevy::render::view::RenderLayers;
+use bevy::render::render_resource::{PrimitiveTopology, TextureFormat};
+use bevy::render::view::{RenderLayers, ViewTarget};
 use bevy::render::{Extract, ExtractSchedule, Render, RenderSet};
 use bevy::utils::{HashMap, HashSet};
 
@@ -218,7 +218,16 @@ fn material_of(mat: &StandardMaterial) -> st::Material<EngineParams> {
     }
 }
 
-fn apply(mut engine: ResMut<EngineResource>, mut pending: ResMut<Pending>, mut synced: ResMut<Synced>, views: Query<(Entity, &ExtractedCamera)>) {
+/// The engine's format for a view's main texture: the reference composes into `view_target.main_texture_format()`
+/// (`/bevy-strolle/src/stages/prepare.rs:297`), which for the HDR cameras it requires is `Rgba16Float`.
+fn viewport_format(format: TextureFormat) -> Option<st::ViewportFormat> {
+    match format {
+        TextureFormat::Rgba16Float => Some(st::ViewportFormat::Rgba16Float),
+        _ => None,
+    }
+}
+
+fn apply(mut engine: ResMut<EngineResource>, mut pending: ResMut<Pending>, mut synced: ResMut<Synced>, views: Query<(Entity, &ExtractedCamera, &ViewTarget)>) {
     let engine = &mut engine.0;
     let p = std::mem::take(&mut *pending);
     for id in p.meshes_removed.iter().copied().chain(p.meshes.iter().map(|(id, _)| *id)) {
@@ -259,10 +268,14 @@ fn apply(mut engine: ResMut<EngineResource>, mut pending: ResMut<Pending>, mut s
     // cameras: create / update the ones seen this frame, delete the rest (`/bevy-strolle/src/stages/prepare.rs:283-347`)
     let mut alive = HashSet::new();
     for cam in p.cameras {
-        let Some((_, view)) = views.iter().find(|(e, _)| *e == cam.entity) else { continue };
+        let Some((_, view, target)) = views.iter().find(|(e, _, _)| *e == cam.entity) else { continue };
         let Some(size) = view.physical_viewport_size else { continue };
+        let Some(format) = viewport_format(target.main_texture_format()) else {
+            error!("strolle: the view's main texture is {:?}; Strolle requires an HDR camera (Rgba16Float)", target.main_texture_format());
+            continue;
+        };
         let position = view.viewport.as_ref().map(|v| v.physical_position).unwrap_or_default();
-        let viewport = st::CameraViewport { format: st::ViewportFormat::Rgba32Float, size, position };
+        let viewport = st::CameraViewport { format, size, position };
         let camera = st::Camera { mode: cam.mode.unwrap_or_default(), viewport: viewport.clone(), transform: cam.transform, projection: cam.projection };
         alive.insert(cam.entity);
         match synced.cameras.get_mut(&cam.entity) {

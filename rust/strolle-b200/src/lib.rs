@@ -8,7 +8,8 @@
 //!   into row strips across them (`st_multi_*`).  `create_camera` / `update_camera` / `tick` lose their `device` / `queue` arguments.
 //! * `render_camera` delivers the composed frame into a [`Frame`] (host pixels in the viewport's format) instead of recording into a
 //!   wgpu command encoder — the CUDA kernels run on the engine's own stream.  A wgpu host uploads it with `Queue::write_texture`
-//!   (what `bevy-strolle-b200` does), or reads the device pointer through `strolle_b200_sys::st_buffer_device_ptr` and interop.
+//!   (what `bevy-strolle-b200` does); `render_camera_to_raw` composes straight into a caller-owned surface in device or host memory
+//!   with a row pitch (e.g. a texture imported through CUDA external memory).
 //! * `ImageData::Texture` (a live wgpu texture) cannot be sampled from CUDA; dynamic images are passed as `ImageData::Raw` each time
 //!   they change.
 //! * Misuse returns `Err(Error)` where the reference panics (`triangles.rs:44-53`, `camera_controllers.rs:21-25`); the infallible
@@ -18,7 +19,7 @@ use std::ffi::CStr;
 use std::fmt::{self, Debug};
 use std::hash::Hash;
 use std::marker::PhantomData;
-use std::os::raw::c_int;
+use std::os::raw::{c_int, c_void};
 
 pub use glam;
 use glam::{Affine3A, Mat4, UVec2, Vec2, Vec3, Vec4};
@@ -259,10 +260,12 @@ impl Default for CameraMode {
     }
 }
 
-/// The two formats the engine composes into (`CameraViewport::format`, `camera.rs:170-185`)
+/// The formats the engine composes into (`CameraViewport::format`, `camera.rs:170-185`).  `Rgba16Float` is the format of an HDR
+/// Bevy view target (`ViewTarget::TEXTURE_FORMAT_HDR`), which is what the reference's Bevy plugin renders into.
 #[derive(Clone, Copy, Debug, PartialEq, Eq)]
 pub enum ViewportFormat {
     Rgba8UnormSrgb,
+    Rgba16Float,
     Rgba32Float,
 }
 
@@ -270,12 +273,14 @@ impl ViewportFormat {
     pub fn bytes_per_pixel(self) -> usize {
         match self {
             Self::Rgba8UnormSrgb => 4,
+            Self::Rgba16Float => 8,
             Self::Rgba32Float => 16,
         }
     }
     fn to_ffi(self) -> c_int {
         match self {
             Self::Rgba8UnormSrgb => sys::ST_FORMAT_RGBA8_SRGB,
+            Self::Rgba16Float => sys::ST_FORMAT_RGBA16F,
             Self::Rgba32Float => sys::ST_FORMAT_RGBA32F,
         }
     }
@@ -558,6 +563,21 @@ impl<P: Params> Engine<P> {
             return Err(Error { code: sys::ST_ERR_INVALID, message: "target frame does not match the camera's viewport".into() });
         }
         check(unsafe { sys::st_multi_render_camera(self.raw, handle.0, target.pixels.as_mut_ptr().cast(), target.format.to_ffi()) })
+    }
+
+    /// Renders camera (`lib.rs:279-286`) into a caller-owned surface, as the reference's composition pass does into the view's
+    /// texture at `viewport.position` (`LoadOp::Load`: only the viewport's `size.x * size.y` texels are written).
+    ///
+    /// `dst` is the address of the viewport's first texel inside the surface (the caller adds `position.y * pitch_bytes +
+    /// position.x * format.bytes_per_pixel()`), `pitch_bytes` the distance between rows (0 = tightly packed).  The surface may be
+    /// device memory (a device of the group or one it reaches by peer access, e.g. a Vulkan image imported as CUDA external memory)
+    /// or host memory; device surfaces are written by the engine's kernels and the call returns once they are enqueued.
+    ///
+    /// # Safety
+    /// `dst` must point to a surface of at least `(size.y - 1) * pitch_bytes + size.x * format.bytes_per_pixel()` bytes that stays
+    /// valid, and is not otherwise accessed, until the engine's work is done.
+    pub unsafe fn render_camera_to_raw(&self, handle: CameraHandle, dst: *mut c_void, pitch_bytes: usize, format: ViewportFormat) -> Result<(), Error> {
+        check(sys::st_multi_render_camera_to(self.raw, handle.0, dst, pitch_bytes, format.to_ffi()))
     }
 
     /// Enqueues the camera's passes without reading the frame back (e.g. `CameraMode::Reference` accumulation frames).

@@ -366,6 +366,12 @@ static uint32_t dispatch_seed(uint32_t base, uint32_t frame, uint32_t k) {
     return (w >> 22) ^ w;
 }
 
+static_assert(OUT_RGBA32F == ST_FORMAT_RGBA32F && OUT_RGBA8_SRGB == ST_FORMAT_RGBA8_SRGB && OUT_RGBA16F == ST_FORMAT_RGBA16F, "kernel output formats follow the C ABI");
+// bytes per pixel of an output format; 0 = not a format
+static size_t format_bpp(int format) { return format == ST_FORMAT_RGBA32F ? 16 : format == ST_FORMAT_RGBA16F ? 8 : format == ST_FORMAT_RGBA8_SRGB ? 4 : 0; }
+// the widest format that is converted through the staging buffer (RGBA32F leaves straight from `output`)
+static const size_t kStagingBpp = 8;
+
 struct CameraSlot {
     bool alive = false;
     st_camera desc;
@@ -375,16 +381,18 @@ struct CameraSlot {
     std::vector<std::pair<std::string, size_t>> sizes;      // float4 count per named buffer
     DevMem arena;
     DevMem svgf_pairs; float4* pair[2] = {nullptr, nullptr};   // interleaved {DI, GI} records of the wide-stride à-trous iterations (ST_OPT_WAVELET_PAIRED); private scratch, never exchanged
-    DevMem rgba8; int rgba8_slot = 0;
-    // asynchronous RGBA8 read-back: slot k of the staging buffer is converted on the engine stream (ev_ready[k]) and copied to
+    // converted frames on their way to host memory or to rank 0 of a strip gather: two frame-sized slots of kStagingBpp bytes per pixel,
+    // allocated at that size from the start because the buffer is exported to the other ranks (a later growth would leave their mappings stale)
+    DevMem staging; int staging_slot = 0;
+    // asynchronous read-back: slot k of the staging buffer is converted on the engine stream (ev_ready[k]) and copied to
     // the host on the copy stream (ev_copied[k]); the engine stream only waits for ev_copied[k] before reusing slot k
     cudaEvent_t ev_ready[2] = {nullptr, nullptr}, ev_copied[2] = {nullptr, nullptr};
-    // peer-memory link of the strip partition: other ranks' arena / flag / rgba8 allocations mapped through CUDA IPC
+    // peer-memory link of the strip partition: other ranks' arena / flag / staging allocations mapped through CUDA IPC
     // sync words: [0, 128) fused-transport flags (slot * 16 + source rank), 128.. legacy k_peer_exchange flags, 144 its block counter,
     // 145 its time-outs, 200/201 need_rows {min, max}, 202 fused-transport wait time-outs, 204 (u64) rows pulled
     // copy-engine pushes of the large GI halos (ST_OPT_STRIP_DMA): one side stream per neighbour (0 = up, 1 = down), `pushed` = the last push issued there
     cudaStream_t side[2] = {nullptr, nullptr}; cudaEvent_t ev_produced = nullptr, ev_pushed[2] = {nullptr, nullptr}; bool pushed_pending[2] = {false, false};
-    struct PeerLink { bool ready = false; bool ipc = false; std::vector<char*> arena, rgba8; std::vector<uint32_t*> flags; DevMem sync; uint32_t seq = 0, fseq = 0; } peer;
+    struct PeerLink { bool ready = false; bool ipc = false; std::vector<char*> arena, staging; std::vector<uint32_t*> flags; DevMem sync; uint32_t seq = 0, fseq = 0; } peer;
 };
 
 struct Step { int pass; std::function<void(cudaStream_t)> run; int sub = -1; };   // sub: à-trous iteration of a K22 step
@@ -1150,7 +1158,7 @@ void st_engine_destroy(st_engine* e) {
     cudaStreamSynchronize(e->stream);
     if (e->copy_stream) cudaStreamSynchronize(e->copy_stream);
     for (CameraSlot* c : e->cameras) { for (int k = 0; k < 2; k++) { if (c->side[k]) { cudaStreamSynchronize(c->side[k]); cudaStreamDestroy(c->side[k]); } if (c->ev_pushed[k]) cudaEventDestroy(c->ev_pushed[k]); } if (c->ev_produced) cudaEventDestroy(c->ev_produced);
-        c->arena.release(); c->svgf_pairs.release(); c->rgba8.release(); for (int k = 0; k < 2; k++) { if (c->ev_ready[k]) cudaEventDestroy(c->ev_ready[k]); if (c->ev_copied[k]) cudaEventDestroy(c->ev_copied[k]); } delete c; }
+        c->arena.release(); c->svgf_pairs.release(); c->staging.release(); for (int k = 0; k < 2; k++) { if (c->ev_ready[k]) cudaEventDestroy(c->ev_ready[k]); if (c->ev_copied[k]) cudaEventDestroy(c->ev_copied[k]); } delete c; }
     DevMem* all[] = {&e->d_triangles, &e->d_bvh, &e->d_materials, &e->d_lights, &e->d_noise, &e->d_tlut, &e->d_slut, &e->d_skylut, &e->d_scratch, &e->d_raycount, &e->d_matpacked, &e->d_unpacklut, &e->d_atlas, &e->d_srgb, &e->d_tri_instance, &e->d_instance_xforms, &e->d_tile_errors};
     for (DevMem* d : all) d->release();
     for (auto& t : e->pending) { cudaEventDestroy(t.a); cudaEventDestroy(t.b); }
@@ -1324,7 +1332,7 @@ int st_delete_camera(st_engine* e, st_camera_handle h) {
     CK(cudaStreamSynchronize(e->stream));
     if (e->copy_stream) CK(cudaStreamSynchronize(e->copy_stream));
     for (int k = 0; k < 2; k++) if (cs->side[k]) CK(cudaStreamSynchronize(cs->side[k]));
-    cs->alive = false; cs->arena.release(); cs->svgf_pairs.release(); cs->pair[0] = cs->pair[1] = nullptr; cs->rgba8.release();
+    cs->alive = false; cs->arena.release(); cs->svgf_pairs.release(); cs->pair[0] = cs->pair[1] = nullptr; cs->staging.release();
     return ST_OK;
 }
 int st_camera_set_strip(st_engine* e, st_camera_handle h, int y0, int y1) {
@@ -1447,37 +1455,91 @@ int st_render_camera(st_engine* e, st_camera_handle h, void* host_out, int forma
     if (host_out) return st_copy_output(e, h, host_out, format);
     return ST_OK;
 }
-// Converts rows [y0, y1) of the composed frame to `format` and copies them to the same rows of `host_out` (a full-frame buffer).
-static int copy_rows_out(st_engine* e, CameraSlot* cs, void* host_out, int format, int y0, int y1) {
-    const size_t W = cs->desc.width, n = W * cs->desc.height;
-    const size_t first = (size_t)y0 * W, count = (size_t)(y1 - y0) * W;
-    if (format == ST_FORMAT_RGBA32F) CK(cudaMemcpyAsync((char*)host_out + first * 16, cs->dev.output + first, count * 16, cudaMemcpyDeviceToHost, e->stream));
-    else if (format == ST_FORMAT_RGBA8_SRGB) {
-        int rc2 = cs->rgba8.ensure(2 * n * 4); if (rc2) return rc2;
-        cs->rgba8_slot ^= 1;
-        SceneDev sc = e->scene(); uchar4* dst8 = (uchar4*)cs->rgba8.p + (cs->rgba8_slot ? n : 0); CameraDev cd = cs->dev; cd.y0 = y0; cd.y1 = y1;
-        const int k = cs->rgba8_slot;
-        if (e->async_output) {   // conversion on the engine stream, copy on the copy stream: the next frame's passes do not queue behind the copy
-            if (!e->copy_stream) CK(cudaStreamCreateWithFlags(&e->copy_stream, cudaStreamNonBlocking));
-            if (!cs->ev_ready[k]) { CK(cudaEventCreateWithFlags(&cs->ev_ready[k], cudaEventDisableTiming)); CK(cudaEventCreateWithFlags(&cs->ev_copied[k], cudaEventDisableTiming)); }
-            else CK(cudaStreamWaitEvent(e->stream, cs->ev_copied[k], 0));   // slot k's previous copy must have left the staging buffer
-        }
-        e->run_timed(P_COMPOSITION, [=](cudaStream_t s) { launch_output_rgba8(cd, sc, dst8, s); });
-        if (e->async_output) {
-            CK(cudaEventRecord(cs->ev_ready[k], e->stream));
-            CK(cudaStreamWaitEvent(e->copy_stream, cs->ev_ready[k], 0));
-            CK(cudaMemcpyAsync((char*)host_out + first * 4, dst8 + first, count * 4, cudaMemcpyDeviceToHost, e->copy_stream));
-            CK(cudaEventRecord(cs->ev_copied[k], e->copy_stream));
-        } else CK(cudaMemcpyAsync((char*)host_out + first * 4, dst8 + first, count * 4, cudaMemcpyDeviceToHost, e->stream));
-    } else return fail(ST_ERR_INVALID, "unsupported output format");
+// Where a frame goes: `dst` = the address of camera pixel (0, 0) inside the caller's surface, rows `pitch` bytes apart.  `device`:
+// memory a kernel on the engine's device stores into (device memory of that device or of a peer, managed memory); otherwise host memory.
+struct OutputTarget { char* dst; size_t pitch; int format; bool device; };
+// The full-frame host buffer of st_render_camera / st_copy_output: tightly packed rows.
+static OutputTarget host_frame(const CameraSlot* cs, void* host_out, int format) { return {(char*)host_out, (size_t)cs->desc.width * format_bpp(format), format, false}; }
+// Checks a caller's surface for a `width`-pixel frame and finds what memory it is (cudaPointerGetAttributes).  Device memory of another
+// device is made reachable with peer access when the two devices allow it (as st_link_local does); otherwise the surface is refused.
+static int resolve_target(st_engine* e, uint32_t width, void* dst, size_t pitch, int format, OutputTarget* t) {
+    const size_t bpp = format_bpp(format);
+    if (!dst) return fail(ST_ERR_INVALID, "null surface");
+    if (!bpp) return fail(ST_ERR_INVALID, "unsupported output format");
+    if (pitch == 0) pitch = (size_t)width * bpp;
+    if (pitch < (size_t)width * bpp) return fail(ST_ERR_INVALID, "row pitch " + std::to_string(pitch) + " is smaller than a row of the frame (" + std::to_string((size_t)width * bpp) + " bytes)");
+    if ((uintptr_t)dst % bpp || pitch % bpp) return fail(ST_ERR_INVALID, "surface address and row pitch must be multiples of the format's " + std::to_string(bpp) + " bytes per pixel");
+    cudaPointerAttributes a{};
+    if (cudaPointerGetAttributes(&a, dst) != cudaSuccess) { cudaGetLastError(); a.type = cudaMemoryTypeUnregistered; }
+    *t = {(char*)dst, pitch, format, a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged};
+    if (a.type == cudaMemoryTypeDevice && a.device != e->device) {
+        int can = 0; CK(cudaDeviceCanAccessPeer(&can, e->device, a.device));
+        if (!can) return fail(ST_ERR_INVALID, "the surface is memory of device " + std::to_string(a.device) + ", which device " + std::to_string(e->device) + " cannot reach");
+        CK(cudaSetDevice(e->device));
+        cudaError_t ce = cudaDeviceEnablePeerAccess(a.device, 0);
+        if (ce != cudaSuccess && ce != cudaErrorPeerAccessAlreadyEnabled) return fail(ST_ERR_CUDA, std::string("cudaDeviceEnablePeerAccess: ") + cudaGetErrorString(ce));
+        cudaGetLastError();
+    }
     return ST_OK;
+}
+// rows of `row_bytes` bytes from device to host memory; one linear copy when both sides are tightly packed
+static int copy_rows_to_host(char* dst, size_t dpitch, const char* src, size_t spitch, size_t row_bytes, size_t rows, cudaStream_t s) {
+    if (dpitch == row_bytes && spitch == row_bytes) CK(cudaMemcpyAsync(dst, src, rows * row_bytes, cudaMemcpyDeviceToHost, s));
+    else CK(cudaMemcpy2DAsync(dst, dpitch, src, spitch, row_bytes, rows, cudaMemcpyDeviceToHost, s));
+    return ST_OK;
+}
+// The one place a frame leaves the engine: rows [y0, y1) of the composed frame, in t.format, land at t.dst + y * t.pitch and nothing
+// else of the surface is written.  A device target is stored by the store kernel directly; a host target receives one copy, from
+// `output` itself (RGBA32F) or from a staging slot the store kernel filled tightly packed.
+static int copy_rows_out(st_engine* e, CameraSlot* cs, const OutputTarget& t, int y0, int y1) {
+    const size_t W = cs->desc.width, n = W * cs->desc.height, bpp = format_bpp(t.format);
+    if (!bpp) return fail(ST_ERR_INVALID, "unsupported output format");
+    const size_t rows = (size_t)(y1 - y0), row_bytes = W * bpp;
+    SceneDev sc = e->scene(); CameraDev cd = cs->dev; cd.y0 = y0; cd.y1 = y1;
+    const int format = t.format;
+    if (t.device) {
+        char* dst = t.dst; const size_t pitch = t.pitch;
+        e->run_timed(P_COMPOSITION, [=](cudaStream_t s) { launch_output_store(cd, sc, format, dst, pitch, s); });
+        CK(cudaGetLastError());
+        return ST_OK;
+    }
+    char* host = t.dst + (size_t)y0 * t.pitch;
+    if (format == ST_FORMAT_RGBA32F) return copy_rows_to_host(host, t.pitch, (const char*)(cs->dev.output + (size_t)y0 * W), row_bytes, row_bytes, rows, e->stream);
+    int rc = cs->staging.ensure(2 * n * kStagingBpp); if (rc) return rc;
+    cs->staging_slot ^= 1;
+    const int k = cs->staging_slot;
+    char* slot = (char*)cs->staging.p + (k ? n * kStagingBpp : 0);
+    if (e->async_output) {   // conversion on the engine stream, copy on the copy stream: the next frame's passes do not queue behind the copy
+        if (!e->copy_stream) CK(cudaStreamCreateWithFlags(&e->copy_stream, cudaStreamNonBlocking));
+        if (!cs->ev_ready[k]) { CK(cudaEventCreateWithFlags(&cs->ev_ready[k], cudaEventDisableTiming)); CK(cudaEventCreateWithFlags(&cs->ev_copied[k], cudaEventDisableTiming)); }
+        else CK(cudaStreamWaitEvent(e->stream, cs->ev_copied[k], 0));   // slot k's previous copy must have left the staging buffer
+    }
+    e->run_timed(P_COMPOSITION, [=](cudaStream_t s) { launch_output_store(cd, sc, format, slot, row_bytes, s); });
+    if (e->async_output) {
+        CK(cudaEventRecord(cs->ev_ready[k], e->stream));
+        CK(cudaStreamWaitEvent(e->copy_stream, cs->ev_ready[k], 0));
+        if ((rc = copy_rows_to_host(host, t.pitch, slot + (size_t)y0 * row_bytes, row_bytes, row_bytes, rows, e->copy_stream))) return rc;
+        CK(cudaEventRecord(cs->ev_copied[k], e->copy_stream));
+        return ST_OK;
+    }
+    return copy_rows_to_host(host, t.pitch, slot + (size_t)y0 * row_bytes, row_bytes, row_bytes, rows, e->stream);
 }
 int st_copy_output(st_engine* e, st_camera_handle h, void* host_out, int format) {
     CameraSlot* cs = e ? get_camera(e, h) : nullptr;
     if (!cs || !host_out) return fail(ST_ERR_NOT_FOUND, "unknown camera");
     CK(cudaSetDevice(e->device));
-    int rc = copy_rows_out(e, cs, host_out, format, 0, (int)cs->desc.height); if (rc) return rc;
+    int rc = copy_rows_out(e, cs, host_frame(cs, host_out, format), 0, (int)cs->desc.height); if (rc) return rc;
     if (!e->async_output) CK(cudaStreamSynchronize(e->stream));
+    return ST_OK;
+}
+int st_render_camera_to(st_engine* e, st_camera_handle h, void* dst, size_t pitch, int format) {
+    CameraSlot* cs = e ? get_camera(e, h) : nullptr;
+    if (!cs) return fail(ST_ERR_NOT_FOUND, "unknown camera");
+    CK(cudaSetDevice(e->device));
+    OutputTarget t; int rc = resolve_target(e, cs->desc.width, dst, pitch, format, &t); if (rc) return rc;   // before any pass runs: a refused call changes nothing
+    if ((rc = st_render_range(e, h, 0, -1))) return rc;
+    if ((rc = copy_rows_out(e, cs, t, 0, (int)cs->desc.height))) return rc;
+    if (!t.device && !e->async_output) CK(cudaStreamSynchronize(e->stream));
     return ST_OK;
 }
 int st_synchronize(st_engine* e) {
@@ -1698,12 +1760,12 @@ int st_peer_export(st_engine* e, st_camera_handle h, uint8_t* out192) {
     if (!cs || !out192) return fail(ST_ERR_NOT_FOUND, "unknown camera");
     CK(cudaSetDevice(e->device));
     size_t n = (size_t)cs->desc.width * cs->desc.height;
-    int rc = cs->rgba8.ensure(2 * n * 4); if (rc) return rc;
+    int rc = cs->staging.ensure(2 * n * kStagingBpp); if (rc) return rc;
     if ((rc = cs->peer.sync.ensure(kSyncBytes))) return rc;
     { const int need0[2] = {(int)cs->desc.height, -1}; CK(cudaMemcpy((uint32_t*)cs->peer.sync.p + kNeedRowsWord, need0, 8, cudaMemcpyHostToDevice)); }
     static_assert(sizeof(cudaIpcMemHandle_t) == 64, "ipc handle size");
     cudaIpcMemHandle_t hs[3];
-    CK(cudaIpcGetMemHandle(&hs[0], cs->arena.p)); CK(cudaIpcGetMemHandle(&hs[1], cs->peer.sync.p)); CK(cudaIpcGetMemHandle(&hs[2], cs->rgba8.p));
+    CK(cudaIpcGetMemHandle(&hs[0], cs->arena.p)); CK(cudaIpcGetMemHandle(&hs[1], cs->peer.sync.p)); CK(cudaIpcGetMemHandle(&hs[2], cs->staging.p));
     std::memcpy(out192, hs, ST_PEER_HANDLE_BYTES);
     return ST_OK;
 }
@@ -1737,16 +1799,16 @@ int st_peer_import(st_engine* e, st_camera_handle h, const uint8_t* all, int ran
     CameraSlot* cs = e ? get_camera(e, h) : nullptr;
     if (!cs || !all) return fail(ST_ERR_NOT_FOUND, "unknown camera");
     if (world < 1 || world > ST_PEER_MAX_RANKS || rank < 0 || rank >= world) return fail(ST_ERR_LIMIT, "peer transport supports up to 16 ranks");
-    if (!cs->peer.sync.p || !cs->rgba8.p) return fail(ST_ERR_INVALID, "st_peer_export first");
+    if (!cs->peer.sync.p || !cs->staging.p) return fail(ST_ERR_INVALID, "st_peer_export first");
     CK(cudaSetDevice(e->device));
-    cs->peer.arena.assign(world, nullptr); cs->peer.rgba8.assign(world, nullptr); cs->peer.flags.assign(world, nullptr);
+    cs->peer.arena.assign(world, nullptr); cs->peer.staging.assign(world, nullptr); cs->peer.flags.assign(world, nullptr);
     for (int r = 0; r < world; r++) {
-        if (r == rank) { cs->peer.arena[r] = (char*)cs->arena.p; cs->peer.flags[r] = (uint32_t*)cs->peer.sync.p; cs->peer.rgba8[r] = (char*)cs->rgba8.p; continue; }
+        if (r == rank) { cs->peer.arena[r] = (char*)cs->arena.p; cs->peer.flags[r] = (uint32_t*)cs->peer.sync.p; cs->peer.staging[r] = (char*)cs->staging.p; continue; }
         cudaIpcMemHandle_t hs[3]; std::memcpy(hs, all + (size_t)r * ST_PEER_HANDLE_BYTES, ST_PEER_HANDLE_BYTES);
         void* p = nullptr;
         CK(cudaIpcOpenMemHandle(&p, hs[0], cudaIpcMemLazyEnablePeerAccess)); cs->peer.arena[r] = (char*)p;
         CK(cudaIpcOpenMemHandle(&p, hs[1], cudaIpcMemLazyEnablePeerAccess)); cs->peer.flags[r] = (uint32_t*)p;
-        CK(cudaIpcOpenMemHandle(&p, hs[2], cudaIpcMemLazyEnablePeerAccess)); cs->peer.rgba8[r] = (char*)p;
+        CK(cudaIpcOpenMemHandle(&p, hs[2], cudaIpcMemLazyEnablePeerAccess)); cs->peer.staging[r] = (char*)p;
     }
     e->rank = rank; e->n_ranks = world; cs->peer.seq = 0; cs->peer.fseq = 0; cs->peer.ready = true; cs->peer.ipc = true;
     return strip_streams_prepare(e, cs);
@@ -1858,27 +1920,29 @@ int st_render_strips(st_engine* e, st_camera_handle h, void* host_out, int forma
     std::vector<std::pair<int, int>> bounds; strip_bounds((int)cs->desc.height, e->n_ranks, &bounds);
     if (gather == 2) {
         if (!host_out) return fail(ST_ERR_INVALID, "gather 2 needs the shared host frame");
-        if ((rc = copy_rows_out(e, cs, host_out, format, bounds[e->rank].first, bounds[e->rank].second))) return rc;
+        if ((rc = copy_rows_out(e, cs, host_frame(cs, host_out, format), bounds[e->rank].first, bounds[e->rank].second))) return rc;
         if (!e->async_output) CK(cudaStreamSynchronize(e->stream));
         return ST_OK;
     }
     // assemble the composed frame on rank 0 (strips travel in the requested output format)
-    const size_t W = cs->desc.width, n = W * cs->desc.height;
-    char* base; size_t px_bytes; ncclDataType_t dt; size_t per_px;
-    if (format == ST_FORMAT_RGBA32F) { base = (char*)cs->dev.output; px_bytes = 16; dt = ncclFloat; per_px = 4; }
-    else if (format == ST_FORMAT_RGBA8_SRGB) {
-        if ((rc = cs->rgba8.ensure(2 * n * 4))) return rc;
-        cs->rgba8_slot ^= 1;
-        SceneDev sc = e->scene(); uchar4* dst8 = (uchar4*)cs->rgba8.p + (cs->rgba8_slot ? n : 0); CameraDev cd = cs->dev;
-        e->run_timed(P_COMPOSITION, [=](cudaStream_t s) { launch_output_rgba8(cd, sc, dst8, s); });
-        base = (char*)dst8; px_bytes = 4; dt = ncclUint8; per_px = 4;
-    } else return fail(ST_ERR_INVALID, "unsupported output format");
+    // RGBA32F strips travel straight from `output` as floats, the converted formats from a staging slot as bytes
+    const size_t W = cs->desc.width, n = W * cs->desc.height, px_bytes = format_bpp(format);
+    if (!px_bytes) return fail(ST_ERR_INVALID, "unsupported output format");
+    char* base; ncclDataType_t dt; size_t per_px;
+    if (format == ST_FORMAT_RGBA32F) { base = (char*)cs->dev.output; dt = ncclFloat; per_px = 4; }
+    else {
+        if ((rc = cs->staging.ensure(2 * n * kStagingBpp))) return rc;
+        cs->staging_slot ^= 1;
+        SceneDev sc = e->scene(); char* slot = (char*)cs->staging.p + (cs->staging_slot ? n * kStagingBpp : 0); CameraDev cd = cs->dev;
+        e->run_timed(P_COMPOSITION, [=](cudaStream_t s) { launch_output_store(cd, sc, format, slot, W * px_bytes, s); });
+        base = slot; dt = ncclUint8; per_px = px_bytes;
+    }
     if (peer) {
         PeerExchange x; peer_fill(e, cs, &x);
         if (e->rank != 0) {
             size_t first = (size_t)bounds[e->rank].first * W * px_bytes, bytes = (size_t)(bounds[e->rank].second - bounds[e->rank].first) * W * px_bytes;
-            if (first % 16 || bytes % 16) return fail(ST_ERR_INVALID, "RGBA8 strip gather needs strips that start and end on 16-byte boundaries");
-            char* remote = format == ST_FORMAT_RGBA32F ? cs->peer.arena[0] + (size_t)(base - (char*)cs->arena.p) : cs->peer.rgba8[0] + (size_t)(base - (char*)cs->rgba8.p);
+            if (first % 16 || bytes % 16) return fail(ST_ERR_INVALID, "the strip gather needs strips that start and end on 16-byte boundaries");
+            char* remote = format == ST_FORMAT_RGBA32F ? cs->peer.arena[0] + (size_t)(base - (char*)cs->arena.p) : cs->peer.staging[0] + (size_t)(base - (char*)cs->staging.p);
             x.seg[x.nseg++] = {(const uint4*)(base + first), (uint4*)(remote + first), bytes / 16};
         }
         peer_flush(e, cs, &x, true);
@@ -1904,7 +1968,7 @@ int st_render_strips(st_engine* e, st_camera_handle h, void* host_out, int forma
 static int link_prepare(st_engine* e, CameraSlot* cs) {
     CK(cudaSetDevice(e->device));
     size_t n = (size_t)cs->desc.width * cs->desc.height;
-    int rc = cs->rgba8.ensure(2 * n * 4); if (rc) return rc;
+    int rc = cs->staging.ensure(2 * n * kStagingBpp); if (rc) return rc;
     if ((rc = cs->peer.sync.ensure(kSyncBytes))) return rc;
     const int need0[2] = {(int)cs->desc.height, -1};
     CK(cudaMemcpy((uint32_t*)cs->peer.sync.p + kNeedRowsWord, need0, 8, cudaMemcpyHostToDevice));
@@ -1930,8 +1994,8 @@ int st_link_local(st_engine* const* engines, const st_camera_handle* cameras, in
     }
     for (int r = 0; r < n; r++) {
         CameraSlot* cs = cams[r];
-        cs->peer.arena.assign(n, nullptr); cs->peer.rgba8.assign(n, nullptr); cs->peer.flags.assign(n, nullptr);
-        for (int q = 0; q < n; q++) { cs->peer.arena[q] = (char*)cams[q]->arena.p; cs->peer.flags[q] = (uint32_t*)cams[q]->peer.sync.p; cs->peer.rgba8[q] = (char*)cams[q]->rgba8.p; }
+        cs->peer.arena.assign(n, nullptr); cs->peer.staging.assign(n, nullptr); cs->peer.flags.assign(n, nullptr);
+        for (int q = 0; q < n; q++) { cs->peer.arena[q] = (char*)cams[q]->arena.p; cs->peer.flags[q] = (uint32_t*)cams[q]->peer.sync.p; cs->peer.staging[q] = (char*)cams[q]->staging.p; }
         engines[r]->rank = r; engines[r]->n_ranks = n; cs->peer.seq = 0; cs->peer.fseq = 0; cs->peer.ready = true; cs->peer.ipc = false;
     }
     for (int r = 0; r < n; r++) { int rc = strip_streams_prepare(engines[r], cams[r]); if (rc) return rc; }
@@ -2038,12 +2102,11 @@ int st_multi_delete_camera(st_multi* m, st_camera_handle h) {
     return ST_OK;
 }
 st_camera_handle st_multi_member_camera(st_multi* m, st_camera_handle h, int rank) { return (m && h >= 0 && (size_t)h < m->cams.size() && rank >= 0 && (size_t)rank < m->e.size()) ? m->cams[h][rank] : -1; }
-// Engine::render_camera for the group.  All ranks' frames are enqueued before any output copy is issued and nothing in between
-// synchronises: the ranks wait for each other on the device (sequence flags), never on the host.
-int st_multi_render_camera(st_multi* m, st_camera_handle h, void* host_out, int format) {
-    if (!m || h < 0 || (size_t)h >= m->cams.size()) return fail(ST_ERR_NOT_FOUND, "unknown camera");
+// Engine::render_camera for the group.  All ranks' frames are enqueued before any output is issued and nothing in between
+// synchronises: the ranks wait for each other on the device (sequence flags), never on the host.  Then every rank stores its own rows
+// [y0, y1) into its target (targets[rank]: the same surface, reached from that rank's device); targets == nullptr = enqueue only.
+static int multi_render(st_multi* m, st_camera_handle h, const OutputTarget* targets) {
     const size_t n = m->e.size();
-    if (n == 1) return st_render_camera(m->e[0], m->cams[h][0], host_out, format);
     std::vector<CameraSlot*> cs(n);
     for (size_t i = 0; i < n; i++) {   // first-use allocations and LUT generation synchronise their device: do them before anything can wait on a peer
         cs[i] = get_camera(m->e[i], m->cams[h][i]);
@@ -2052,11 +2115,34 @@ int st_multi_render_camera(st_multi* m, st_camera_handle h, void* host_out, int 
         int rc = ensure_luts(m->e[i]); if (rc) return rc;
     }
     for (size_t i = 0; i < n; i++) { CK(cudaSetDevice(m->e[i]->device)); int rc = enqueue_strip_frame(m->e[i], cs[i], 16); if (rc) return rc; }
-    if (!host_out) return ST_OK;
+    if (!targets) return ST_OK;
     std::vector<std::pair<int, int>> bounds; strip_bounds((int)cs[0]->desc.height, (int)n, &bounds);
-    for (size_t i = 0; i < n; i++) { CK(cudaSetDevice(m->e[i]->device)); int rc = copy_rows_out(m->e[i], cs[i], host_out, format, bounds[i].first, bounds[i].second); if (rc) return rc; }
-    for (size_t i = 0; i < n; i++) if (!m->e[i]->async_output) { CK(cudaSetDevice(m->e[i]->device)); CK(cudaStreamSynchronize(m->e[i]->stream)); }
+    for (size_t i = 0; i < n; i++) { CK(cudaSetDevice(m->e[i]->device)); int rc = copy_rows_out(m->e[i], cs[i], targets[i], bounds[i].first, bounds[i].second); if (rc) return rc; }
+    for (size_t i = 0; i < n; i++) if (!targets[i].device && !m->e[i]->async_output) { CK(cudaSetDevice(m->e[i]->device)); CK(cudaStreamSynchronize(m->e[i]->stream)); }
     return ST_OK;
+}
+int st_multi_render_camera(st_multi* m, st_camera_handle h, void* host_out, int format) {
+    if (!m || h < 0 || (size_t)h >= m->cams.size()) return fail(ST_ERR_NOT_FOUND, "unknown camera");
+    if (m->e.size() == 1) return st_render_camera(m->e[0], m->cams[h][0], host_out, format);
+    std::vector<OutputTarget> t;
+    for (size_t i = 0; host_out && i < m->e.size(); i++) {
+        CameraSlot* cs = get_camera(m->e[i], m->cams[h][i]);
+        if (!cs) return fail(ST_ERR_NOT_FOUND, "unknown camera");
+        t.push_back(host_frame(cs, host_out, format));
+    }
+    return multi_render(m, h, host_out ? t.data() : nullptr);
+}
+int st_multi_render_camera_to(st_multi* m, st_camera_handle h, void* dst, size_t pitch, int format) {
+    if (!m || h < 0 || (size_t)h >= m->cams.size()) return fail(ST_ERR_NOT_FOUND, "unknown camera");
+    if (m->e.size() == 1) return st_render_camera_to(m->e[0], m->cams[h][0], dst, pitch, format);
+    std::vector<OutputTarget> t(m->e.size());
+    for (size_t i = 0; i < m->e.size(); i++) {   // every member must reach the surface before any of them renders
+        CameraSlot* cs = get_camera(m->e[i], m->cams[h][i]);
+        if (!cs) return fail(ST_ERR_NOT_FOUND, "unknown camera");
+        CK(cudaSetDevice(m->e[i]->device));
+        int rc = resolve_target(m->e[i], cs->desc.width, dst, pitch, format, &t[i]); if (rc) return rc;
+    }
+    return multi_render(m, h, t.data());
 }
 // per-camera buffer of the whole frame, assembled from the members' strips (test hook, cf. st_read_buffer)
 int st_multi_read_buffer(st_multi* m, st_camera_handle h, const char* name, float* dst, size_t cap, size_t* count) {

@@ -1225,22 +1225,32 @@ __global__ void __launch_bounds__(ST_BLOCK) k_composition(KPARAMS, int cur, u32 
 }
 
 
-// Rgba8UnormSrgb store of the composed frame (the reference's default CameraViewport::format,
+// One channel of an Rgba8UnormSrgb render-target store (the reference's default CameraViewport::format,
 // strolle/src/camera.rs:177-185): clamp to [0,1], sRGB OETF, round to nearest.
-__global__ void __launch_bounds__(ST_BLOCK) k_output_rgba8(KPARAMS, uchar4* __restrict__ out) {
+ST_DEV u32 srgb8_encode(float v) {
+    float x = sat(v);
+    float e = (x <= 0.0031308f) ? 12.92f * x : 1.055f * pow_det(x, 1.0f / 2.4f) - 0.055f;
+    return to_u32_sat(sat(e) * 255.0f + 0.5f);
+}
+
+// Store of rows [y0, y1) of the composed frame into a surface of format FMT (CameraViewport::format): pixel (x, y) goes to
+// dst + y * pitch + x * bytes per pixel, one aligned store per pixel; nothing else of the surface is touched (LoadOp::Load).
+// RGBA32F copies `output`; RGBA16F converts each channel with round-to-nearest-even (what a store to an Rgba16Float target does),
+// alpha 1.0; RGBA8 is the sRGB encode above.
+template <int FMT>
+__global__ void __launch_bounds__(ST_BLOCK) k_output_store(KPARAMS, char* __restrict__ dst, size_t pitch) {
     Px p = pixel_full(cam);
     if (!p.in) return;
-    size_t i = pix(cam, p.x, p.y);
-    float4 c = cam.output[i];
-    float v[3] = {c.x, c.y, c.z};
-    u32 q[3];
-#pragma unroll
-    for (int k = 0; k < 3; k++) {
-        float x = sat(v[k]);
-        float e = (x <= 0.0031308f) ? 12.92f * x : 1.055f * pow_det(x, 1.0f / 2.4f) - 0.055f;
-        q[k] = to_u32_sat(sat(e) * 255.0f + 0.5f);
+    float4 c = cam.output[pix(cam, p.x, p.y)];
+    char* row = dst + (size_t)p.y * pitch;
+    if (FMT == OUT_RGBA32F) {
+        reinterpret_cast<float4*>(row)[p.x] = c;
+    } else if (FMT == OUT_RGBA16F) {
+        const u32 r = __half_as_ushort(__float2half_rn(c.x)), g = __half_as_ushort(__float2half_rn(c.y)), b = __half_as_ushort(__float2half_rn(c.z));
+        reinterpret_cast<uint2*>(row)[p.x] = make_uint2(r | (g << 16), b | (0x3C00u << 16));
+    } else {
+        reinterpret_cast<uchar4*>(row)[p.x] = make_uchar4((unsigned char)srgb8_encode(c.x), (unsigned char)srgb8_encode(c.y), (unsigned char)srgb8_encode(c.z), 255);
     }
-    out[i] = make_uchar4((unsigned char)q[0], (unsigned char)q[1], (unsigned char)q[2], 255);
 }
 
 // K1 ref_tracing::main (ref_tracing.rs:4-60)
@@ -1761,7 +1771,11 @@ bool launch_denoise_variance_tiled(const CameraDev& c, const SceneDev& s, int cu
     return fast ? variance_tiled_go<true>(c, s, cur, errors, st) : variance_tiled_go<false>(c, s, cur, errors, st);
 }
 void launch_composition(const CameraDev& c, const SceneDev& s, int cur, u32 mode, const float4* di_diff, const float4* gi_diff, cudaStream_t st) { k_composition<<<grid_full(c), ST_BLOCK, 0, st>>>(c, s, cur, mode, di_diff, gi_diff); }
-void launch_output_rgba8(const CameraDev& c, const SceneDev& s, uchar4* out, cudaStream_t st) { k_output_rgba8<<<grid_full(c), ST_BLOCK, 0, st>>>(c, s, out); }
+void launch_output_store(const CameraDev& c, const SceneDev& s, int format, void* dst, size_t pitch, cudaStream_t st) {
+    if (format == OUT_RGBA32F) k_output_store<OUT_RGBA32F><<<grid_full(c), ST_BLOCK, 0, st>>>(c, s, (char*)dst, pitch);
+    else if (format == OUT_RGBA16F) k_output_store<OUT_RGBA16F><<<grid_full(c), ST_BLOCK, 0, st>>>(c, s, (char*)dst, pitch);
+    else k_output_store<OUT_RGBA8_SRGB><<<grid_full(c), ST_BLOCK, 0, st>>>(c, s, (char*)dst, pitch);
+}
 void launch_ref_tracing(const CameraDev& c, const SceneDev& s, u32 depth, cudaStream_t st) { k_ref_tracing<<<grid_full(c), ST_BLOCK, 0, st>>>(c, s, depth); }
 void launch_ref_shading(const CameraDev& c, const SceneDev& s, u32 seed, u32 depth, cudaStream_t st) { k_ref_shading<<<grid_full(c), ST_BLOCK, 0, st>>>(c, s, seed, depth); }
 void launch_bvh_heatmap(const CameraDev& c, const SceneDev& s, cudaStream_t st) { k_bvh_heatmap<<<grid_full(c), ST_BLOCK, 0, st>>>(c, s); }

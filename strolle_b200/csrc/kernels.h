@@ -34,7 +34,10 @@ void launch_denoise_wavelet(const CameraDev& c, const SceneDev& s, int cur, u32 
 bool launch_denoise_wavelet_tiled(const CameraDev& c, const SceneDev& s, u32 frame, u32 stride, float strength, const float4* di_in, float4* di_out, const float4* gi_in, float4* gi_out, float4* pair_out, bool fast, int cfg, u32* errors, cudaStream_t st);
 bool launch_denoise_variance_tiled(const CameraDev& c, const SceneDev& s, int cur, bool fast, u32* errors, cudaStream_t st);
 void launch_composition(const CameraDev& c, const SceneDev& s, int cur, u32 mode, const float4* di_diff, const float4* gi_diff, cudaStream_t st);
-void launch_output_rgba8(const CameraDev& c, const SceneDev& s, uchar4* out, cudaStream_t st);
+// output pixel formats of launch_output_store, numbered like ST_FORMAT_* (include/strolle_b200.h)
+enum OutputFormat { OUT_RGBA32F = 0, OUT_RGBA8_SRGB = 1, OUT_RGBA16F = 2 };
+// rows [c.y0, c.y1) of c.output stored at dst + y * pitch (pitch and dst aligned to the format's bytes per pixel)
+void launch_output_store(const CameraDev& c, const SceneDev& s, int format, void* dst, size_t pitch, cudaStream_t st);
 void launch_ref_tracing(const CameraDev& c, const SceneDev& s, u32 depth, cudaStream_t st);
 void launch_ref_shading(const CameraDev& c, const SceneDev& s, u32 seed, u32 depth, cudaStream_t st);
 void launch_bvh_heatmap(const CameraDev& c, const SceneDev& s, cudaStream_t st);

@@ -11,7 +11,7 @@ import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 PASS_COUNT = 27
-FORMAT_RGBA32F, FORMAT_RGBA8_SRGB = 0, 1
+FORMAT_RGBA32F, FORMAT_RGBA8_SRGB, FORMAT_RGBA16F = 0, 1, 2
 OPT_SVGF_FAST_MATH = 1
 OPT_ASYNC_OUTPUT = 2
 OPT_HALO_NCCL = 3
@@ -89,6 +89,7 @@ def load_library():
         "st_insert_light": [P, u64, C.POINTER(_Light)], "st_remove_light": [P, u64], "st_update_sun": [P, C.c_float, C.c_float],
         "st_create_camera": [P, C.POINTER(_Camera), C.POINTER(i32)], "st_update_camera": [P, i32, C.POINTER(_Camera)], "st_delete_camera": [P, i32],
         "st_tick": [P], "st_render_camera": [P, i32, P, C.c_int], "st_copy_output": [P, i32, P, C.c_int], "st_synchronize": [P],
+        "st_render_camera_to": [P, i32, P, C.c_size_t, C.c_int], "st_multi_render_camera_to": [P, i32, P, C.c_size_t, C.c_int],
         "st_set_seed_base": [P, u32], "st_set_blue_noise": [P, C.c_void_p],
         "st_read_buffer": [P, i32, C.c_char_p, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)],
         "st_read_scene": [P, C.c_char_p, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)],
@@ -212,6 +213,49 @@ class BvhBuilder:
             pass
 
 
+_FORMAT_DTYPES = {FORMAT_RGBA32F: "float32", FORMAT_RGBA8_SRGB: "uint8", FORMAT_RGBA16F: "float16"}
+
+
+class _Surface:
+    """A caller's output surface: a numpy array or a torch tensor (CPU, pinned or not, or CUDA) of shape (h, w, 4) whose dtype matches
+    the format, last two dimensions contiguous, any row stride.  `ptr` = address of pixel (0, 0), `pitch` = bytes between rows."""
+
+    def __init__(self, out, fmt, size):
+        if hasattr(out, "data_ptr"):   # torch.Tensor
+            dtype, itemsize = str(out.dtype).replace("torch.", ""), out.element_size()
+            self.ptr, self.cuda = out.data_ptr(), out.is_cuda
+            shape, strides = tuple(out.shape), tuple(st * itemsize for st in out.stride())
+            self.device = out.device if out.is_cuda else None
+        else:
+            out = out if isinstance(out, np.ndarray) else np.asarray(out)
+            dtype, itemsize = out.dtype.name, out.itemsize
+            self.ptr, self.cuda, self.device = out.ctypes.data, False, None
+            shape, strides = out.shape, out.strides
+        want = _FORMAT_DTYPES.get(fmt)
+        if want is not None and dtype != want:
+            raise ValueError(f"output format {fmt} needs a {want} surface, got {dtype}")
+        if size is not None and shape != (size[1], size[0], 4):
+            raise ValueError(f"output surface must have shape (h, w, 4) = {(size[1], size[0], 4)}, got {shape}")
+        if len(shape) != 3 or shape[2] != 4 or strides[2] != itemsize or strides[1] != 4 * itemsize:
+            raise ValueError(f"output surface must have contiguous pixels and channels (strides (*, {4 * itemsize}, {itemsize}) bytes), got strides {strides}")
+        if strides[0] < 0:
+            raise ValueError(f"output surface rows must run forward in memory, got a row stride of {strides[0]} bytes")
+        self.pitch = strides[0]
+        self.packed = strides[0] == shape[1] * 4 * itemsize
+
+    def render(self, fn_packed, fn_to, synchronize):
+        """Host surfaces without row padding go through the packed entry point; everything else through the *_to one.  A CUDA surface
+        is ordered after the torch work queued on it before the engine writes, and holds the frame when this returns."""
+        if not self.cuda and self.packed:
+            return fn_packed(self.ptr)
+        if self.cuda:
+            import torch
+            torch.cuda.current_stream(self.device).synchronize()
+        fn_to(self.ptr, self.pitch)
+        if self.cuda:
+            synchronize()
+
+
 class Engine:
     """strolle::Engine on one B200 (CUDA device `device`)."""
 
@@ -313,9 +357,20 @@ class Engine:
         self._check(self.lib.st_tick(self._h))
 
     def render_camera(self, cam, out=None, fmt=FORMAT_RGBA32F):
-        """Runs the frame's passes.  With `out` (host ndarray) the composed frame is copied back."""
-        ptr = out.ctypes.data if out is not None else None
-        self._check(self.lib.st_render_camera(self._h, cam, ptr, fmt))
+        """Runs the frame's passes.  With `out` the composed frame is stored there in format `fmt`: a numpy array or torch tensor of shape
+        (h, w, 4) and dtype float32 / uint8 / float16 (FORMAT_RGBA32F / FORMAT_RGBA8_SRGB / FORMAT_RGBA16F), in host memory or on a CUDA
+        device, with any row stride; `out=big[y:y + h, x:x + w]` composes into a viewport of a larger surface and leaves the rest of it
+        untouched.  A CUDA `out` holds the frame when this returns."""
+        if out is None:
+            self._check(self.lib.st_render_camera(self._h, cam, None, fmt))
+            return
+        _Surface(out, fmt, self._cams.get(cam)).render(lambda p: self._check(self.lib.st_render_camera(self._h, cam, p, fmt)),
+                                                       lambda p, pitch: self._check(self.lib.st_render_camera_to(self._h, cam, p, pitch, fmt)),
+                                                       self.synchronize)
+
+    def render_camera_to(self, cam, ptr, pitch_bytes, fmt):
+        """st_render_camera_to on a raw address (pixel (0, 0) of the camera inside the surface); returns once enqueued for device memory."""
+        self._check(self.lib.st_render_camera_to(self._h, cam, ptr, pitch_bytes, fmt))
 
     def copy_output(self, cam, out, fmt=FORMAT_RGBA32F):
         self._check(self.lib.st_copy_output(self._h, cam, out.ctypes.data, fmt))
@@ -475,6 +530,7 @@ class MultiEngine:
         self._check(self.lib.st_multi_create(arr, len(devices), C.byref(h)))
         self._h = h
         self.n = len(devices)
+        self._cams = {}
         if blue_noise is None:
             from . import scenes
             blue_noise = scenes.blue_noise()
@@ -550,18 +606,28 @@ class MultiEngine:
         c = Engine._cam(mode, denoise, ref_depth, w, h, transform16, projection16)
         out = C.c_int32()
         self._check(self.lib.st_multi_create_camera(self._h, C.byref(c), C.byref(out)))
+        self._cams[out.value] = (w, h)
         return out.value
 
     def update_camera(self, cam, mode, denoise, ref_depth, w, h, transform16, projection16):
         c = Engine._cam(mode, denoise, ref_depth, w, h, transform16, projection16)
         self._check(self.lib.st_multi_update_camera(self._h, cam, C.byref(c)))
+        self._cams[cam] = (w, h)
 
     def tick(self):
         self._check(self.lib.st_multi_tick(self._h))
 
     def render_camera(self, cam, out=None, fmt=FORMAT_RGBA32F):
-        ptr = out.ctypes.data if out is not None else None
-        self._check(self.lib.st_multi_render_camera(self._h, cam, ptr, fmt))
+        """As `Engine.render_camera`; every member stores its own rows of the frame into `out`."""
+        if out is None:
+            self._check(self.lib.st_multi_render_camera(self._h, cam, None, fmt))
+            return
+        _Surface(out, fmt, self._cams.get(cam)).render(lambda p: self._check(self.lib.st_multi_render_camera(self._h, cam, p, fmt)),
+                                                       lambda p, pitch: self._check(self.lib.st_multi_render_camera_to(self._h, cam, p, pitch, fmt)),
+                                                       self.synchronize)
+
+    def render_camera_to(self, cam, ptr, pitch_bytes, fmt):
+        self._check(self.lib.st_multi_render_camera_to(self._h, cam, ptr, pitch_bytes, fmt))
 
     def synchronize(self):
         self._check(self.lib.st_multi_synchronize(self._h))
