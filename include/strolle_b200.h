@@ -147,6 +147,18 @@ int st_copy_output(st_engine* e, st_camera_handle camera, void* host_out, int fo
 int st_render_camera_to(st_engine* e, st_camera_handle camera, void* dst, size_t pitch_bytes, int format);
 int st_synchronize(st_engine* e);
 
+/* ---- several cameras per frame (no reference counterpart: the reference renders one camera per call) ---- */
+/* Renders `n` cameras of this engine for the current frame.  The result is, camera for camera, what st_render_camera_to(e, cameras[i],
+ * dsts[i], pitch_bytes[i], format) gives when called for i = 0..n-1 in order: bit-identical buffers and output bytes.  Cameras with the
+ * same width, height, mode, denoise and ref_depth run as ONE launch per pass (the view index is blockIdx.z); groups run in the order of
+ * their first camera in the list, a group larger than one launch holds runs as several launches per pass.  dsts == NULL, or
+ * dsts[i] == NULL: no output for that camera (enqueue only, as st_render_camera with NULL).  pitch_bytes may be NULL (all packed).
+ * Device surfaces only enqueue (one store launch per group); host surfaces get one copy each and the call blocks unless
+ * ST_OPT_ASYNC_OUTPUT.  Everything is checked before any pass runs; on a refusal nothing is rendered or written: ST_ERR_NOT_FOUND for an
+ * unknown or deleted camera, ST_ERR_INVALID for n <= 0, a camera listed twice, a camera restricted to a row strip
+ * (st_camera_set_strip) or linked into a strip group, a surface st_render_camera_to refuses, or a call before the first st_tick. */
+int st_render_cameras(st_engine* e, const st_camera_handle* cameras, int n, void* const* dsts, const size_t* pitch_bytes, int format);
+
 /* ---- hooks that the reference does not have (SURVEY §8b) -------------------------------- */
 /* Explicit per-dispatch seeds: seed(frame f, dispatch k) = pcg(base ^ (f*64 + k)); the reference
  * draws rand::thread_rng() per dispatch (camera_controller.rs:189-194) and is not reproducible. */

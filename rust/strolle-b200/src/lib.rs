@@ -580,6 +580,31 @@ impl<P: Params> Engine<P> {
         check(sys::st_multi_render_camera_to(self.raw, handle.0, dst, pitch_bytes, format.to_ffi()))
     }
 
+    /// Renders several cameras for this frame, each as [`Self::render_camera_to_raw`] with `dsts[i]` and `pitches[i]` would, bit for
+    /// bit; cameras of one size and mode run as one launch per pass.  A null `dsts[i]` renders camera `i` without output; empty
+    /// `dsts` / `pitches` mean no outputs / packed rows.  Only a group of one device renders batches (the cameras of a strip group are
+    /// split across devices): with several devices this returns `ST_ERR_INVALID`.
+    ///
+    /// # Safety
+    /// Every non-null `dsts[i]` must satisfy the requirements of [`Self::render_camera_to_raw`] for camera `handles[i]`.
+    pub unsafe fn render_cameras_to_raw(&self, handles: &[CameraHandle], dsts: &[*mut c_void], pitches: &[usize], format: ViewportFormat) -> Result<(), Error> {
+        if (!dsts.is_empty() && dsts.len() != handles.len()) || (!pitches.is_empty() && pitches.len() != handles.len()) {
+            return Err(Error { code: sys::ST_ERR_INVALID, message: "one surface and one pitch per camera".into() });
+        }
+        if sys::st_multi_size(self.raw) != 1 {
+            return Err(Error { code: sys::ST_ERR_INVALID, message: "batched rendering needs a group of one device".into() });
+        }
+        let members: Vec<sys::st_camera_handle> = handles.iter().map(|h| sys::st_multi_member_camera(self.raw, h.0, 0)).collect();
+        check(sys::st_render_cameras(
+            sys::st_multi_engine(self.raw, 0),
+            members.as_ptr(),
+            members.len() as c_int,
+            if dsts.is_empty() { std::ptr::null() } else { dsts.as_ptr() },
+            if pitches.is_empty() { std::ptr::null() } else { pitches.as_ptr() },
+            format.to_ffi(),
+        ))
+    }
+
     /// Enqueues the camera's passes without reading the frame back (e.g. `CameraMode::Reference` accumulation frames).
     pub fn render_camera_offscreen(&self, handle: CameraHandle) -> Result<(), Error> {
         check(unsafe { sys::st_multi_render_camera(self.raw, handle.0, std::ptr::null_mut(), sys::ST_FORMAT_RGBA32F) })

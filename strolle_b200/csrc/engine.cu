@@ -12,6 +12,7 @@
 #include <deque>
 #include <functional>
 #include <limits>
+#include <memory>
 #include <string>
 #include <unordered_map>
 #include <vector>
@@ -656,10 +657,23 @@ static int allocate_camera(st_engine* e, CameraSlot* cs) {
 // those buffers has to travel.  All zero = every pass runs on [y0, y1).
 struct StripExt { int gbuffer = 0, variance = 0, wavelet[5] = {0, 0, 0, 0, 0}; int preview_mirror[2] = {0, 0}; bool still = false; /* nothing moved: no rows of last frame are pulled */ };
 static CameraDev grown(const CameraDev& c, int rows) { CameraDev g = c; g.y0 = std::max(0, c.y0 - rows); g.y1 = std::min(c.h, c.y1 + rows); return g; }
-static void build_schedule(st_engine* e, CameraSlot* cs, std::vector<Step>* steps, const StripExt* ext = nullptr) {
+// camera `c` as a view of a launch whose view 0 is `first` (same size: the arenas have the same layout), rows grown by `rows`
+static ViewDev view_of(const CameraSlot* c, const CameraSlot* first, int rows) {
+    ViewDev v; v.cam = grown(c->dev, rows);
+    v.arena_delta = (const char*)c->arena.p - (const char*)first->arena.p; v.pair_delta = (const char*)c->svgf_pairs.p - (const char*)first->svgf_pairs.p;
+    v.dst = nullptr; v.pitch = 0;
+    return v;
+}
+typedef std::shared_ptr<const ViewSet> Views;
+// `group`: one camera, or up to kBatchViews cameras of one size, mode, denoise and ref_depth rendered after the same tick (they share the
+// frame id, hence every pass, seed and buffer parity), each pass one launch over all of them.  Pointer arguments are group[0]'s.
+static void build_schedule(st_engine* e, const std::vector<CameraSlot*>& group, std::vector<Step>* steps, const StripExt* ext = nullptr) {
+    CameraSlot* cs = group[0];
     const CameraDev cam = cs->dev;   // snapshot (pointers + cameras)
     const StripExt no_ext; const StripExt& x = ext ? *ext : no_ext;
-    const CameraDev camG = grown(cam, x.gbuffer), camV = grown(cam, x.variance);
+    auto views = [&](int rows) { auto v = std::make_shared<ViewSet>(); for (CameraSlot* c : group) v->push_back(view_of(c, cs, rows)); return Views(v); };
+    const Views V = views(0), VG = views(x.gbuffer), VV = views(x.variance);
+    const bool one = group.size() == 1;   // the tile-staged K21 / K22 encode one camera's planes; several views run the gather kernels (same bits)
     const int pm0 = x.preview_mirror[0], pm1 = x.preview_mirror[1];
     const SceneDev sc = e->scene();
     const uint32_t f = cs->frame;
@@ -671,18 +685,18 @@ static void build_schedule(st_engine* e, CameraSlot* cs, std::vector<Step>* step
     const float4* di_final = (d.denoise && (d.mode == ST_MODE_IMAGE || d.mode == ST_MODE_DI_DIFFUSE)) ? cam.di_diff_curr_colors : cam.di_diff_samples;
     const float4* gi_final = (d.denoise && (d.mode == ST_MODE_IMAGE || d.mode == ST_MODE_GI_DIFFUSE)) ? cam.gi_diff_curr_colors : cam.gi_diff_samples;
     if (d.mode == ST_MODE_BVH_HEATMAP) {
-        add(P_BVH_HEATMAP, [=](cudaStream_t s) { launch_bvh_heatmap(cam, sc, s); });
-        add(P_COMPOSITION, [=](cudaStream_t s) { launch_composition(cam, sc, cur, 5u, di_final, gi_final, s); });
+        add(P_BVH_HEATMAP, [=](cudaStream_t s) { launch_bvh_heatmap(*V, sc, s); });
+        add(P_COMPOSITION, [=](cudaStream_t s) { launch_composition(*V, sc, cur, 5u, di_final, gi_final, s); });
         return;
     }
     if (d.mode == ST_MODE_REFERENCE) {
         for (uint32_t depth = 0; depth <= (uint32_t)d.ref_depth; depth++) {
             uint32_t sd = seed(P_REF_SHADING_SEED + depth);
-            add(P_REF_TRACING, [=](cudaStream_t s) { launch_ref_tracing(cam, sc, depth, s); });
-            add(P_REF_SHADING, [=](cudaStream_t s) { launch_ref_shading(cam, sc, sd, depth, s); });
+            add(P_REF_TRACING, [=](cudaStream_t s) { launch_ref_tracing(*V, sc, depth, s); });
+            add(P_REF_SHADING, [=](cudaStream_t s) { launch_ref_shading(*V, sc, sd, depth, s); });
         }
-        add(P_REF_SHADING, [=](cudaStream_t s) { launch_ref_shading(cam, sc, 0u, 255u, s); });
-        add(P_COMPOSITION, [=](cudaStream_t s) { launch_composition(cam, sc, cur, 6u, di_final, gi_final, s); });
+        add(P_REF_SHADING, [=](cudaStream_t s) { launch_ref_shading(*V, sc, 0u, 255u, s); });
+        add(P_COMPOSITION, [=](cudaStream_t s) { launch_composition(*V, sc, cur, 6u, di_final, gi_final, s); });
         return;
     }
     const bool needs_di = d.mode == ST_MODE_IMAGE || d.mode == ST_MODE_DI_DIFFUSE || d.mode == ST_MODE_DI_SPECULAR;
@@ -690,75 +704,75 @@ static void build_schedule(st_engine* e, CameraSlot* cs, std::vector<Step>* step
     // K4 inside the G-buffer launch: only where nothing has to happen between the two (a strip pulls last frame's rows in between,
     // unless nothing moved: then every reprojected read is the pixel itself)
     const int k4_in_k0 = (e->fused_passes && (ext == nullptr || ext->still) && !e->instances.empty()) ? 1 : 0;
-    add(P_PRIM_GBUFFER, [=](cudaStream_t s) { launch_prim_gbuffer(camG, sc, cur, k4_in_k0, s); });
+    add(P_PRIM_GBUFFER, [=](cudaStream_t s) { launch_prim_gbuffer(*VG, sc, cur, k4_in_k0, s); });
     // ST_OPT_FUSED_PASSES: passes whose hand-over is private to a pixel (or to a checkerboard pair) run as one launch; the step keeps
     // the pass id of the member that gathers from other pixels, which is what the strip plans key on.
     const bool fp = e->fused_passes;
     if (!e->instances.empty()) {
-        if (!k4_in_k0) add(P_FRAME_REPROJECTION, [=](cudaStream_t s) { launch_frame_reprojection(cam, sc, cur, s); });
+        if (!k4_in_k0) add(P_FRAME_REPROJECTION, [=](cudaStream_t s) { launch_frame_reprojection(*V, sc, cur, s); });
         if (needs_di) {
             uint32_t s1 = seed(P_DI_SAMPLING), s2 = seed(P_DI_TEMPORAL), s3 = seed(P_DI_SPATIAL_PICK), s5 = seed(P_DI_SPATIAL_SAMPLE);
             if (fp) {
-                add(P_DI_TEMPORAL, [=](cudaStream_t s) { (fs ? stf::launch_di_sample_temporal : st::launch_di_sample_temporal)(cam, sc, cur, s1, s2, f, s); });
-                add(P_DI_SPATIAL_PICK, [=](cudaStream_t s) { (fs ? stf::launch_di_spatial_fused : st::launch_di_spatial_fused)(cam, sc, cur, s3, s5, f, s); });
+                add(P_DI_TEMPORAL, [=](cudaStream_t s) { (fs ? stf::launch_di_sample_temporal : st::launch_di_sample_temporal)(*V, sc, cur, s1, s2, f, s); });
+                add(P_DI_SPATIAL_PICK, [=](cudaStream_t s) { (fs ? stf::launch_di_spatial_fused : st::launch_di_spatial_fused)(*V, sc, cur, s3, s5, f, s); });
             } else {
-                add(P_DI_SAMPLING, [=](cudaStream_t s) { (fs ? stf::launch_di_sampling : st::launch_di_sampling)(cam, sc, cur, s1, f, s); });
-                add(P_DI_TEMPORAL, [=](cudaStream_t s) { (fs ? stf::launch_di_temporal : st::launch_di_temporal)(cam, sc, cur, s2, s); });
-                add(P_DI_SPATIAL_PICK, [=](cudaStream_t s) { (fs ? stf::launch_di_spatial_pick : st::launch_di_spatial_pick)(cam, sc, cur, s3, f, s); });
-                add(P_DI_SPATIAL_TRACE, [=](cudaStream_t s) { (fs ? stf::launch_spatial_trace : st::launch_spatial_trace)(cam, sc, cam.di_diff_samples, cam.di_diff_curr_colors, cam.di_diff_stash, s); });
-                add(P_DI_SPATIAL_SAMPLE, [=](cudaStream_t s) { (fs ? stf::launch_di_spatial_sample : st::launch_di_spatial_sample)(cam, sc, s5, f, s); });
+                add(P_DI_SAMPLING, [=](cudaStream_t s) { (fs ? stf::launch_di_sampling : st::launch_di_sampling)(*V, sc, cur, s1, f, s); });
+                add(P_DI_TEMPORAL, [=](cudaStream_t s) { (fs ? stf::launch_di_temporal : st::launch_di_temporal)(*V, sc, cur, s2, s); });
+                add(P_DI_SPATIAL_PICK, [=](cudaStream_t s) { (fs ? stf::launch_di_spatial_pick : st::launch_di_spatial_pick)(*V, sc, cur, s3, f, s); });
+                add(P_DI_SPATIAL_TRACE, [=](cudaStream_t s) { (fs ? stf::launch_spatial_trace : st::launch_spatial_trace)(*V, sc, cam.di_diff_samples, cam.di_diff_curr_colors, cam.di_diff_stash, s); });
+                add(P_DI_SPATIAL_SAMPLE, [=](cudaStream_t s) { (fs ? stf::launch_di_spatial_sample : st::launch_di_spatial_sample)(*V, sc, s5, f, s); });
             }
-            add(P_DI_RESOLVING, [=](cudaStream_t s) { (fs ? stf::launch_di_resolving : st::launch_di_resolving)(cam, sc, cur, s); });
+            add(P_DI_RESOLVING, [=](cudaStream_t s) { (fs ? stf::launch_di_resolving : st::launch_di_resolving)(*V, sc, cur, s); });
         }
         if (needs_gi) {
             uint32_t sa = seed(P_GI_SAMPLING_A), sb = seed(P_GI_SAMPLING_B), st_ = seed(P_GI_TEMPORAL), sp = seed(P_GI_SPATIAL_PICK), ss = seed(P_GI_SPATIAL_SAMPLE), sv = seed(P_GI_PREVIEW);
             uint32_t source;
             const bool tracing = f % 6u < 4u;
             const int inline_rp = (fp && tracing) ? 1 : 0;   // K11 inside K14; validation frames keep K11 (K12 / K13 read its output)
-            if (!inline_rp) add(P_GI_REPROJECTION, [=](cudaStream_t s) { (fs ? stf::launch_gi_reprojection : st::launch_gi_reprojection)(cam, sc, cur, s); });
+            if (!inline_rp) add(P_GI_REPROJECTION, [=](cudaStream_t s) { (fs ? stf::launch_gi_reprojection : st::launch_gi_reprojection)(*V, sc, cur, s); });
             auto sampling = [&]() {
-                if (fp) { add(P_GI_SAMPLING_B, [=](cudaStream_t s) { (fs ? stf::launch_gi_sampling_fused : st::launch_gi_sampling_fused)(cam, sc, cur, sa, sb, f, s); }); return; }
-                add(P_GI_SAMPLING_A, [=](cudaStream_t s) { (fs ? stf::launch_gi_sampling_a : st::launch_gi_sampling_a)(cam, sc, cur, sa, f, s); });
-                add(P_GI_SAMPLING_B, [=](cudaStream_t s) { (fs ? stf::launch_gi_sampling_b : st::launch_gi_sampling_b)(cam, sc, cur, sb, f, s); });
+                if (fp) { add(P_GI_SAMPLING_B, [=](cudaStream_t s) { (fs ? stf::launch_gi_sampling_fused : st::launch_gi_sampling_fused)(*V, sc, cur, sa, sb, f, s); }); return; }
+                add(P_GI_SAMPLING_A, [=](cudaStream_t s) { (fs ? stf::launch_gi_sampling_a : st::launch_gi_sampling_a)(*V, sc, cur, sa, f, s); });
+                add(P_GI_SAMPLING_B, [=](cudaStream_t s) { (fs ? stf::launch_gi_sampling_b : st::launch_gi_sampling_b)(*V, sc, cur, sb, f, s); });
             };
             if (tracing) {
                 if (f % 2u == 0u) sampling();
-                add(P_GI_TEMPORAL, [=](cudaStream_t s) { (fs ? stf::launch_gi_temporal : st::launch_gi_temporal)(cam, sc, cur, st_, f, inline_rp, s); });
+                add(P_GI_TEMPORAL, [=](cudaStream_t s) { (fs ? stf::launch_gi_temporal : st::launch_gi_temporal)(*V, sc, cur, st_, f, inline_rp, s); });
                 if (f % 2u == 1u) {
-                    if (fp) add(P_GI_SPATIAL_PICK, [=](cudaStream_t s) { (fs ? stf::launch_gi_spatial_fused : st::launch_gi_spatial_fused)(cam, sc, cur, sp, ss, f, s); });
+                    if (fp) add(P_GI_SPATIAL_PICK, [=](cudaStream_t s) { (fs ? stf::launch_gi_spatial_fused : st::launch_gi_spatial_fused)(*V, sc, cur, sp, ss, f, s); });
                     else {
-                        add(P_GI_SPATIAL_PICK, [=](cudaStream_t s) { (fs ? stf::launch_gi_spatial_pick : st::launch_gi_spatial_pick)(cam, sc, cur, sp, f, s); });
-                        add(P_GI_SPATIAL_TRACE, [=](cudaStream_t s) { (fs ? stf::launch_spatial_trace : st::launch_spatial_trace)(cam, sc, cam.gi_d0, cam.gi_d1, cam.gi_d2, s); });
-                        add(P_GI_SPATIAL_SAMPLE, [=](cudaStream_t s) { (fs ? stf::launch_gi_spatial_sample : st::launch_gi_spatial_sample)(cam, sc, ss, f, s); });
+                        add(P_GI_SPATIAL_PICK, [=](cudaStream_t s) { (fs ? stf::launch_gi_spatial_pick : st::launch_gi_spatial_pick)(*V, sc, cur, sp, f, s); });
+                        add(P_GI_SPATIAL_TRACE, [=](cudaStream_t s) { (fs ? stf::launch_spatial_trace : st::launch_spatial_trace)(*V, sc, cam.gi_d0, cam.gi_d1, cam.gi_d2, s); });
+                        add(P_GI_SPATIAL_SAMPLE, [=](cudaStream_t s) { (fs ? stf::launch_gi_spatial_sample : st::launch_gi_spatial_sample)(*V, sc, ss, f, s); });
                     }
                     source = 1;
                 } else source = 0;
             } else {
                 sampling();
-                add(P_GI_TEMPORAL, [=](cudaStream_t s) { (fs ? stf::launch_gi_temporal : st::launch_gi_temporal)(cam, sc, cur, st_, f, 0, s); });
+                add(P_GI_TEMPORAL, [=](cudaStream_t s) { (fs ? stf::launch_gi_temporal : st::launch_gi_temporal)(*V, sc, cur, st_, f, 0, s); });
                 source = 0;
             }
             const float4* src0 = source == 0 ? cam.gi_reservoirs[1] : cam.gi_reservoirs[2];
-            add(P_GI_PREVIEW, [=](cudaStream_t s) { (fs ? stf::launch_gi_preview : st::launch_gi_preview)(cam, sc, cur, sv, 0u, src0, cam.gi_reservoirs[3], pm0, s); });
-            if (fp) add(P_GI_PREVIEW, [=](cudaStream_t s) { (fs ? stf::launch_gi_preview_resolve : st::launch_gi_preview_resolve)(cam, sc, cur, sv, cam.gi_reservoirs[3], src0, s); });
+            add(P_GI_PREVIEW, [=](cudaStream_t s) { (fs ? stf::launch_gi_preview : st::launch_gi_preview)(*V, sc, cur, sv, 0u, src0, cam.gi_reservoirs[3], pm0, s); });
+            if (fp) add(P_GI_PREVIEW, [=](cudaStream_t s) { (fs ? stf::launch_gi_preview_resolve : st::launch_gi_preview_resolve)(*V, sc, cur, sv, cam.gi_reservoirs[3], src0, s); });
             else {
-                add(P_GI_PREVIEW, [=](cudaStream_t s) { (fs ? stf::launch_gi_preview : st::launch_gi_preview)(cam, sc, cur, sv, 1u, cam.gi_reservoirs[3], cam.gi_reservoirs[0], pm1, s); });
-                add(P_GI_RESOLVING, [=](cudaStream_t s) { (fs ? stf::launch_gi_resolving : st::launch_gi_resolving)(cam, sc, cur, src0, s); });
+                add(P_GI_PREVIEW, [=](cudaStream_t s) { (fs ? stf::launch_gi_preview : st::launch_gi_preview)(*V, sc, cur, sv, 1u, cam.gi_reservoirs[3], cam.gi_reservoirs[0], pm1, s); });
+                add(P_GI_RESOLVING, [=](cudaStream_t s) { (fs ? stf::launch_gi_resolving : st::launch_gi_resolving)(*V, sc, cur, src0, s); });
             }
         }
     }
     if (d.denoise) {   // FrameDenoisingPass::run (passes/frame_denoising.rs:143-190)
         if (e->fuse_reproject) {   // ST_OPT_FUSE_REPROJECT: both signals in one launch (same arithmetic, shared surface/reprojection reads)
-            add(P_DENOISE_REPROJECT, [=](cudaStream_t s) { launch_denoise_reproject_pair(cam, sc, cur, s); });
+            add(P_DENOISE_REPROJECT, [=](cudaStream_t s) { launch_denoise_reproject_pair(*V, sc, cur, s); });
         } else {
-            add(P_DENOISE_REPROJECT, [=](cudaStream_t s) { launch_denoise_reproject(cam, sc, cur, cam.di_diff_prev_colors, cam.di_diff_moments[cur ^ 1], cam.di_diff_samples, cam.di_diff_curr_colors, cam.di_diff_moments[cur], s); });
-            add(P_DENOISE_REPROJECT, [=](cudaStream_t s) { launch_denoise_reproject(cam, sc, cur, cam.gi_diff_prev_colors, cam.gi_diff_moments[cur ^ 1], cam.gi_diff_samples, cam.gi_diff_curr_colors, cam.gi_diff_moments[cur], s); });
+            add(P_DENOISE_REPROJECT, [=](cudaStream_t s) { launch_denoise_reproject(*V, sc, cur, cam.di_diff_prev_colors, cam.di_diff_moments[cur ^ 1], cam.di_diff_samples, cam.di_diff_curr_colors, cam.di_diff_moments[cur], s); });
+            add(P_DENOISE_REPROJECT, [=](cudaStream_t s) { launch_denoise_reproject(*V, sc, cur, cam.gi_diff_prev_colors, cam.gi_diff_moments[cur ^ 1], cam.gi_diff_samples, cam.gi_diff_curr_colors, cam.gi_diff_moments[cur], s); });
         }
         const bool fast = e->svgf_fast;
-        const bool var_tiled = e->variance_tiled; uint32_t* verr = (uint32_t*)e->d_tile_errors.p;
+        const bool var_tiled = one && e->variance_tiled; uint32_t* verr = (uint32_t*)e->d_tile_errors.p;
         add(P_DENOISE_VARIANCE, [=](cudaStream_t s) {
-            if (var_tiled && launch_denoise_variance_tiled(camV, sc, cur, fast, verr, s)) { e->variance_tiled_launches++; return; }
-            launch_denoise_variance(camV, sc, cur, fast, s);
+            if (var_tiled && launch_denoise_variance_tiled(VV->front().cam, sc, cur, fast, verr, s)) { e->variance_tiled_launches++; return; }
+            launch_denoise_variance(*VV, sc, cur, fast, s);
         });
         float4* di_io[5][2] = {{cam.di_diff_stash, cam.di_diff_prev_colors}, {cam.di_diff_prev_colors, cam.di_diff_stash}, {cam.di_diff_stash, cam.di_diff_curr_colors},
                                {cam.di_diff_curr_colors, cam.di_diff_stash}, {cam.di_diff_stash, cam.di_diff_curr_colors}};
@@ -771,18 +785,18 @@ static void build_schedule(st_engine* e, CameraSlot* cs, std::vector<Step>* step
             float4 *a = di_io[nth][0], *b = di_io[nth][1], *c = gi_io[nth][0], *g = gi_io[nth][1];
             const bool reads_pair = (int)nth >= first_paired_read, writes_pair = (int)nth + 1 >= first_paired_read && nth < 4;
             const float4* pin = reads_pair ? cs->pair[nth & 1] : nullptr; float4* pout = writes_pair ? cs->pair[(nth + 1) & 1] : nullptr;
-            const bool tiled = !reads_pair && ((e->wavelet_tiled >> nth) & 1) != 0; const int cfg = (e->wavelet_cfg >> (4 * nth)) & 15;
+            const bool tiled = one && !reads_pair && ((e->wavelet_tiled >> nth) & 1) != 0; const int cfg = (e->wavelet_cfg >> (4 * nth)) & 15;
             uint32_t* terr = (uint32_t*)e->d_tile_errors.p;
-            const CameraDev camW = grown(cam, x.wavelet[nth]);
+            const Views VW = views(x.wavelet[nth]);
             add(P_DENOISE_WAVELET, [=](cudaStream_t s) {
-                if (tiled && launch_denoise_wavelet_tiled(camW, sc, f, 1u << nth, (float)(1 + nth), a, b, c, g, pout, fast, cfg, terr, s)) { e->wavelet_tiled_launches++; return; }
-                launch_denoise_wavelet(camW, sc, cur, f, 1u << nth, (float)(1 + nth), a, b, c, g, pin, pout, fast, s);
+                if (tiled && launch_denoise_wavelet_tiled(VW->front().cam, sc, f, 1u << nth, (float)(1 + nth), a, b, c, g, pout, fast, cfg, terr, s)) { e->wavelet_tiled_launches++; return; }
+                launch_denoise_wavelet(*VW, sc, cur, f, 1u << nth, (float)(1 + nth), a, b, c, g, pin, pout, fast, s);
             });
             steps->back().sub = (int)nth;
         }
     }
     uint32_t mode = (uint32_t)d.mode;
-    add(P_COMPOSITION, [=](cudaStream_t s) { launch_composition(cam, sc, cur, mode, di_final, gi_final, s); });
+    add(P_COMPOSITION, [=](cudaStream_t s) { launch_composition(*V, sc, cur, mode, di_final, gi_final, s); });
 }
 
 
@@ -1039,7 +1053,7 @@ static int render_strips_fused(st_engine* e, CameraSlot* cs, const std::vector<s
     // frame at the pixel itself — no rows to pull, K4 can run inside the G-buffer launch.  Every rank sees the same updates, hence decides alike.
     ext.still = cs->frame > 1 && !e->moved_last_tick && std::memcmp(&cs->dev.curr, &cs->dev.prev, sizeof(GpuCamera)) == 0;
     if (ext.still) d.need_rows = nullptr;
-    std::vector<Step> steps; build_schedule(e, cs, &steps, &ext);
+    std::vector<Step> steps; build_schedule(e, {cs}, &steps, &ext);
 
     StripSync ss; ss.my_flags = sync; ss.errors = sync + kStripErrorWord; ss.n_ranks = N; ss.rank = R;
     for (int r = 0; r < ST_PEER_MAX_RANKS; r++) ss.peer_flags[r] = (r < N && r != R) ? cs->peer.flags[r] : nullptr;
@@ -1433,7 +1447,7 @@ int st_tick(st_engine* e) {   // Engine::tick (lib.rs:301-395)
 int st_frame_schedule(st_engine* e, st_camera_handle h, int* pass_ids, int cap, int* count) {
     CameraSlot* cs = e ? get_camera(e, h) : nullptr;
     if (!cs || !count) return fail(ST_ERR_NOT_FOUND, "unknown camera");
-    std::vector<Step> steps; build_schedule(e, cs, &steps);
+    std::vector<Step> steps; build_schedule(e, {cs}, &steps);
     *count = (int)steps.size();
     for (int i = 0; i < cap && i < *count; i++) pass_ids[i] = steps[i].pass;
     return ST_OK;
@@ -1444,7 +1458,7 @@ int st_render_range(st_engine* e, st_camera_handle h, int first, int last) {
     if (cs->frame == 0) return fail(ST_ERR_INVALID, "st_tick must precede st_render_camera");
     CK(cudaSetDevice(e->device));
     int rc = ensure_luts(e); if (rc) return rc;
-    std::vector<Step> steps; build_schedule(e, cs, &steps);
+    std::vector<Step> steps; build_schedule(e, {cs}, &steps);
     if (last < 0 || last >= (int)steps.size()) last = (int)steps.size() - 1;
     for (int i = std::max(first, 0); i <= last; i++) e->run_timed(steps[i].pass, steps[i].run, steps[i].sub);
     CK(cudaGetLastError());
@@ -1495,11 +1509,11 @@ static int copy_rows_out(st_engine* e, CameraSlot* cs, const OutputTarget& t, in
     const size_t W = cs->desc.width, n = W * cs->desc.height, bpp = format_bpp(t.format);
     if (!bpp) return fail(ST_ERR_INVALID, "unsupported output format");
     const size_t rows = (size_t)(y1 - y0), row_bytes = W * bpp;
-    SceneDev sc = e->scene(); CameraDev cd = cs->dev; cd.y0 = y0; cd.y1 = y1;
+    SceneDev sc = e->scene(); ViewSet v(1, view_of(cs, cs, 0)); v[0].cam.y0 = y0; v[0].cam.y1 = y1;
     const int format = t.format;
     if (t.device) {
-        char* dst = t.dst; const size_t pitch = t.pitch;
-        e->run_timed(P_COMPOSITION, [=](cudaStream_t s) { launch_output_store(cd, sc, format, dst, pitch, s); });
+        v[0].dst = t.dst; v[0].pitch = t.pitch;
+        e->run_timed(P_COMPOSITION, [&](cudaStream_t s) { launch_output_store(v, sc, format, s); });
         CK(cudaGetLastError());
         return ST_OK;
     }
@@ -1514,7 +1528,8 @@ static int copy_rows_out(st_engine* e, CameraSlot* cs, const OutputTarget& t, in
         if (!cs->ev_ready[k]) { CK(cudaEventCreateWithFlags(&cs->ev_ready[k], cudaEventDisableTiming)); CK(cudaEventCreateWithFlags(&cs->ev_copied[k], cudaEventDisableTiming)); }
         else CK(cudaStreamWaitEvent(e->stream, cs->ev_copied[k], 0));   // slot k's previous copy must have left the staging buffer
     }
-    e->run_timed(P_COMPOSITION, [=](cudaStream_t s) { launch_output_store(cd, sc, format, slot, row_bytes, s); });
+    v[0].dst = slot; v[0].pitch = row_bytes;
+    e->run_timed(P_COMPOSITION, [&](cudaStream_t s) { launch_output_store(v, sc, format, s); });
     if (e->async_output) {
         CK(cudaEventRecord(cs->ev_ready[k], e->stream));
         CK(cudaStreamWaitEvent(e->copy_stream, cs->ev_ready[k], 0));
@@ -1540,6 +1555,53 @@ int st_render_camera_to(st_engine* e, st_camera_handle h, void* dst, size_t pitc
     if ((rc = st_render_range(e, h, 0, -1))) return rc;
     if ((rc = copy_rows_out(e, cs, t, 0, (int)cs->desc.height))) return rc;
     if (!t.device && !e->async_output) CK(cudaStreamSynchronize(e->stream));
+    return ST_OK;
+}
+// Several cameras of one frame.  Every camera rendered after the same tick has the same frame id, so cameras of one size and mode run
+// the same passes with the same seeds; such a group runs as one launch per pass, blockIdx.z selecting the camera.
+int st_render_cameras(st_engine* e, const st_camera_handle* cameras, int n, void* const* dsts, const size_t* pitch_bytes, int format) {
+    if (!e) return fail(ST_ERR_INVALID, "null engine");
+    if (n <= 0 || !cameras) return fail(ST_ERR_INVALID, "no cameras to render");
+    CK(cudaSetDevice(e->device));
+    std::vector<CameraSlot*> cs(n);
+    std::vector<OutputTarget> t(n);
+    for (int i = 0; i < n; i++) {   // everything is checked before any pass runs: a refused call changes nothing
+        if (!(cs[i] = get_camera(e, cameras[i]))) return fail(ST_ERR_NOT_FOUND, "unknown camera " + std::to_string(cameras[i]));
+        if (std::find(cameras, cameras + i, cameras[i]) != cameras + i) return fail(ST_ERR_INVALID, "camera " + std::to_string(cameras[i]) + " is listed twice");
+        if (cs[i]->dev.y0 != 0 || cs[i]->dev.y1 != (int)cs[i]->desc.height || cs[i]->peer.ready)
+            return fail(ST_ERR_INVALID, "camera " + std::to_string(cameras[i]) + " renders a row strip; st_render_cameras takes whole-frame cameras only");
+        if (cs[i]->frame == 0) return fail(ST_ERR_INVALID, "st_tick must precede st_render_camera");
+        t[i].dst = nullptr;
+        if (dsts && dsts[i]) { int rc = resolve_target(e, cs[i]->desc.width, dsts[i], pitch_bytes ? pitch_bytes[i] : 0, format, &t[i]); if (rc) return rc; }
+    }
+    int rc = ensure_luts(e); if (rc) return rc;
+    // groups by (width, height, mode, denoise, ref_depth), in the order of their first camera; list order within a group
+    std::vector<std::vector<int>> groups;
+    for (int i = 0; i < n; i++) {
+        const st_camera& d = cs[i]->desc;
+        auto same = [&](const std::vector<int>& g) {
+            const st_camera& a = cs[g[0]]->desc;
+            return a.width == d.width && a.height == d.height && a.mode == d.mode && a.denoise == d.denoise && a.ref_depth == d.ref_depth;
+        };
+        auto it = std::find_if(groups.begin(), groups.end(), same);
+        if (it == groups.end()) groups.push_back({i}); else it->push_back(i);
+    }
+    bool host_out = false;
+    for (const std::vector<int>& g : groups) {
+        for (size_t c0 = 0; c0 < g.size(); c0 += kBatchViews) {
+            const std::vector<int> idx(g.begin() + c0, g.begin() + std::min(g.size(), c0 + kBatchViews));
+            std::vector<CameraSlot*> chunk;
+            for (int i : idx) chunk.push_back(cs[i]);
+            std::vector<Step> steps; build_schedule(e, chunk, &steps);
+            for (const Step& s : steps) e->run_timed(s.pass, s.run, s.sub);
+            ViewSet store;   // the device surfaces of the chunk: one store launch
+            for (int i : idx) if (t[i].dst && t[i].device) { store.push_back(view_of(cs[i], chunk[0], 0)); store.back().dst = t[i].dst; store.back().pitch = t[i].pitch; }
+            if (!store.empty()) { const SceneDev sc = e->scene(); e->run_timed(P_COMPOSITION, [&](cudaStream_t s) { launch_output_store(store, sc, format, s); }); }
+            for (int i : idx) if (t[i].dst && !t[i].device) { host_out = true; if ((rc = copy_rows_out(e, cs[i], t[i], 0, (int)cs[i]->desc.height))) return rc; }
+        }
+    }
+    CK(cudaGetLastError());
+    if (host_out && !e->async_output) CK(cudaStreamSynchronize(e->stream));
     return ST_OK;
 }
 int st_synchronize(st_engine* e) {
@@ -1852,7 +1914,7 @@ static int enqueue_strip_frame(st_engine* e, CameraSlot* cs, int temporal_reach)
         if ((rc = render_strips_fused(e, cs, bounds))) return rc;
         // rows mirrored into this rank by its neighbours (the K6 / K14 / K17 / K18 / K20 stores); the temporal pull is counted on the device
         const uint64_t W = cs->desc.width; const int nbs = (e->rank > 0 ? 1 : 0) + (e->rank + 1 < e->n_ranks ? 1 : 0);
-        std::vector<Step> steps; build_schedule(e, cs, &steps);
+        std::vector<Step> steps; build_schedule(e, {cs}, &steps);
         bool di = false, gi = false, sp = false, dn = cs->desc.denoise != 0;
         for (const Step& st : steps) { di |= st.pass == P_DI_TEMPORAL; gi |= st.pass == P_GI_TEMPORAL; sp |= st.pass == P_GI_SPATIAL_PICK; }
         uint64_t per_nb = 0;
@@ -1862,7 +1924,7 @@ static int enqueue_strip_frame(st_engine* e, CameraSlot* cs, int temporal_reach)
         e->halo_bytes_last_frame = per_nb * W * nbs;
     } else {
         cs->dev.mirror_up = cs->dev.mirror_dn = 0; cs->dev.need_rows = nullptr;
-        std::vector<Step> steps; build_schedule(e, cs, &steps);
+        std::vector<Step> steps; build_schedule(e, {cs}, &steps);
         std::vector<int> ids; for (const Step& st : steps) ids.push_back(st.pass);
         std::vector<HaloExchange> plan;
         // The exchange-point transports ship a FIXED number of last frame's rows.  That is only enough while nothing moves: with a moving
@@ -1933,8 +1995,9 @@ int st_render_strips(st_engine* e, st_camera_handle h, void* host_out, int forma
     else {
         if ((rc = cs->staging.ensure(2 * n * kStagingBpp))) return rc;
         cs->staging_slot ^= 1;
-        SceneDev sc = e->scene(); char* slot = (char*)cs->staging.p + (cs->staging_slot ? n * kStagingBpp : 0); CameraDev cd = cs->dev;
-        e->run_timed(P_COMPOSITION, [=](cudaStream_t s) { launch_output_store(cd, sc, format, slot, W * px_bytes, s); });
+        SceneDev sc = e->scene(); char* slot = (char*)cs->staging.p + (cs->staging_slot ? n * kStagingBpp : 0);
+        ViewSet v(1, view_of(cs, cs, 0)); v[0].dst = slot; v[0].pitch = W * px_bytes;
+        e->run_timed(P_COMPOSITION, [&](cudaStream_t s) { launch_output_store(v, sc, format, s); });
         base = slot; dt = ncclUint8; per_px = px_bytes;
     }
     if (peer) {

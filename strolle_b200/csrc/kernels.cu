@@ -69,6 +69,14 @@ ST_DEV Hit load_hit_lut(const SceneDev& sc, const GpuCamera& c, const float4* __
     TraceStack stk; stk.base = s_stack + threadIdx.x;
 
 #define KPARAMS const __grid_constant__ CameraDev cam, const __grid_constant__ SceneDev sc
+// The per-pixel kernels are instantiated twice: BATCHED = false reads its one camera at fixed parameter offsets (every single-camera
+// frame runs this), BATCHED = true takes the view from blockIdx.z (st_render_cameras).  The choice follows the launch's view count.
+#define VPARAMS const __grid_constant__ ViewBatch<BATCHED> views, const __grid_constant__ SceneDev sc
+#define VIEW const ViewDev& view = views.v[BATCHED ? blockIdx.z : 0]; const CameraDev& cam = view.cam
+#define VIEW_ARENA(p) p = arena_ptr<BATCHED>(p, view)
+// a buffer pointer passed as a launch argument (view 0's) moved to the same buffer of this thread's view
+template <bool BATCHED, class T> ST_DEV T* arena_ptr(T* p, const ViewDev& v) { return (BATCHED && p) ? (T*)((char*)p + v.arena_delta) : p; }
+template <bool BATCHED, class T> ST_DEV T* pair_ptr(T* p, const ViewDev& v) { return (BATCHED && p) ? (T*)((char*)p + v.pair_delta) : p; }
 
 // Launch bounds per kernel: ST_LB_<KERNEL> is __launch_bounds__(128) (ptxas' own register choice) unless a minimum number
 // of resident CTAs per SM is set (ST_MINB_<KERNEL> = N caps registers at 65536 / (128 N)); values tuned on a B200 with
@@ -90,8 +98,10 @@ ST_DEV Hit load_hit_lut(const SceneDev& sc, const GpuCamera& c, const float4* __
 #else
 #define ST_MINB_ALL_OR_0 0
 #endif
+// The caps hold for the single-camera instantiations.  A batched instantiation (BATCHED, see VPARAMS) reads the camera through register-
+// indexed constant loads, which need registers of their own; under the same cap it would spill, so ptxas chooses its registers.
 template <int ALL, int ONE> struct LbMin { static constexpr int value = ALL > 0 ? ALL : ONE; };
-#define ST_LB_CHOOSE(all, one) __launch_bounds__(ST_BLOCK, (LbMin<all, one>::value > 0 ? LbMin<all, one>::value : 1))
+#define ST_LB_CHOOSE(all, one) __launch_bounds__(ST_BLOCK, (!BATCHED && LbMin<all, one>::value > 0 ? LbMin<all, one>::value : 1))
 #ifndef ST_MINB_PRIM_GBUFFER
 #define ST_MINB_PRIM_GBUFFER 0
 #endif
@@ -151,7 +161,9 @@ template <int ALL, int ONE> struct LbMin { static constexpr int value = ALL > 0 
 // ---------------------------------------------------------------------------------------------
 ST_DEV float4 frame_reprojection_px(const CameraDev& cam, int cur, Px p, float4 surface_texel, float4 vel);
 // `with_reprojection` (ST_OPT_FUSED_PASSES; single GPU, or a strip on a frame where nothing moved): K4 runs in this launch too — its inputs for the pixel are still in registers
-__global__ void ST_LB_PRIM_GBUFFER k_prim_gbuffer(KPARAMS, int cur, int with_reprojection) {
+template <bool BATCHED>
+__global__ void ST_LB_PRIM_GBUFFER k_prim_gbuffer(VPARAMS, int cur, int with_reprojection) {
+    VIEW;
     ST_TRACE_STACK();
     Px p = pixel_full(cam);
     if (!p.in) return;
@@ -218,7 +230,9 @@ ST_DEV float4 frame_reprojection_px(const CameraDev& cam, int cur, Px p, float4 
     }
     return reproj_encode(rp);
 }
-__global__ void __launch_bounds__(ST_BLOCK) k_frame_reprojection(KPARAMS, int cur) {
+template <bool BATCHED>
+__global__ void __launch_bounds__(ST_BLOCK) k_frame_reprojection(VPARAMS, int cur) {
+    VIEW;
     Px p = pixel_full(cam);
     if (!p.in) return;
     size_t i = pix(cam, p.x, p.y);
@@ -240,7 +254,9 @@ ST_DEV DiRes di_sampling_px(const CameraDev& cam, const SceneDev& sc, const Trac
     }
     return out;
 }
-__global__ void ST_LB_DI_SAMPLING k_di_sampling(KPARAMS, int cur, u32 seed, u32 frame) {
+template <bool BATCHED>
+__global__ void ST_LB_DI_SAMPLING k_di_sampling(VPARAMS, int cur, u32 seed, u32 frame) {
+    VIEW;
     ST_TRACE_STACK();
     Px p = pixel_full(cam);
     if (!p.in) return;
@@ -287,7 +303,9 @@ ST_DEV DiRes di_temporal_px(const CameraDev& cam, const SceneDev& sc, int cur, u
     main_.w = res_norm(main_.w, main_pdf, 1.0f, 1.0f);
     return main_;
 }
-__global__ void ST_LB_DI_TEMPORAL k_di_temporal(KPARAMS, int cur, u32 seed) {
+template <bool BATCHED>
+__global__ void ST_LB_DI_TEMPORAL k_di_temporal(VPARAMS, int cur, u32 seed) {
+    VIEW;
     Px p = pixel_full(cam);
     if (!p.in) return;
     size_t lhs_idx = screen_idx(cam, p.x, p.y);
@@ -298,7 +316,9 @@ __global__ void ST_LB_DI_TEMPORAL k_di_temporal(KPARAMS, int cur, u32 seed) {
 // K5 + K6 in one launch (ST_OPT_FUSED_PASSES): the pixel's fresh sample goes from K5 to K6 in registers instead of through di_reservoirs[1]
 // (the hit is decoded once).  What di_store / di_load would do to the sample on the way (confidence -> byte) is the identity for K5's
 // output (confidence 0), so the result is the two-launch result bit for bit.
-__global__ void ST_LB_DI_SAMPLING k_di_sample_temporal(KPARAMS, int cur, u32 seed_sampling, u32 seed_temporal, u32 frame) {
+template <bool BATCHED>
+__global__ void ST_LB_DI_SAMPLING k_di_sample_temporal(VPARAMS, int cur, u32 seed_sampling, u32 seed_temporal, u32 frame) {
+    VIEW;
     ST_TRACE_STACK();
     Px p = pixel_full(cam);
     if (!p.in) return;
@@ -361,7 +381,9 @@ ST_DEV void store_pair_texels(const CameraDev& cam, const PairTexels& o, float4*
     if (o.state == 2) { tex_store(buf_d0, cam, ax, g.y, o.a0); tex_store(buf_d0, cam, bx, g.y, o.b0); }
     tex_store(buf_d1, cam, ax, g.y, o.a1); tex_store(buf_d1, cam, bx, g.y, o.b1);
 }
-__global__ void ST_LB_DI_SPATIAL_PICK k_di_spatial_pick(KPARAMS, int cur, u32 seed, u32 frame) {
+template <bool BATCHED>
+__global__ void ST_LB_DI_SPATIAL_PICK k_di_spatial_pick(VPARAMS, int cur, u32 seed, u32 frame) {
+    VIEW;
     Px g = pixel_half(cam);
     if (!g.in) return;
     store_pair_texels(cam, di_spatial_pick_pair(cam, sc, cur, seed, frame, g), cam.di_diff_samples, cam.di_diff_curr_colors, g);
@@ -374,7 +396,9 @@ ST_DEV float4 spatial_trace_texel(const SceneDev& sc, const TraceStack& stk, flo
     bool occ = trace_any(ray, sc, stk);
     return f4(occ ? 0.0f : 1.0f, d1.z, d1.w, 0.0f);
 }
-__global__ void ST_LB_SPATIAL_TRACE k_spatial_trace(KPARAMS, const float4* __restrict__ buf_d0, const float4* __restrict__ buf_d1, float4* __restrict__ buf_d2) {
+template <bool BATCHED>
+__global__ void ST_LB_SPATIAL_TRACE k_spatial_trace(VPARAMS, const float4* __restrict__ buf_d0, const float4* __restrict__ buf_d1, float4* __restrict__ buf_d2) {
+    VIEW; VIEW_ARENA(buf_d0); VIEW_ARENA(buf_d1); VIEW_ARENA(buf_d2);
     ST_TRACE_STACK();
     Px p = pixel_full(cam);
     if (!p.in) return;
@@ -417,7 +441,9 @@ ST_DEV void di_spatial_sample_pair(const CameraDev& cam, u32 seed, u32 frame, Px
     uint2 op = checker(g.x, g.y, frame / 2u);
     if (cam_contains_u(cam.curr, op.x, op.y)) { size_t oi = screen_idx(cam, op.x, op.y); di_store(di_load(in, oi), out, oi); }
 }
-__global__ void __launch_bounds__(ST_BLOCK) k_di_spatial_sample(KPARAMS, u32 seed, u32 frame) {
+template <bool BATCHED>
+__global__ void __launch_bounds__(ST_BLOCK) k_di_spatial_sample(VPARAMS, u32 seed, u32 frame) {
+    VIEW;
     Px g = pixel_half(cam);
     if (!g.in) return;
     di_spatial_sample_pair(cam, seed, frame, g, tex_or_zero(cam.di_diff_stash, cam, g.x * 2u, g.y), tex_or_zero(cam.di_diff_stash, cam, g.x * 2u + 1u, g.y));
@@ -425,7 +451,9 @@ __global__ void __launch_bounds__(ST_BLOCK) k_di_spatial_sample(KPARAMS, u32 see
 // K7 + K8 + K9 in one launch (ST_OPT_FUSED_PASSES): one thread per checkerboard pair picks the neighbour, traces the pair's two shadow
 // rays and merges — the three scratch textures (48 B per pixel written and read back) never leave the registers.  Same draws, same rays
 // (direction through the same octahedral round trip), same merge as the three-launch sequence.
-__global__ void ST_LB_DI_SPATIAL_PICK k_di_spatial_fused(KPARAMS, int cur, u32 seed_pick, u32 seed_sample, u32 frame) {
+template <bool BATCHED>
+__global__ void ST_LB_DI_SPATIAL_PICK k_di_spatial_fused(VPARAMS, int cur, u32 seed_pick, u32 seed_sample, u32 frame) {
+    VIEW;
     ST_TRACE_STACK();
     Px g = pixel_half(cam);
     if (!g.in) return;
@@ -436,7 +464,9 @@ __global__ void ST_LB_DI_SPATIAL_PICK k_di_spatial_fused(KPARAMS, int cur, u32 s
 }
 
 // K10 di_resolving::main (di_resolving.rs:4-119)
-__global__ void ST_LB_DI_RESOLVING k_di_resolving(KPARAMS, int cur) {
+template <bool BATCHED>
+__global__ void ST_LB_DI_RESOLVING k_di_resolving(VPARAMS, int cur) {
+    VIEW;
     ST_TRACE_STACK();
     Px p = pixel_full(cam);
     if (!p.in) return;
@@ -477,7 +507,9 @@ ST_DEV GiRes gi_reprojection_px(const CameraDev& cam, const Hit& hit, const Repr
     res.v1 = hit.point;
     return res;
 }
-__global__ void __launch_bounds__(ST_BLOCK) k_gi_reprojection(KPARAMS, int cur) {
+template <bool BATCHED>
+__global__ void __launch_bounds__(ST_BLOCK) k_gi_reprojection(VPARAMS, int cur) {
+    VIEW;
     Px p = pixel_full(cam);
     if (!p.in) return;
     Hit hit = load_hit_lut(sc, cam.curr, cam.prim_gbuffer_d0[cur], cam.prim_gbuffer_d1[cur], cam, p.x, p.y);
@@ -524,7 +556,9 @@ ST_DEV bool gi_sampling_a_pair(const CameraDev& cam, const SceneDev& sc, const T
     *t0 = f4(gi_r.d, gi_pdf_);
     return true;
 }
-__global__ void ST_LB_GI_SAMPLING_A k_gi_sampling_a(KPARAMS, int cur, u32 seed, u32 frame) {
+template <bool BATCHED>
+__global__ void ST_LB_GI_SAMPLING_A k_gi_sampling_a(VPARAMS, int cur, u32 seed, u32 frame) {
+    VIEW;
     ST_TRACE_STACK();
     Px g = pixel_half(cam);
     if (!g.in) return;
@@ -592,7 +626,9 @@ ST_DEV void gi_sampling_b_pair(const CameraDev& cam, const SceneDev& sc, const T
     }
     gi_store(res, cam.gi_reservoirs[1], idx);
 }
-__global__ void ST_LB_GI_SAMPLING_B k_gi_sampling_b(KPARAMS, int cur, u32 seed, u32 frame) {
+template <bool BATCHED>
+__global__ void ST_LB_GI_SAMPLING_B k_gi_sampling_b(VPARAMS, int cur, u32 seed, u32 frame) {
+    VIEW;
     ST_TRACE_STACK();
     Px g = pixel_half(cam);
     if (!g.in) return;
@@ -601,7 +637,9 @@ __global__ void ST_LB_GI_SAMPLING_B k_gi_sampling_b(KPARAMS, int cur, u32 seed, 
 }
 // K12 + K13 in one launch (ST_OPT_FUSED_PASSES): the bounce ray is traced and shaded by the same thread; the hit still goes through
 // GBufferEntry's pack / unpack (its 8-bit quantisation is part of the result), just not through memory.
-__global__ void ST_LB_GI_SAMPLING_B k_gi_sampling_fused(KPARAMS, int cur, u32 seed_a, u32 seed_b, u32 frame) {
+template <bool BATCHED>
+__global__ void ST_LB_GI_SAMPLING_B k_gi_sampling_fused(VPARAMS, int cur, u32 seed_a, u32 seed_b, u32 frame) {
+    VIEW;
     ST_TRACE_STACK();
     Px g = pixel_half(cam);
     if (!g.in) return;
@@ -615,7 +653,9 @@ __global__ void ST_LB_GI_SAMPLING_B k_gi_sampling_fused(KPARAMS, int cur, u32 se
 // reservoir is fetched from gi_reservoirs[0] at the reprojected position directly, and handed on as K11 would have left it in
 // gi_reservoirs[2] (its normal goes through the same octahedral store / load round trip).  gi_reservoirs[2] itself is then only written
 // for the columns a later pass still reads there (those the checkerboard passes do not cover when the width is odd).
-__global__ void ST_LB_GI_TEMPORAL k_gi_temporal(KPARAMS, int cur, u32 seed, u32 frame, int inline_reprojection) {
+template <bool BATCHED>
+__global__ void ST_LB_GI_TEMPORAL k_gi_temporal(VPARAMS, int cur, u32 seed, u32 frame, int inline_reprojection) {
+    VIEW;
     Px p = pixel_full(cam);
     if (!p.in) return;
     bool tracing = gi_tracing_frame(frame);
@@ -717,7 +757,9 @@ ST_DEV PairTexels gi_spatial_pick_pair(const CameraDev& cam, const SceneDev& sc,
     o.state = 2;
     return o;
 }
-__global__ void ST_LB_GI_SPATIAL_PICK k_gi_spatial_pick(KPARAMS, int cur, u32 seed, u32 frame) {
+template <bool BATCHED>
+__global__ void ST_LB_GI_SPATIAL_PICK k_gi_spatial_pick(VPARAMS, int cur, u32 seed, u32 frame) {
+    VIEW;
     Px g = pixel_half(cam);
     if (!g.in) return;
     store_pair_texels(cam, gi_spatial_pick_pair(cam, sc, cur, seed, frame, g), cam.gi_d0, cam.gi_d1, g);
@@ -755,13 +797,17 @@ ST_DEV void gi_spatial_sample_pair(const CameraDev& cam, u32 seed, u32 frame, Px
     uint2 op = checker(g.x, g.y, frame / 2u);
     if (cam_contains_u(cam.curr, op.x, op.y)) { size_t oi = screen_idx(cam, op.x, op.y); gi_store_m(cam, gi_load(in, oi), out, oi, op.y, cam.gi_mirror_reach); }
 }
-__global__ void ST_LB_GI_SPATIAL_SAMPLE k_gi_spatial_sample(KPARAMS, u32 seed, u32 frame) {
+template <bool BATCHED>
+__global__ void ST_LB_GI_SPATIAL_SAMPLE k_gi_spatial_sample(VPARAMS, u32 seed, u32 frame) {
+    VIEW;
     Px g = pixel_half(cam);
     if (!g.in) return;
     gi_spatial_sample_pair(cam, seed, frame, g, tex_or_zero(cam.gi_d2, cam, g.x * 2u, g.y), tex_or_zero(cam.gi_d2, cam, g.x * 2u + 1u, g.y));
 }
 // K15 + K16 + K17 in one launch (ST_OPT_FUSED_PASSES), like k_di_spatial_fused
-__global__ void ST_LB_GI_SPATIAL_PICK k_gi_spatial_fused(KPARAMS, int cur, u32 seed_pick, u32 seed_sample, u32 frame) {
+template <bool BATCHED>
+__global__ void ST_LB_GI_SPATIAL_PICK k_gi_spatial_fused(VPARAMS, int cur, u32 seed_pick, u32 seed_sample, u32 frame) {
+    VIEW;
     ST_TRACE_STACK();
     Px g = pixel_half(cam);
     if (!g.in) return;
@@ -809,7 +855,9 @@ ST_DEV bool gi_preview_px(const CameraDev& cam, const SceneDev& sc, const Hit& c
     *result = main_;
     return true;
 }
-__global__ void ST_LB_GI_PREVIEW k_gi_preview(KPARAMS, int cur, u32 seed, u32 nth, const float4* __restrict__ in, float4* __restrict__ out, int reach) {
+template <bool BATCHED>
+__global__ void ST_LB_GI_PREVIEW k_gi_preview(VPARAMS, int cur, u32 seed, u32 nth, const float4* __restrict__ in, float4* __restrict__ out, int reach) {
+    VIEW; VIEW_ARENA(in); VIEW_ARENA(out);
     Px p = pixel_full(cam);
     if (!p.in) return;
     Hit chit = load_hit_lut(sc, cam.curr, cam.prim_gbuffer_d0[cur], cam.prim_gbuffer_d1[cur], cam, p.x, p.y);
@@ -831,7 +879,9 @@ ST_DEV void gi_resolving_px(const CameraDev& cam, const Hit& hit, const GiRes& r
     cam.gi_spec_samples[i] = f4(radiance * spec, confidence);
     gi_store(gi_load(in, idx), cam.gi_reservoirs[0], idx);
 }
-__global__ void ST_LB_GI_RESOLVING k_gi_resolving(KPARAMS, int cur, const float4* __restrict__ in) {
+template <bool BATCHED>
+__global__ void ST_LB_GI_RESOLVING k_gi_resolving(VPARAMS, int cur, const float4* __restrict__ in) {
+    VIEW; VIEW_ARENA(in);
     Px p = pixel_full(cam);
     if (!p.in) return;
     Hit hit = load_hit_lut(sc, cam.curr, cam.prim_gbuffer_d0[cur], cam.prim_gbuffer_d1[cur], cam, p.x, p.y);
@@ -840,7 +890,9 @@ __global__ void ST_LB_GI_RESOLVING k_gi_resolving(KPARAMS, int cur, const float4
 // second preview pass + K19 in one launch (ST_OPT_FUSED_PASSES): the pass's result is shaded straight away instead of going through
 // gi_reservoirs[0] (K19 only consumes fields that a store / load leaves untouched); where the pass exits without writing (quirk C-6) K19
 // sees last frame's entry, which is what is loaded here then.
-__global__ void ST_LB_GI_PREVIEW k_gi_preview_resolve(KPARAMS, int cur, u32 seed, const float4* __restrict__ in, const float4* __restrict__ source) {
+template <bool BATCHED>
+__global__ void ST_LB_GI_PREVIEW k_gi_preview_resolve(VPARAMS, int cur, u32 seed, const float4* __restrict__ in, const float4* __restrict__ source) {
+    VIEW; VIEW_ARENA(in); VIEW_ARENA(source);
     Px p = pixel_full(cam);
     if (!p.in) return;
     Hit chit = load_hit_lut(sc, cam.curr, cam.prim_gbuffer_d0[cur], cam.prim_gbuffer_d1[cur], cam, p.x, p.y);
@@ -851,8 +903,10 @@ __global__ void ST_LB_GI_PREVIEW k_gi_preview_resolve(KPARAMS, int cur, u32 seed
 
 #if ST_EXACT_ONLY
 // K20 frame_denoising::reproject (frame_denoising.rs:4-78)
-__global__ void __launch_bounds__(ST_BLOCK) k_denoise_reproject(KPARAMS, int cur, const float4* __restrict__ prev_colors, const float4* __restrict__ prev_moments,
+template <bool BATCHED>
+__global__ void __launch_bounds__(ST_BLOCK) k_denoise_reproject(VPARAMS, int cur, const float4* __restrict__ prev_colors, const float4* __restrict__ prev_moments,
                                                                 const float4* __restrict__ samples, float4* __restrict__ colors, float4* __restrict__ moments) {
+    VIEW; VIEW_ARENA(prev_colors); VIEW_ARENA(prev_moments); VIEW_ARENA(samples); VIEW_ARENA(colors); VIEW_ARENA(moments);
     Px p = pixel_full(cam);
     if (!p.in) return;
     size_t i = pix(cam, p.x, p.y);
@@ -890,9 +944,7 @@ ST_DEV void denoise_reproject_signal(const CameraDev& cam, size_t i, u32 y, floa
     store4m(cam, g.colors + i, f4(color, 0.0f), y, ST_REACH_SVGF);
     store4m(cam, g.moments + i, f4(moment, 0.0f), y, ST_REACH_SVGF);
 }
-__global__ void __launch_bounds__(ST_BLOCK) k_denoise_reproject_pair(KPARAMS, int cur, const __grid_constant__ ReprojectSignal di, const __grid_constant__ ReprojectSignal gi) {
-    Px p = pixel_full(cam);
-    if (!p.in) return;
+ST_DEV void denoise_reproject_pair_px(const CameraDev& cam, int cur, Px p, const ReprojectSignal& di, const ReprojectSignal& gi) {
     size_t i = pix(cam, p.x, p.y);
     float4 sd = di.samples[i], sg = gi.samples[i];
     if (cam.prim_surface_map[cur][i].z == 0.0f) { store4m(cam, di.colors + i, sd, p.y, ST_REACH_SVGF); store4m(cam, gi.colors + i, sg, p.y, ST_REACH_SVGF); return; }
@@ -900,6 +952,17 @@ __global__ void __launch_bounds__(ST_BLOCK) k_denoise_reproject_pair(KPARAMS, in
     bool has_rp = reproj_some(rp);
     denoise_reproject_signal(cam, i, p.y, sd, rp, has_rp, di);
     denoise_reproject_signal(cam, i, p.y, sg, rp, has_rp, gi);
+}
+ST_DEV ReprojectSignal signal_in_view(const ReprojectSignal& g, const ViewDev& v) {
+    return {arena_ptr<true>(g.prev_colors, v), arena_ptr<true>(g.prev_moments, v), arena_ptr<true>(g.samples, v), arena_ptr<true>(g.colors, v), arena_ptr<true>(g.moments, v)};
+}
+template <bool BATCHED>
+__global__ void __launch_bounds__(ST_BLOCK) k_denoise_reproject_pair(VPARAMS, int cur, const __grid_constant__ ReprojectSignal di, const __grid_constant__ ReprojectSignal gi) {
+    VIEW;
+    Px p = pixel_full(cam);
+    if (!p.in) return;
+    if (BATCHED) denoise_reproject_pair_px(cam, cur, p, signal_in_view(di, view), signal_in_view(gi, view));
+    else denoise_reproject_pair_px(cam, cur, p, di, gi);
 }
 
 // frame_denoising::sample_weight (frame_denoising.rs:363-392), split into the part that is common to
@@ -934,8 +997,9 @@ template <bool FAST> ST_DEV float svgf_luma_weight(float sqrt_center_luma, float
 }
 
 // K21 frame_denoising::estimate_variance (frame_denoising.rs:81-217)
-template <bool FAST>
-__global__ void __launch_bounds__(ST_BLOCK) k_denoise_variance(KPARAMS, int cur) {
+template <bool BATCHED, bool FAST>
+__global__ void __launch_bounds__(ST_BLOCK) k_denoise_variance(VPARAMS, int cur) {
+    VIEW;
     Px p = pixel_full(cam);
     if (!p.in) return;
     size_t i = pix(cam, p.x, p.y);
@@ -988,11 +1052,13 @@ __global__ void __launch_bounds__(ST_BLOCK) k_denoise_variance(KPARAMS, int cur)
 // PAIR_IN: the two signals arrive interleaved, {DI, GI} = one 32-byte record per pixel (`pair_in`, written by the previous iteration
 // through `pair_out`), so that a jittered tap of the wide strides is one full sector and one 256-bit load instead of two half-used
 // sectors; `pair_out` != nullptr writes that layout.  Values and arithmetic are those of the planar layout.
-template <bool FAST, bool PAIR_IN>
-__global__ void __launch_bounds__(ST_BLOCK, ST_WAVELET_MIN_BLOCKS) k_denoise_wavelet(KPARAMS, int cur, u32 frame, u32 stride, float strength,
+template <bool BATCHED, bool FAST, bool PAIR_IN>
+__global__ void __launch_bounds__(ST_BLOCK, ST_WAVELET_MIN_BLOCKS) k_denoise_wavelet(VPARAMS, int cur, u32 frame, u32 stride, float strength,
                                                               const float4* __restrict__ di_in, float4* __restrict__ di_out,
                                                               const float4* __restrict__ gi_in, float4* __restrict__ gi_out,
                                                               const float4* __restrict__ pair_in, float4* __restrict__ pair_out) {
+    VIEW; VIEW_ARENA(di_in); VIEW_ARENA(di_out); VIEW_ARENA(gi_in); VIEW_ARENA(gi_out);
+    pair_in = pair_ptr<BATCHED>(pair_in, view); pair_out = pair_ptr<BATCHED>(pair_out, view);
     Px p = pixel_full(cam);
     if (!p.in) return;
     size_t i = pix(cam, p.x, p.y);
@@ -1204,7 +1270,9 @@ __global__ void __launch_bounds__(TW * TH, (TW * TH <= 256 && S <= 8) ? ST_WAVEL
 }
 
 // R2 frame_composition::fs (frame_composition.rs:19-82), linear HDR out
-__global__ void __launch_bounds__(ST_BLOCK) k_composition(KPARAMS, int cur, u32 mode, const float4* __restrict__ di_diff, const float4* __restrict__ gi_diff) {
+template <bool BATCHED>
+__global__ void __launch_bounds__(ST_BLOCK) k_composition(VPARAMS, int cur, u32 mode, const float4* __restrict__ di_diff, const float4* __restrict__ gi_diff) {
+    VIEW; VIEW_ARENA(di_diff); VIEW_ARENA(gi_diff);
     Px p = pixel_full(cam);
     if (!p.in) return;
     size_t i = pix(cam, p.x, p.y);
@@ -1237,8 +1305,10 @@ ST_DEV u32 srgb8_encode(float v) {
 // dst + y * pitch + x * bytes per pixel, one aligned store per pixel; nothing else of the surface is touched (LoadOp::Load).
 // RGBA32F copies `output`; RGBA16F converts each channel with round-to-nearest-even (what a store to an Rgba16Float target does),
 // alpha 1.0; RGBA8 is the sRGB encode above.
-template <int FMT>
-__global__ void __launch_bounds__(ST_BLOCK) k_output_store(KPARAMS, char* __restrict__ dst, size_t pitch) {
+template <bool BATCHED, int FMT>
+__global__ void __launch_bounds__(ST_BLOCK) k_output_store(VPARAMS) {
+    VIEW;
+    char* __restrict__ dst = view.dst; const size_t pitch = view.pitch;
     Px p = pixel_full(cam);
     if (!p.in) return;
     float4 c = cam.output[pix(cam, p.x, p.y)];
@@ -1254,7 +1324,9 @@ __global__ void __launch_bounds__(ST_BLOCK) k_output_store(KPARAMS, char* __rest
 }
 
 // K1 ref_tracing::main (ref_tracing.rs:4-60)
-__global__ void __launch_bounds__(ST_BLOCK) k_ref_tracing(KPARAMS, u32 depth) {
+template <bool BATCHED>
+__global__ void __launch_bounds__(ST_BLOCK) k_ref_tracing(VPARAMS, u32 depth) {
+    VIEW;
     ST_TRACE_STACK();
     Px p = pixel_full(cam);
     if (!p.in) return;
@@ -1272,7 +1344,9 @@ __global__ void __launch_bounds__(ST_BLOCK) k_ref_tracing(KPARAMS, u32 depth) {
 }
 
 // K2 ref_shading::main (ref_shading.rs:4-177)
-__global__ void __launch_bounds__(ST_BLOCK) k_ref_shading(KPARAMS, u32 seed, u32 depth) {
+template <bool BATCHED>
+__global__ void __launch_bounds__(ST_BLOCK) k_ref_shading(VPARAMS, u32 seed, u32 depth) {
+    VIEW;
     ST_TRACE_STACK();
     Px p = pixel_full(cam);
     if (!p.in) return;
@@ -1322,7 +1396,9 @@ __global__ void __launch_bounds__(ST_BLOCK) k_ref_shading(KPARAMS, u32 seed, u32
 }
 
 // K3 bvh_heatmap::main (bvh_heatmap.rs:4-77)
-__global__ void __launch_bounds__(ST_BLOCK) k_bvh_heatmap(KPARAMS) {
+template <bool BATCHED>
+__global__ void __launch_bounds__(ST_BLOCK) k_bvh_heatmap(VPARAMS) {
+    VIEW;
     ST_TRACE_STACK();
     Px p = pixel_full(cam);
     if (!p.in) return;
@@ -1549,42 +1625,56 @@ __global__ void k_atm_sky(const float4* __restrict__ tl, const float4* __restric
 // ---------------------------------------------------------------------------------------------
 static dim3 grid_full(const CameraDev& cam) { return dim3((cam.w + TILE_W - 1) / TILE_W, (cam.y1 - cam.y0 + TILE_H - 1) / TILE_H); }
 static dim3 grid_half(const CameraDev& cam) { int hw = 8 * (((cam.w + 7) / 8) / 2); return dim3((hw + TILE_W - 1) / TILE_W, (cam.y1 - cam.y0 + TILE_H - 1) / TILE_H); }
-#define HALF_LAUNCH(kernel, c, st, ...) do { dim3 g_ = grid_half(c); if (g_.x > 0 && g_.y > 0) kernel<<<g_, ST_BLOCK, 0, st>>>(__VA_ARGS__); } while (0)
+// One launch over the views of `v` (blockIdx.z = view): the single-camera instantiation `one` for one view, the batched `many` otherwise.
+template <class K1, class K2, class... A>
+static void vlaunch(K1 one, K2 many, dim3 g, const ViewSet& v, cudaStream_t st, const A&... args) {
+    if (g.x == 0 || g.y == 0) return;
+    g.z = (unsigned)v.size();
+    if (v.size() == 1) { ViewBatch<false> b; b.v[0] = v[0]; one<<<g, ST_BLOCK, 0, st>>>(b, args...); return; }
+    ViewBatch<true> b;
+    std::copy(v.begin(), v.end(), b.v);
+    many<<<g, ST_BLOCK, 0, st>>>(b, args...);
+}
+#define FULL_LAUNCH(kernel, v, st, ...) vlaunch(kernel<false>, kernel<true>, grid_full(v[0].cam), v, st, __VA_ARGS__)
+#define HALF_LAUNCH(kernel, v, st, ...) vlaunch(kernel<false>, kernel<true>, grid_half(v[0].cam), v, st, __VA_ARGS__)
 
-void launch_di_sampling(const CameraDev& c, const SceneDev& s, int cur, u32 seed, u32 frame, cudaStream_t st) { k_di_sampling<<<grid_full(c), ST_BLOCK, 0, st>>>(c, s, cur, seed, frame); }
-void launch_di_temporal(const CameraDev& c, const SceneDev& s, int cur, u32 seed, cudaStream_t st) { k_di_temporal<<<grid_full(c), ST_BLOCK, 0, st>>>(c, s, cur, seed); }
-void launch_di_spatial_pick(const CameraDev& c, const SceneDev& s, int cur, u32 seed, u32 frame, cudaStream_t st) { HALF_LAUNCH(k_di_spatial_pick, c, st, c, s, cur, seed, frame); }
-void launch_spatial_trace(const CameraDev& c, const SceneDev& s, const float4* d0, const float4* d1, float4* d2, cudaStream_t st) { k_spatial_trace<<<grid_full(c), ST_BLOCK, 0, st>>>(c, s, d0, d1, d2); }
-void launch_di_spatial_sample(const CameraDev& c, const SceneDev& s, u32 seed, u32 frame, cudaStream_t st) { HALF_LAUNCH(k_di_spatial_sample, c, st, c, s, seed, frame); }
-void launch_di_resolving(const CameraDev& c, const SceneDev& s, int cur, cudaStream_t st) { k_di_resolving<<<grid_full(c), ST_BLOCK, 0, st>>>(c, s, cur); }
-void launch_gi_reprojection(const CameraDev& c, const SceneDev& s, int cur, cudaStream_t st) { k_gi_reprojection<<<grid_full(c), ST_BLOCK, 0, st>>>(c, s, cur); }
-void launch_gi_sampling_a(const CameraDev& c, const SceneDev& s, int cur, u32 seed, u32 frame, cudaStream_t st) { HALF_LAUNCH(k_gi_sampling_a, c, st, c, s, cur, seed, frame); }
-void launch_gi_sampling_b(const CameraDev& c, const SceneDev& s, int cur, u32 seed, u32 frame, cudaStream_t st) { HALF_LAUNCH(k_gi_sampling_b, c, st, c, s, cur, seed, frame); }
-void launch_gi_temporal(const CameraDev& c, const SceneDev& s, int cur, u32 seed, u32 frame, int inline_reprojection, cudaStream_t st) { k_gi_temporal<<<grid_full(c), ST_BLOCK, 0, st>>>(c, s, cur, seed, frame, inline_reprojection); }
-void launch_gi_spatial_pick(const CameraDev& c, const SceneDev& s, int cur, u32 seed, u32 frame, cudaStream_t st) { HALF_LAUNCH(k_gi_spatial_pick, c, st, c, s, cur, seed, frame); }
-void launch_gi_spatial_sample(const CameraDev& c, const SceneDev& s, u32 seed, u32 frame, cudaStream_t st) { HALF_LAUNCH(k_gi_spatial_sample, c, st, c, s, seed, frame); }
-void launch_gi_preview(const CameraDev& c, const SceneDev& s, int cur, u32 seed, u32 nth, const float4* in, float4* out, int mirror_reach, cudaStream_t st) { k_gi_preview<<<grid_full(c), ST_BLOCK, 0, st>>>(c, s, cur, seed, nth, in, out, mirror_reach); }
-void launch_gi_resolving(const CameraDev& c, const SceneDev& s, int cur, const float4* in, cudaStream_t st) { k_gi_resolving<<<grid_full(c), ST_BLOCK, 0, st>>>(c, s, cur, in); }
-void launch_di_sample_temporal(const CameraDev& c, const SceneDev& s, int cur, u32 seed_sampling, u32 seed_temporal, u32 frame, cudaStream_t st) { k_di_sample_temporal<<<grid_full(c), ST_BLOCK, 0, st>>>(c, s, cur, seed_sampling, seed_temporal, frame); }
-void launch_di_spatial_fused(const CameraDev& c, const SceneDev& s, int cur, u32 seed_pick, u32 seed_sample, u32 frame, cudaStream_t st) { HALF_LAUNCH(k_di_spatial_fused, c, st, c, s, cur, seed_pick, seed_sample, frame); }
-void launch_gi_sampling_fused(const CameraDev& c, const SceneDev& s, int cur, u32 seed_a, u32 seed_b, u32 frame, cudaStream_t st) { HALF_LAUNCH(k_gi_sampling_fused, c, st, c, s, cur, seed_a, seed_b, frame); }
-void launch_gi_spatial_fused(const CameraDev& c, const SceneDev& s, int cur, u32 seed_pick, u32 seed_sample, u32 frame, cudaStream_t st) { HALF_LAUNCH(k_gi_spatial_fused, c, st, c, s, cur, seed_pick, seed_sample, frame); }
-void launch_gi_preview_resolve(const CameraDev& c, const SceneDev& s, int cur, u32 seed, const float4* in, const float4* source, cudaStream_t st) { k_gi_preview_resolve<<<grid_full(c), ST_BLOCK, 0, st>>>(c, s, cur, seed, in, source); }
+void launch_di_sampling(const ViewSet& v, const SceneDev& s, int cur, u32 seed, u32 frame, cudaStream_t st) { FULL_LAUNCH(k_di_sampling, v, st, s, cur, seed, frame); }
+void launch_di_temporal(const ViewSet& v, const SceneDev& s, int cur, u32 seed, cudaStream_t st) { FULL_LAUNCH(k_di_temporal, v, st, s, cur, seed); }
+void launch_di_spatial_pick(const ViewSet& v, const SceneDev& s, int cur, u32 seed, u32 frame, cudaStream_t st) { HALF_LAUNCH(k_di_spatial_pick, v, st, s, cur, seed, frame); }
+void launch_spatial_trace(const ViewSet& v, const SceneDev& s, const float4* d0, const float4* d1, float4* d2, cudaStream_t st) { FULL_LAUNCH(k_spatial_trace, v, st, s, d0, d1, d2); }
+void launch_di_spatial_sample(const ViewSet& v, const SceneDev& s, u32 seed, u32 frame, cudaStream_t st) { HALF_LAUNCH(k_di_spatial_sample, v, st, s, seed, frame); }
+void launch_di_resolving(const ViewSet& v, const SceneDev& s, int cur, cudaStream_t st) { FULL_LAUNCH(k_di_resolving, v, st, s, cur); }
+void launch_gi_reprojection(const ViewSet& v, const SceneDev& s, int cur, cudaStream_t st) { FULL_LAUNCH(k_gi_reprojection, v, st, s, cur); }
+void launch_gi_sampling_a(const ViewSet& v, const SceneDev& s, int cur, u32 seed, u32 frame, cudaStream_t st) { HALF_LAUNCH(k_gi_sampling_a, v, st, s, cur, seed, frame); }
+void launch_gi_sampling_b(const ViewSet& v, const SceneDev& s, int cur, u32 seed, u32 frame, cudaStream_t st) { HALF_LAUNCH(k_gi_sampling_b, v, st, s, cur, seed, frame); }
+void launch_gi_temporal(const ViewSet& v, const SceneDev& s, int cur, u32 seed, u32 frame, int inline_reprojection, cudaStream_t st) { FULL_LAUNCH(k_gi_temporal, v, st, s, cur, seed, frame, inline_reprojection); }
+void launch_gi_spatial_pick(const ViewSet& v, const SceneDev& s, int cur, u32 seed, u32 frame, cudaStream_t st) { HALF_LAUNCH(k_gi_spatial_pick, v, st, s, cur, seed, frame); }
+void launch_gi_spatial_sample(const ViewSet& v, const SceneDev& s, u32 seed, u32 frame, cudaStream_t st) { HALF_LAUNCH(k_gi_spatial_sample, v, st, s, seed, frame); }
+void launch_gi_preview(const ViewSet& v, const SceneDev& s, int cur, u32 seed, u32 nth, const float4* in, float4* out, int mirror_reach, cudaStream_t st) { FULL_LAUNCH(k_gi_preview, v, st, s, cur, seed, nth, in, out, mirror_reach); }
+void launch_gi_resolving(const ViewSet& v, const SceneDev& s, int cur, const float4* in, cudaStream_t st) { FULL_LAUNCH(k_gi_resolving, v, st, s, cur, in); }
+void launch_di_sample_temporal(const ViewSet& v, const SceneDev& s, int cur, u32 seed_sampling, u32 seed_temporal, u32 frame, cudaStream_t st) { FULL_LAUNCH(k_di_sample_temporal, v, st, s, cur, seed_sampling, seed_temporal, frame); }
+void launch_di_spatial_fused(const ViewSet& v, const SceneDev& s, int cur, u32 seed_pick, u32 seed_sample, u32 frame, cudaStream_t st) { HALF_LAUNCH(k_di_spatial_fused, v, st, s, cur, seed_pick, seed_sample, frame); }
+void launch_gi_sampling_fused(const ViewSet& v, const SceneDev& s, int cur, u32 seed_a, u32 seed_b, u32 frame, cudaStream_t st) { HALF_LAUNCH(k_gi_sampling_fused, v, st, s, cur, seed_a, seed_b, frame); }
+void launch_gi_spatial_fused(const ViewSet& v, const SceneDev& s, int cur, u32 seed_pick, u32 seed_sample, u32 frame, cudaStream_t st) { HALF_LAUNCH(k_gi_spatial_fused, v, st, s, cur, seed_pick, seed_sample, frame); }
+void launch_gi_preview_resolve(const ViewSet& v, const SceneDev& s, int cur, u32 seed, const float4* in, const float4* source, cudaStream_t st) { FULL_LAUNCH(k_gi_preview_resolve, v, st, s, cur, seed, in, source); }
 #if ST_EXACT_ONLY
-void launch_prim_gbuffer(const CameraDev& c, const SceneDev& s, int cur, int with_reprojection, cudaStream_t st) { k_prim_gbuffer<<<grid_full(c), ST_BLOCK, 0, st>>>(c, s, cur, with_reprojection); }
-void launch_frame_reprojection(const CameraDev& c, const SceneDev& s, int cur, cudaStream_t st) { k_frame_reprojection<<<grid_full(c), ST_BLOCK, 0, st>>>(c, s, cur); }
-void launch_denoise_reproject(const CameraDev& c, const SceneDev& s, int cur, const float4* pc, const float4* pm, const float4* smp, float4* col, float4* mom, cudaStream_t st) { k_denoise_reproject<<<grid_full(c), ST_BLOCK, 0, st>>>(c, s, cur, pc, pm, smp, col, mom); }
-void launch_denoise_reproject_pair(const CameraDev& c, const SceneDev& s, int cur, cudaStream_t st) {
+void launch_prim_gbuffer(const ViewSet& v, const SceneDev& s, int cur, int with_reprojection, cudaStream_t st) { FULL_LAUNCH(k_prim_gbuffer, v, st, s, cur, with_reprojection); }
+void launch_frame_reprojection(const ViewSet& v, const SceneDev& s, int cur, cudaStream_t st) { FULL_LAUNCH(k_frame_reprojection, v, st, s, cur); }
+void launch_denoise_reproject(const ViewSet& v, const SceneDev& s, int cur, const float4* pc, const float4* pm, const float4* smp, float4* col, float4* mom, cudaStream_t st) { FULL_LAUNCH(k_denoise_reproject, v, st, s, cur, pc, pm, smp, col, mom); }
+void launch_denoise_reproject_pair(const ViewSet& v, const SceneDev& s, int cur, cudaStream_t st) {
+    const CameraDev& c = v[0].cam;
     ReprojectSignal di{c.di_diff_prev_colors, c.di_diff_moments[cur ^ 1], c.di_diff_samples, c.di_diff_curr_colors, c.di_diff_moments[cur]};
     ReprojectSignal gi{c.gi_diff_prev_colors, c.gi_diff_moments[cur ^ 1], c.gi_diff_samples, c.gi_diff_curr_colors, c.gi_diff_moments[cur]};
-    k_denoise_reproject_pair<<<grid_full(c), ST_BLOCK, 0, st>>>(c, s, cur, di, gi);
+    FULL_LAUNCH(k_denoise_reproject_pair, v, st, s, cur, di, gi);
 }
-void launch_denoise_variance(const CameraDev& c, const SceneDev& s, int cur, bool fast, cudaStream_t st) {
-    if (fast) k_denoise_variance<true><<<grid_full(c), ST_BLOCK, 0, st>>>(c, s, cur); else k_denoise_variance<false><<<grid_full(c), ST_BLOCK, 0, st>>>(c, s, cur);
+void launch_denoise_variance(const ViewSet& v, const SceneDev& s, int cur, bool fast, cudaStream_t st) {
+    const dim3 g = grid_full(v[0].cam);
+    if (fast) vlaunch(k_denoise_variance<false, true>, k_denoise_variance<true, true>, g, v, st, s, cur);
+    else vlaunch(k_denoise_variance<false, false>, k_denoise_variance<true, false>, g, v, st, s, cur);
 }
-void launch_denoise_wavelet(const CameraDev& c, const SceneDev& s, int cur, u32 frame, u32 stride, float strength, const float4* di_in, float4* di_out, const float4* gi_in, float4* gi_out,
+void launch_denoise_wavelet(const ViewSet& v, const SceneDev& s, int cur, u32 frame, u32 stride, float strength, const float4* di_in, float4* di_out, const float4* gi_in, float4* gi_out,
                             const float4* pair_in, float4* pair_out, bool fast, cudaStream_t st) {
-#define ST_WG(F_, P_) k_denoise_wavelet<F_, P_><<<grid_full(c), ST_BLOCK, 0, st>>>(c, s, cur, frame, stride, strength, di_in, di_out, gi_in, gi_out, pair_in, pair_out)
+#define ST_WG(F_, P_) vlaunch(k_denoise_wavelet<false, F_, P_>, k_denoise_wavelet<true, F_, P_>, grid_full(v[0].cam), v, st, s, cur, frame, stride, strength, di_in, di_out, gi_in, gi_out, pair_in, pair_out)
     if (pair_in) { if (fast) ST_WG(true, true); else ST_WG(false, true); }
     else { if (fast) ST_WG(true, false); else ST_WG(false, false); }
 #undef ST_WG
@@ -1770,15 +1860,16 @@ bool launch_denoise_variance_tiled(const CameraDev& c, const SceneDev& s, int cu
     if (c.curr.screen.x != (float)c.w || c.curr.screen.y != (float)c.h) return false;   // zero fill == Camera::contains only then
     return fast ? variance_tiled_go<true>(c, s, cur, errors, st) : variance_tiled_go<false>(c, s, cur, errors, st);
 }
-void launch_composition(const CameraDev& c, const SceneDev& s, int cur, u32 mode, const float4* di_diff, const float4* gi_diff, cudaStream_t st) { k_composition<<<grid_full(c), ST_BLOCK, 0, st>>>(c, s, cur, mode, di_diff, gi_diff); }
-void launch_output_store(const CameraDev& c, const SceneDev& s, int format, void* dst, size_t pitch, cudaStream_t st) {
-    if (format == OUT_RGBA32F) k_output_store<OUT_RGBA32F><<<grid_full(c), ST_BLOCK, 0, st>>>(c, s, (char*)dst, pitch);
-    else if (format == OUT_RGBA16F) k_output_store<OUT_RGBA16F><<<grid_full(c), ST_BLOCK, 0, st>>>(c, s, (char*)dst, pitch);
-    else k_output_store<OUT_RGBA8_SRGB><<<grid_full(c), ST_BLOCK, 0, st>>>(c, s, (char*)dst, pitch);
+void launch_composition(const ViewSet& v, const SceneDev& s, int cur, u32 mode, const float4* di_diff, const float4* gi_diff, cudaStream_t st) { FULL_LAUNCH(k_composition, v, st, s, cur, mode, di_diff, gi_diff); }
+void launch_output_store(const ViewSet& v, const SceneDev& s, int format, cudaStream_t st) {
+    const dim3 g = grid_full(v[0].cam);
+    if (format == OUT_RGBA32F) vlaunch(k_output_store<false, OUT_RGBA32F>, k_output_store<true, OUT_RGBA32F>, g, v, st, s);
+    else if (format == OUT_RGBA16F) vlaunch(k_output_store<false, OUT_RGBA16F>, k_output_store<true, OUT_RGBA16F>, g, v, st, s);
+    else vlaunch(k_output_store<false, OUT_RGBA8_SRGB>, k_output_store<true, OUT_RGBA8_SRGB>, g, v, st, s);
 }
-void launch_ref_tracing(const CameraDev& c, const SceneDev& s, u32 depth, cudaStream_t st) { k_ref_tracing<<<grid_full(c), ST_BLOCK, 0, st>>>(c, s, depth); }
-void launch_ref_shading(const CameraDev& c, const SceneDev& s, u32 seed, u32 depth, cudaStream_t st) { k_ref_shading<<<grid_full(c), ST_BLOCK, 0, st>>>(c, s, seed, depth); }
-void launch_bvh_heatmap(const CameraDev& c, const SceneDev& s, cudaStream_t st) { k_bvh_heatmap<<<grid_full(c), ST_BLOCK, 0, st>>>(c, s); }
+void launch_ref_tracing(const ViewSet& v, const SceneDev& s, u32 depth, cudaStream_t st) { FULL_LAUNCH(k_ref_tracing, v, st, s, depth); }
+void launch_ref_shading(const ViewSet& v, const SceneDev& s, u32 seed, u32 depth, cudaStream_t st) { FULL_LAUNCH(k_ref_shading, v, st, s, seed, depth); }
+void launch_bvh_heatmap(const ViewSet& v, const SceneDev& s, cudaStream_t st) { FULL_LAUNCH(k_bvh_heatmap, v, st, s); }
 void launch_trace_stream_closest(const SceneDev& s, const float4* rays, long n, float4* out, cudaStream_t st) { k_trace_stream_closest<<<(unsigned)((n + ST_BLOCK - 1) / ST_BLOCK), ST_BLOCK, 0, st>>>(s, rays, n, out); }
 void launch_trace_stream_any(const SceneDev& s, const float4* rays, long n, u32* out, cudaStream_t st) { k_trace_stream_any<<<(unsigned)((n + ST_BLOCK - 1) / ST_BLOCK), ST_BLOCK, 0, st>>>(s, rays, n, out); }
 void launch_math(int op, const float* a, const float* b, float* out, long n, cudaStream_t st) { k_math<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(op, a, b, out, n); }
@@ -1924,7 +2015,7 @@ int preload_kernels() {
     cudaGetLastError();
     if (!get_module || !get_count || !enumerate || !load) return state = 1;
     cudaFunction_t anchor = nullptr;
-    if (cudaGetFuncBySymbol(&anchor, (const void*)k_di_sample_temporal) != cudaSuccess) { cudaGetLastError(); return state = 2; }
+    if (cudaGetFuncBySymbol(&anchor, (const void*)k_di_sample_temporal<false>) != cudaSuccess) { cudaGetLastError(); return state = 2; }
     CUmodule mod = nullptr; unsigned int n = 0;
     if (get_module(&mod, (CUfunction)anchor) != CUDA_SUCCESS || get_count(&n, mod) != CUDA_SUCCESS || n == 0u) return state = 3;
     std::vector<CUfunction> fns(n);

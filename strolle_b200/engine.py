@@ -90,6 +90,7 @@ def load_library():
         "st_create_camera": [P, C.POINTER(_Camera), C.POINTER(i32)], "st_update_camera": [P, i32, C.POINTER(_Camera)], "st_delete_camera": [P, i32],
         "st_tick": [P], "st_render_camera": [P, i32, P, C.c_int], "st_copy_output": [P, i32, P, C.c_int], "st_synchronize": [P],
         "st_render_camera_to": [P, i32, P, C.c_size_t, C.c_int], "st_multi_render_camera_to": [P, i32, P, C.c_size_t, C.c_int],
+        "st_render_cameras": [P, C.POINTER(i32), C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_int],
         "st_set_seed_base": [P, u32], "st_set_blue_noise": [P, C.c_void_p],
         "st_read_buffer": [P, i32, C.c_char_p, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)],
         "st_read_scene": [P, C.c_char_p, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)],
@@ -367,6 +368,28 @@ class Engine:
         _Surface(out, fmt, self._cams.get(cam)).render(lambda p: self._check(self.lib.st_render_camera(self._h, cam, p, fmt)),
                                                        lambda p, pitch: self._check(self.lib.st_render_camera_to(self._h, cam, p, pitch, fmt)),
                                                        self.synchronize)
+
+    def render_cameras(self, cams, outs=None, fmt=FORMAT_RGBA32F):
+        """Renders the cameras `cams` for this frame; cameras of one size, mode, denoise and ref_depth run as one launch per pass.  Each
+        camera's buffers and output are bit for bit what `render_camera` gives when called for the cameras one after another.  `outs`:
+        None, or one entry per camera, each None (no output) or a surface as `render_camera`'s `out`, in format `fmt`.  CUDA surfaces
+        hold their frames when this returns."""
+        cams = [int(c) for c in cams]
+        n = len(cams)
+        if outs is not None and len(outs) != n:
+            raise ValueError(f"{n} cameras but {len(outs)} output surfaces")
+        surfaces = [None if o is None else _Surface(o, fmt, self._cams.get(c)) for c, o in zip(cams, outs or [None] * n)]
+        handles = (C.c_int32 * max(n, 1))(*cams)
+        dsts = (C.c_void_p * max(n, 1))(*[s.ptr if s is not None else None for s in surfaces])
+        pitches = (C.c_size_t * max(n, 1))(*[s.pitch if s is not None else 0 for s in surfaces])
+        cuda = [s for s in surfaces if s is not None and s.cuda]
+        if cuda:
+            import torch
+            for d in {s.device for s in cuda}:
+                torch.cuda.current_stream(d).synchronize()
+        self._check(self.lib.st_render_cameras(self._h, handles, n, dsts if outs is not None else None, pitches, fmt))
+        if cuda:
+            self.synchronize()
 
     def render_camera_to(self, cam, ptr, pitch_bytes, fmt):
         """st_render_camera_to on a raw address (pixel (0, 0) of the camera inside the surface); returns once enqueued for device memory."""
