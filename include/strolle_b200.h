@@ -102,6 +102,20 @@ int st_remove_material(st_engine* e, st_handle material);
  * (the reference warns and drops the image, images.rs:71-79). */
 int st_insert_image(st_engine* e, st_handle image, const uint8_t* rgba8, uint32_t width, uint32_t height);
 int st_remove_image(st_engine* e, st_handle image);
+/* ImageData::Texture { is_dynamic: true } (strolle/src/images.rs:97-102): an image whose texels live in a caller-owned surface of width x height
+ * RGBA8 texels in the atlas format Rgba8UnormSrgb (what a camera renders with ST_FORMAT_RGBA8_SRGB), rows `pitch_bytes` apart (0 = packed).
+ * The image gets its atlas rectangle as st_insert_image would place it (a handle that has one of the same size keeps it); this call copies
+ * nothing.  Each st_tick then copies every dynamic image's surface into its rectangle (Images::flush, images.rs:189-214), enqueued on the
+ * engine's stream before anything else the tick enqueues, and after every write this engine has queued to the surface (its kernel stores,
+ * its output copies under ST_OPT_ASYNC_OUTPUT, and in a strip group every member's rows); writes from other streams are the caller's to
+ * order.  So every camera rendered after a tick sees the same snapshot, and a frame a camera writes into the surface is seen by the
+ * cameras of the next frame.  `src` may be memory of this engine's device, of a device it can reach by peer access, managed memory, or
+ * page-locked host memory (read through its device pointer); it must stay valid while the image is dynamic.  st_remove_image,
+ * st_insert_image on the same handle, or st_insert_dynamic_image with another surface end the refresh, and synchronise the engine's
+ * stream before returning, so the old surface may be freed then.  ST_ERR_INVALID for a NULL src, a zero size, a pitch below 4 * width, an
+ * address or pitch not a multiple of 4, pageable host memory, or device memory this device cannot reach; ST_ERR_LIMIT when the atlas is
+ * full.  A refused call changes nothing: an image already on the handle keeps its rectangle, its texels and its refresh. */
+int st_insert_dynamic_image(st_engine* e, st_handle image, const void* src, size_t pitch_bytes, uint32_t width, uint32_t height);
 /* The Option<ImageHandle> fields of strolle::Material (strolle/src/material.rs:13-22); bit i of `mask` = texture i set
  * (0 base_color, 1 emissive, 2 metallic_roughness, 3 normal_map — the last is carried but unused, as in the reference). */
 typedef struct st_material_textures { st_handle base_color, emissive, metallic_roughness, normal_map; uint32_t mask; } st_material_textures;
@@ -172,6 +186,9 @@ int st_read_buffer(st_engine* e, st_camera_handle camera, const char* name, floa
 /* Scene buffers as uploaded: "triangles", "bvh", "materials", "lights", "world", "transmittance_lut",
  * "scattering_lut", "sky_lut". */
 int st_read_scene(st_engine* e, const char* name, float* dst, size_t cap_floats, size_t* count);
+/* An image's atlas rectangle (static or dynamic), tightly packed RGBA8, after the work queued on the engine's stream: *bytes = width *
+ * height * 4; with dst == NULL only the size is returned, cap_bytes below it is ST_ERR_LIMIT.  ST_ERR_NOT_FOUND for an unknown image. */
+int st_read_image(st_engine* e, st_handle image, uint8_t* dst, size_t cap_bytes, size_t* bytes);
 int st_bvh_depth(st_engine* e, int* depth);
 uint32_t st_frame(st_engine* e);
 /* Sets the id of the frame the next st_tick prepares (ids start at 1, strolle/src/lib.rs:152).  Used by the
@@ -346,6 +363,9 @@ int st_multi_has_material(st_multi* m, st_handle material);
 int st_multi_remove_material(st_multi* m, st_handle material);
 int st_multi_insert_image(st_multi* m, st_handle image, const uint8_t* rgba8, uint32_t width, uint32_t height);
 int st_multi_remove_image(st_multi* m, st_handle image);
+/* st_insert_dynamic_image for the group: every member refreshes its own atlas from the same surface, which must be reachable from every
+ * member's device (or be page-locked host memory); otherwise it is refused with nothing registered on any member. */
+int st_multi_insert_dynamic_image(st_multi* m, st_handle image, const void* src, size_t pitch_bytes, uint32_t width, uint32_t height);
 int st_multi_set_material_textures(st_multi* m, st_handle material, const st_material_textures* textures);
 int st_multi_insert_instance(st_multi* m, st_handle instance, st_handle mesh, st_handle material, const float affine[12]);
 int st_multi_remove_instance(st_multi* m, st_handle instance);

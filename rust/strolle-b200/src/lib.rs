@@ -10,8 +10,9 @@
 //!   wgpu command encoder — the CUDA kernels run on the engine's own stream.  A wgpu host uploads it with `Queue::write_texture`
 //!   (what `bevy-strolle-b200` does); `render_camera_to_raw` composes straight into a caller-owned surface in device or host memory
 //!   with a row pitch (e.g. a texture imported through CUDA external memory).
-//! * `ImageData::Texture` (a live wgpu texture) cannot be sampled from CUDA; dynamic images are passed as `ImageData::Raw` each time
-//!   they change.
+//! * `ImageData::Texture` (a live wgpu texture) cannot be sampled from CUDA.  Its dynamic case, a texture that the atlas copies at every
+//!   tick, is `insert_dynamic_image_raw` over a CUDA address instead (device, managed or page-locked host memory, e.g. another camera's
+//!   `render_camera_to_raw` target); a static texture is passed as `ImageData::Raw`.
 //! * Misuse returns `Err(Error)` where the reference panics (`triangles.rs:44-53`, `camera_controllers.rs:21-25`); the infallible
 //!   scene verbs log the error and carry on like the reference's `warn!` paths (`images.rs:71-79`).
 use std::collections::HashMap;
@@ -494,6 +495,22 @@ impl<P: Params> Engine<P> {
             return;
         }
         soft("insert_image", unsafe { sys::st_multi_insert_image(self.raw, id, data.as_ptr(), image.size.x, image.size.y) });
+    }
+
+    /// Creates or updates a dynamic image (`ImageData::Texture { is_dynamic: true }`, `images.rs:97-102`): its texels live in a
+    /// caller-owned surface of `size.x * size.y` Rgba8UnormSrgb texels, rows `pitch_bytes` apart (0 = packed), which every
+    /// [`Self::tick`] copies into the image's atlas rectangle before the tick's other work, and after the writes the engine itself queued
+    /// to it.  A camera that renders into the surface with [`Self::render_camera_to_raw`] and [`ViewportFormat::Rgba8UnormSrgb`] is
+    /// therefore seen by the other cameras one frame later, as in the reference.  [`Self::remove_image`], [`Self::insert_image`] or
+    /// another call of this on the handle end the refresh; they return once the engine no longer reads the old surface.
+    ///
+    /// # Safety
+    /// `src` must point to device memory every device of the group can reach, managed memory, or page-locked host memory, of at least
+    /// `(size.y - 1) * pitch_bytes + size.x * 4` bytes, valid until the refresh ends.  Writes to it from other CUDA streams must be
+    /// ordered before [`Self::tick`] by the caller.
+    pub unsafe fn insert_dynamic_image_raw(&mut self, handle: P::ImageHandle, src: *const u8, pitch_bytes: usize, size: UVec2) -> Result<(), Error> {
+        let id = self.images.id(handle);
+        check(sys::st_multi_insert_dynamic_image(self.raw, id, src as *const c_void, pitch_bytes, size.x, size.y))
     }
 
     /// Removes an image (`lib.rs:211-214`).

@@ -415,6 +415,12 @@ struct st_engine {
     // materials (Images::lookup) is visible to the kernels
     struct ImageRect { st_handle handle; uint32_t x, y, w, h; };
     std::vector<ImageRect> images; uint32_t shelf_x = 0, shelf_y = 0, shelf_h = 0; bool images_dirty = false;
+    // dynamic images (st_insert_dynamic_image): at each tick, before anything else the tick enqueues, every surface is copied into its image's
+    // rectangle.  `src` = the address this device reads (device, peer, managed, or the device pointer of page-locked host memory).
+    struct DynImage { st_handle handle; const char* src; size_t pitch; };
+    std::vector<DynImage> dynamic;
+    cudaEvent_t ev_output = nullptr;   // recorded on copy_stream: the refresh waits for queued output copies into host surfaces
+    cudaEvent_t ev_queued = nullptr;   // recorded on `stream` by st_multi_tick: the other members' refreshes wait for this member's row stores
     DevMem d_atlas, d_srgb, d_tri_instance, d_instance_xforms;
     bool motion_dirty = true;
     bool moved_last_tick = false;   // an instance was inserted / moved / removed in the tick that prepared the current frame
@@ -1177,6 +1183,8 @@ void st_engine_destroy(st_engine* e) {
     for (DevMem* d : all) d->release();
     for (auto& t : e->pending) { cudaEventDestroy(t.a); cudaEventDestroy(t.b); }
     for (cudaEvent_t ev : e->event_pool) cudaEventDestroy(ev);
+    if (e->ev_output) cudaEventDestroy(e->ev_output);
+    if (e->ev_queued) cudaEventDestroy(e->ev_queued);
     if (e->comm) g_nccl.CommDestroy(e->comm);
     if (e->own_stream) cudaStreamDestroy(e->stream);
     if (e->copy_stream) cudaStreamDestroy(e->copy_stream);
@@ -1209,9 +1217,11 @@ int st_remove_material(st_engine* e, st_handle h) {
     return ST_OK;
 }
 
-int st_insert_image(st_engine* e, st_handle h, const uint8_t* rgba8, uint32_t w, uint32_t hgt) {   // Images::insert (images.rs:54-104), ImageData::Raw
-    if (!e || !rgba8 || w == 0 || hgt == 0) return fail(ST_ERR_INVALID, "null argument");
-    CK(cudaSetDevice(e->device));
+}  // extern "C"
+namespace st {
+// The atlas rectangle of image `h` for a w x hgt image (Images::insert, images.rs:54-104): a handle that has one of that size keeps it, otherwise
+// the shelf allocator places a new one.  ST_ERR_LIMIT leaves the handle's rectangle as it was.
+static int place_image(st_engine* e, st_handle h, uint32_t w, uint32_t hgt, st_engine::ImageRect** out) {
     int rc;
     if (!e->d_atlas.p) {
         if ((rc = e->d_atlas.ensure((size_t)kAtlasSize * kAtlasSize * 4))) return rc;
@@ -1227,14 +1237,55 @@ int st_insert_image(st_engine* e, st_handle h, const uint8_t* rgba8, uint32_t w,
         e->shelf_x += w; if (hgt > e->shelf_h) e->shelf_h = hgt;
         if (r) *r = nr; else { e->images.push_back(nr); r = &e->images.back(); }
     }
+    *out = r;
+    return ST_OK;
+}
+// Ends the refresh of image `h`; true if it was dynamic.  The caller then synchronises the stream, so that the old surface may be freed.
+static bool drop_dynamic(st_engine* e, st_handle h) {
+    const size_t before = e->dynamic.size();
+    e->dynamic.erase(std::remove_if(e->dynamic.begin(), e->dynamic.end(), [&](const st_engine::DynImage& d) { return d.handle == h; }), e->dynamic.end());
+    return e->dynamic.size() != before;
+}
+// Copies every dynamic image's surface into its atlas rectangle: one launch (per kAtlasCopies images) on the engine stream, after the output
+// copies the copy stream has queued (ST_OPT_ASYNC_OUTPUT may still be writing a page-locked source).  Kernel stores into a source were queued
+// on the engine stream itself and come first anyway.
+static int wait_output_copies(st_engine* e) {
+    if (!e->copy_stream) return ST_OK;
+    if (!e->ev_output) CK(cudaEventCreateWithFlags(&e->ev_output, cudaEventDisableTiming));
+    CK(cudaEventRecord(e->ev_output, e->copy_stream));
+    CK(cudaStreamWaitEvent(e->stream, e->ev_output, 0));
+    return ST_OK;
+}
+static int refresh_dynamic_images(st_engine* e) {
+    int rc = wait_output_copies(e); if (rc) return rc;
+    std::vector<AtlasCopy> copies;
+    for (const st_engine::DynImage& d : e->dynamic)
+        for (const st_engine::ImageRect& r : e->images) if (r.handle == d.handle) {
+            AtlasCopy c{}; c.src = d.src; c.pitch = d.pitch; c.x = r.x; c.y = r.y; c.w = r.w; c.h = r.h;
+            copies.push_back(c);
+        }
+    launch_atlas_refresh(copies, (uchar4*)e->d_atlas.p, e->stream);
+    CK(cudaGetLastError());
+    return ST_OK;
+}
+}  // namespace st
+extern "C" {
+
+int st_insert_image(st_engine* e, st_handle h, const uint8_t* rgba8, uint32_t w, uint32_t hgt) {   // Images::insert (images.rs:54-104), ImageData::Raw
+    if (!e || !rgba8 || w == 0 || hgt == 0) return fail(ST_ERR_INVALID, "null argument");
+    CK(cudaSetDevice(e->device));
+    st_engine::ImageRect* r = nullptr;
+    int rc = place_image(e, h, w, hgt, &r); if (rc) return rc;
     CK(cudaMemcpy2DAsync((char*)e->d_atlas.p + 4 * ((size_t)r->y * kAtlasSize + r->x), (size_t)kAtlasSize * 4, rgba8, (size_t)w * 4, (size_t)w * 4, hgt, cudaMemcpyHostToDevice, e->stream));
-    CK(cudaStreamSynchronize(e->stream));   // the caller's pixels may be freed after return
+    CK(cudaStreamSynchronize(e->stream));   // the caller's pixels may be freed after return (and so may a dynamic surface this replaces)
+    drop_dynamic(e, h);
     e->images_dirty = true;
     return ST_OK;
 }
 int st_remove_image(st_engine* e, st_handle h) {   // Images::remove (images.rs:106-112): the rect is released, materials keep their stale rect until re-serialised
     if (!e) return fail(ST_ERR_INVALID, "null engine");
     e->images.erase(std::remove_if(e->images.begin(), e->images.end(), [&](const st_engine::ImageRect& r) { return r.handle == h; }), e->images.end());
+    if (drop_dynamic(e, h)) { CK(cudaSetDevice(e->device)); CK(cudaStreamSynchronize(e->stream)); }   // the surface may be freed after return
     e->images_dirty = true;
     return ST_OK;
 }
@@ -1361,6 +1412,7 @@ int st_tick(st_engine* e) {   // Engine::tick (lib.rs:301-395)
     if (!e) return fail(ST_ERR_INVALID, "null engine");
     CK(cudaSetDevice(e->device));
     int rc; bool too_deep = false;
+    if (!e->dynamic.empty() && (rc = refresh_dynamic_images(e))) return rc;   // Images::flush (images.rs:189-214), lib.rs:311
     if (e->materials_dirty || e->images_dirty) {   // Materials::refresh + Material::serialize (materials.rs:79-85, material.rs:29-50)
         e->materials_dirty = false; e->images_dirty = false;
         auto rect = [&](const st_engine::MatTex& mt, int k) {   // Images::lookup (images.rs:114-127)
@@ -1471,7 +1523,9 @@ int st_render_camera(st_engine* e, st_camera_handle h, void* host_out, int forma
 }
 // Where a frame goes: `dst` = the address of camera pixel (0, 0) inside the caller's surface, rows `pitch` bytes apart.  `device`:
 // memory a kernel on the engine's device stores into (device memory of that device or of a peer, managed memory); otherwise host memory.
-struct OutputTarget { char* dst; size_t pitch; int format; bool device; };
+// `kind`: what cudaPointerGetAttributes found (cudaMemoryTypeUnregistered = pageable host memory); `mapped`: the address a kernel on the
+// engine's device uses for it (null for pageable memory).
+struct OutputTarget { char* dst; size_t pitch; int format; bool device; int kind = cudaMemoryTypeUnregistered; const char* mapped = nullptr; };
 // The full-frame host buffer of st_render_camera / st_copy_output: tightly packed rows.
 static OutputTarget host_frame(const CameraSlot* cs, void* host_out, int format) { return {(char*)host_out, (size_t)cs->desc.width * format_bpp(format), format, false}; }
 // Checks a caller's surface for a `width`-pixel frame and finds what memory it is (cudaPointerGetAttributes).  Device memory of another
@@ -1486,6 +1540,8 @@ static int resolve_target(st_engine* e, uint32_t width, void* dst, size_t pitch,
     cudaPointerAttributes a{};
     if (cudaPointerGetAttributes(&a, dst) != cudaSuccess) { cudaGetLastError(); a.type = cudaMemoryTypeUnregistered; }
     *t = {(char*)dst, pitch, format, a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged};
+    t->kind = a.type;
+    t->mapped = a.type == cudaMemoryTypeHost ? (const char*)a.devicePointer : a.type == cudaMemoryTypeUnregistered ? nullptr : (const char*)dst;
     if (a.type == cudaMemoryTypeDevice && a.device != e->device) {
         int can = 0; CK(cudaDeviceCanAccessPeer(&can, e->device, a.device));
         if (!can) return fail(ST_ERR_INVALID, "the surface is memory of device " + std::to_string(a.device) + ", which device " + std::to_string(e->device) + " cannot reach");
@@ -1609,6 +1665,45 @@ int st_synchronize(st_engine* e) {
     CK(cudaSetDevice(e->device)); CK(cudaStreamSynchronize(e->stream));
     if (e->copy_stream) CK(cudaStreamSynchronize(e->copy_stream));
     for (CameraSlot* c : e->cameras) for (int k = 0; k < 2; k++) if (c->side[k]) CK(cudaStreamSynchronize(c->side[k]));   // copy-engine pushes of strip halos
+    return ST_OK;
+}
+
+// ---- dynamic images (ImageData::Texture { is_dynamic: true }, strolle/src/images.rs:97-102, 189-214) ----------------------------------
+// A w x hgt RGBA8 surface this engine's device can read: resolve_target's checks for an Rgba8UnormSrgb frame of width w, and no pageable memory.
+static int dynamic_source(st_engine* e, const void* src, size_t pitch, uint32_t w, uint32_t hgt, OutputTarget* t) {
+    if (w == 0 || hgt == 0) return fail(ST_ERR_INVALID, "empty image");
+    int rc = resolve_target(e, w, const_cast<void*>(src), pitch, ST_FORMAT_RGBA8_SRGB, t); if (rc) return rc;
+    if (t->kind == cudaMemoryTypeUnregistered || !t->mapped)
+        return fail(ST_ERR_INVALID, "a dynamic image's surface must be device, managed or page-locked host memory (st_insert_image takes pageable pixels)");
+    return ST_OK;
+}
+static int insert_dynamic(st_engine* e, st_handle h, const OutputTarget& t, uint32_t w, uint32_t hgt) {
+    CK(cudaSetDevice(e->device));
+    st_engine::ImageRect* r = nullptr;
+    int rc = place_image(e, h, w, hgt, &r); if (rc) return rc;
+    const bool replaced = drop_dynamic(e, h);
+    e->dynamic.push_back({h, t.mapped, t.pitch ? t.pitch : (size_t)w * 4});
+    e->images_dirty = true;
+    if (replaced) CK(cudaStreamSynchronize(e->stream));   // the previous surface may be freed after return
+    return ST_OK;
+}
+int st_insert_dynamic_image(st_engine* e, st_handle image, const void* src, size_t pitch_bytes, uint32_t width, uint32_t height) {
+    if (!e) return fail(ST_ERR_INVALID, "null engine");
+    CK(cudaSetDevice(e->device));
+    OutputTarget t; int rc = dynamic_source(e, src, pitch_bytes, width, height, &t); if (rc) return rc;
+    return insert_dynamic(e, image, t, width, height);
+}
+int st_read_image(st_engine* e, st_handle image, uint8_t* dst, size_t cap_bytes, size_t* bytes) {
+    if (!e || !bytes) return fail(ST_ERR_INVALID, "null argument");
+    const st_engine::ImageRect* r = nullptr;
+    for (const auto& k : e->images) if (k.handle == image) r = &k;
+    if (!r) return fail(ST_ERR_NOT_FOUND, "unknown image");
+    *bytes = (size_t)r->w * r->h * 4;
+    if (!dst) return ST_OK;
+    if (cap_bytes < *bytes) return fail(ST_ERR_LIMIT, "buffer too small");
+    CK(cudaSetDevice(e->device));
+    CK(cudaStreamSynchronize(e->stream));
+    CK(cudaMemcpy2D(dst, (size_t)r->w * 4, (const char*)e->d_atlas.p + 4 * ((size_t)r->y * kAtlasSize + r->x), (size_t)kAtlasSize * 4, (size_t)r->w * 4, r->h, cudaMemcpyDeviceToHost));
     return ST_OK;
 }
 
@@ -2134,7 +2229,36 @@ int st_multi_update_sun(st_multi* m, float az, float alt) { ST_MULTI_ALL(st_upda
 int st_multi_set_option(st_multi* m, int option, int value) { ST_MULTI_ALL(st_set_option(e, option, value)); }
 int st_multi_set_seed_base(st_multi* m, uint32_t base) { ST_MULTI_ALL(st_set_seed_base(e, base)); }
 int st_multi_set_blue_noise(st_multi* m, const uint8_t* rgba) { ST_MULTI_ALL(st_set_blue_noise(e, rgba)); }
-int st_multi_tick(st_multi* m) { ST_MULTI_ALL(st_tick(e)); }
+int st_multi_insert_dynamic_image(st_multi* m, st_handle h, const void* src, size_t pitch, uint32_t w, uint32_t hgt) {
+    if (!m) return fail(ST_ERR_INVALID, "null group");
+    std::vector<OutputTarget> t(m->e.size());
+    for (size_t i = 0; i < m->e.size(); i++) {   // every member must reach the surface before any of them registers it
+        CK(cudaSetDevice(m->e[i]->device));
+        int rc = dynamic_source(m->e[i], src, pitch, w, hgt, &t[i]); if (rc) return rc;
+    }
+    for (size_t i = 0; i < m->e.size(); i++) { int rc = insert_dynamic(m->e[i], h, t[i], w, hgt); if (rc) return rc; }
+    return ST_OK;
+}
+int st_multi_tick(st_multi* m) {
+    if (!m) return fail(ST_ERR_INVALID, "null group");
+    // Every member stores its own rows of a group camera's frame, so a surface one member refreshes from may hold rows the others wrote: each
+    // member's refresh first waits for everything the other members have queued (their output copies included).
+    bool dynamic = false;
+    for (st_engine* e : m->e) dynamic |= !e->dynamic.empty();
+    if (dynamic && m->e.size() > 1) {
+        for (st_engine* e : m->e) {
+            CK(cudaSetDevice(e->device));
+            if (!e->ev_queued) CK(cudaEventCreateWithFlags(&e->ev_queued, cudaEventDisableTiming));
+            int rc = wait_output_copies(e); if (rc) return rc;
+            CK(cudaEventRecord(e->ev_queued, e->stream));
+        }
+        for (st_engine* e : m->e) {
+            CK(cudaSetDevice(e->device));
+            for (st_engine* o : m->e) if (o != e) CK(cudaStreamWaitEvent(e->stream, o->ev_queued, 0));
+        }
+    }
+    ST_MULTI_ALL(st_tick(e));
+}
 int st_multi_synchronize(st_multi* m) { ST_MULTI_ALL(st_synchronize(e)); }
 int st_multi_create_camera(st_multi* m, const st_camera* c, st_camera_handle* out) {
     if (!m || !c || !out) return fail(ST_ERR_INVALID, "null argument");

@@ -1876,6 +1876,53 @@ void launch_math(int op, const float* a, const float* b, float* out, long n, cud
 void launch_material_derive(const GpuMaterial* mats, u32 n, u32* packed, cudaStream_t st) { if (n) k_material_derive<<<(n + 127) / 128, 128, 0, st>>>(mats, n, packed); }
 void launch_srgb_lut(float* lut, cudaStream_t st) { k_srgb_lut<<<1, 256, 0, st>>>(lut); }
 void launch_unpack_lut(float* lut, cudaStream_t st) { k_unpack_lut<<<1, 256, 0, st>>>(lut); }
+// ---- dynamic images: caller surfaces -> atlas rectangles, one launch per tick for every image (st_tick) --------------------------------------
+// A block copies rows [r0, r1) of one image: the tile's units (4-byte texels of the ragged head and tail, 16-byte groups in between) are
+// spread over the block's threads.  Sources may be peer device memory or mapped host memory; every load is read once.
+constexpr u32 kAtlasRefreshThreads = 256;
+__global__ void __launch_bounds__(kAtlasRefreshThreads) k_atlas_refresh(const __grid_constant__ AtlasCopyBatch b, uchar4* __restrict__ atlas) {
+    int lo = 0, hi = b.n - 1;
+    while (lo < hi) { const int mid = (lo + hi + 1) >> 1; if (b.c[mid].block0 <= blockIdx.x) lo = mid; else hi = mid - 1; }
+    const AtlasCopy& c = b.c[lo];
+    const u32 r0 = (blockIdx.x - c.block0) * c.rows_per_block, rows = min(c.h - r0, c.rows_per_block);
+    const u32 units = c.head + c.body + c.tail, total = rows * units;
+    for (u32 i = threadIdx.x; i < total; i += kAtlasRefreshThreads) {
+        const u32 r = r0 + i / units, u = i % units;
+        const char* s = c.src + (size_t)r * c.pitch;
+        uchar4* d = atlas + (size_t)(c.y + r) * kAtlasSize + c.x;
+        if (u >= c.head && u < c.head + c.body) {
+            const u32 t = c.head + 4u * (u - c.head);
+            *reinterpret_cast<uint4*>(d + t) = __ldcs(reinterpret_cast<const uint4*>(s + 4 * (size_t)t));
+        } else {
+            const u32 t = u < c.head ? u : u + 3u * c.body;   // tail texel: head + 4 * body + (u - head - body)
+            d[t] = __ldcs(reinterpret_cast<const uchar4*>(s + 4 * (size_t)t));
+        }
+    }
+}
+int launch_atlas_refresh(std::vector<AtlasCopy>& copies, uchar4* atlas, cudaStream_t st) {
+    int launches = 0;
+    for (size_t c0 = 0; c0 < copies.size(); c0 += kAtlasCopies) {
+        AtlasCopyBatch b; b.n = (int)std::min<size_t>(kAtlasCopies, copies.size() - c0);
+        u32 blocks = 0;
+        for (int k = 0; k < b.n; k++) {
+            AtlasCopy& c = copies[c0 + k];
+            // 16-byte groups need the source row and the atlas row to share their address modulo 16 on every row
+            const u32 dmis = (4u * c.x) & 15u;
+            const bool wide = ((uintptr_t)c.src & 15u) == dmis && c.pitch % 16 == 0;
+            c.head = wide ? std::min(c.w, ((16u - dmis) & 15u) / 4u) : c.w;
+            c.body = wide ? (c.w - c.head) / 4u : 0u;
+            c.tail = c.w - c.head - 4u * c.body;
+            const u32 units = c.head + c.body + c.tail;
+            c.rows_per_block = std::max(1u, std::min(c.h, kAtlasRefreshThreads / units));   // about one unit per thread
+            c.block0 = blocks;
+            blocks += (c.h + c.rows_per_block - 1) / c.rows_per_block;
+            b.c[k] = c;
+        }
+        k_atlas_refresh<<<blocks, kAtlasRefreshThreads, 0, st>>>(b, atlas);
+        launches++;
+    }
+    return launches;
+}
 // ---- strips, fused transport: sequence flags between ranks + the temporal pull -------------------------------------------
 // Flags live in each rank's own memory, word [slot * ST_PEER_MAX_RANKS + source rank]; a rank raises its word in a peer's array to
 // the frame's sequence number with a system-scope release store after the kernels that produced the rows have completed

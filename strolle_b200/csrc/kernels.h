@@ -56,6 +56,19 @@ void launch_composition(const ViewSet& v, const SceneDev& s, int cur, u32 mode, 
 enum OutputFormat { OUT_RGBA32F = 0, OUT_RGBA8_SRGB = 1, OUT_RGBA16F = 2 };
 // per view: rows [cam.y0, cam.y1) of cam.output stored at dst + y * pitch (pitch and dst aligned to the format's bytes per pixel)
 void launch_output_store(const ViewSet& v, const SceneDev& s, int format, cudaStream_t st);
+// Dynamic images (st_insert_dynamic_image): at each tick every image's caller-owned surface is copied into its atlas rectangle.  One record per
+// image; a block copies `rows_per_block` rows of one image, and finds its record from the running block offsets (`block0`, ascending).
+// Each row is `head` 4-byte texels, `body` 16-byte groups of four, then `tail` 4-byte texels; body > 0 only when the source row and the atlas
+// row have the same address modulo 16 on every row (the host sets head = texels up to the atlas row's first 16-byte boundary).
+struct AtlasCopy {
+    const char* src; unsigned long long pitch;   // source texel (0, 0) (a device, peer, managed or mapped host address) and its row pitch
+    u32 x, y, w, h;                               // atlas rectangle
+    u32 head, body, tail, rows_per_block, block0;
+};
+constexpr int kAtlasCopies = 128;   // records per launch (5 KB of parameters); more images run as several launches
+struct AtlasCopyBatch { AtlasCopy c[kAtlasCopies]; int n; };
+// Splits `copies` into launches of kAtlasCopies records; fills head / body / tail / rows_per_block / block0.  Returns the launch count.
+int launch_atlas_refresh(std::vector<AtlasCopy>& copies, uchar4* atlas, cudaStream_t st);
 void launch_ref_tracing(const ViewSet& v, const SceneDev& s, u32 depth, cudaStream_t st);
 void launch_ref_shading(const ViewSet& v, const SceneDev& s, u32 seed, u32 depth, cudaStream_t st);
 void launch_bvh_heatmap(const ViewSet& v, const SceneDev& s, cudaStream_t st);

@@ -84,7 +84,8 @@ def load_library():
         "st_engine_create": [C.c_int, C.POINTER(P)], "st_engine_destroy": [P],
         "st_insert_mesh": [P, u64, C.POINTER(_MeshTriangle), C.c_size_t], "st_remove_mesh": [P, u64],
         "st_insert_material": [P, u64, C.POINTER(_Material)], "st_has_material": [P, u64], "st_remove_material": [P, u64],
-        "st_insert_image": [P, u64, C.c_void_p, u32, u32], "st_remove_image": [P, u64], "st_set_material_textures": [P, u64, C.POINTER(_MaterialTextures)],
+        "st_insert_image": [P, u64, C.c_void_p, u32, u32], "st_remove_image": [P, u64], "st_insert_dynamic_image": [P, u64, C.c_void_p, C.c_size_t, u32, u32],
+        "st_read_image": [P, u64, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)], "st_set_material_textures": [P, u64, C.POINTER(_MaterialTextures)],
         "st_insert_instance": [P, u64, u64, u64, f32p], "st_remove_instance": [P, u64],
         "st_insert_light": [P, u64, C.POINTER(_Light)], "st_remove_light": [P, u64], "st_update_sun": [P, C.c_float, C.c_float],
         "st_create_camera": [P, C.POINTER(_Camera), C.POINTER(i32)], "st_update_camera": [P, i32, C.POINTER(_Camera)], "st_delete_camera": [P, i32],
@@ -115,7 +116,8 @@ def load_library():
         "st_multi_create": [C.POINTER(C.c_int), C.c_int, C.POINTER(P)],
         "st_multi_insert_mesh": [P, u64, C.POINTER(_MeshTriangle), C.c_size_t], "st_multi_remove_mesh": [P, u64],
         "st_multi_insert_material": [P, u64, C.POINTER(_Material)], "st_multi_has_material": [P, u64], "st_multi_remove_material": [P, u64],
-        "st_multi_insert_image": [P, u64, C.c_void_p, u32, u32], "st_multi_remove_image": [P, u64], "st_multi_set_material_textures": [P, u64, C.POINTER(_MaterialTextures)],
+        "st_multi_insert_image": [P, u64, C.c_void_p, u32, u32], "st_multi_remove_image": [P, u64],
+        "st_multi_insert_dynamic_image": [P, u64, C.c_void_p, C.c_size_t, u32, u32], "st_multi_set_material_textures": [P, u64, C.POINTER(_MaterialTextures)],
         "st_multi_insert_instance": [P, u64, u64, u64, f32p], "st_multi_remove_instance": [P, u64],
         "st_multi_insert_light": [P, u64, C.POINTER(_Light)], "st_multi_remove_light": [P, u64], "st_multi_update_sun": [P, C.c_float, C.c_float],
         "st_multi_create_camera": [P, C.POINTER(_Camera), C.POINTER(i32)], "st_multi_update_camera": [P, i32, C.POINTER(_Camera)], "st_multi_delete_camera": [P, i32],
@@ -257,6 +259,32 @@ class _Surface:
             synchronize()
 
 
+def _dynamic_source(surface):
+    """A dynamic image's surface: a torch uint8 tensor of shape (h, w, 4) on CUDA or in pinned host memory, pixels and channels
+    contiguous, any row stride (e.g. a slice of a larger tensor).  Returns the checked `_Surface`."""
+    if not hasattr(surface, "data_ptr"):
+        raise TypeError(f"a dynamic image's surface must be a torch tensor on CUDA or in pinned memory, got {type(surface).__name__}; "
+                        "pass host pixels to insert_image instead")
+    s = _Surface(surface, FORMAT_RGBA8_SRGB, None)
+    if not s.cuda and not surface.is_pinned():
+        raise ValueError("a dynamic image's surface must be on CUDA or in pinned memory (the engine reads it at every tick); "
+                         "pass pageable pixels to insert_image instead")
+    return s
+
+
+def _order_dynamic_sources(dynamic):
+    """Before a tick reads the dynamic surfaces: the torch work queued on them (current stream of every device holding one; for pinned
+    sources, of the current device) must be done."""
+    if not dynamic:
+        return
+    import torch
+    devices = {t.device for t in dynamic.values() if t.is_cuda}
+    if any(not t.is_cuda for t in dynamic.values()):
+        devices.add(torch.device("cuda", torch.cuda.current_device()))
+    for d in devices:
+        torch.cuda.current_stream(d).synchronize()
+
+
 class Engine:
     """strolle::Engine on one B200 (CUDA device `device`)."""
 
@@ -278,6 +306,8 @@ class Engine:
             self.set_option(OPT_SHADING_FAST_MATH, 0)
             self.set_option(OPT_FUSED_PASSES, 0)
         self._cams = {}
+        self._images = {}    # handle -> (w, h) of every image inserted here
+        self._dynamic = {}   # handle -> the tensor a dynamic image refreshes from: kept alive while the engine reads it
 
     def _check(self, rc):
         if rc != 0:
@@ -308,6 +338,32 @@ class Engine:
     def insert_image(self, handle, rgba8):
         a = np.ascontiguousarray(rgba8, dtype=np.uint8)
         self._check(self.lib.st_insert_image(self._h, handle, a.ctypes.data, a.shape[1], a.shape[0]))
+        self._images[handle] = (a.shape[1], a.shape[0])
+        self._dynamic.pop(handle, None)
+
+    def insert_dynamic_image(self, handle, surface):
+        """ImageData::Texture { is_dynamic: true }: every `tick()` copies `surface` into the image's atlas rectangle, so cameras rendered after
+        the tick see what the surface held then (e.g. another camera's `render_camera(out=surface, fmt=FORMAT_RGBA8_SRGB)` of the frame
+        before).  `surface`: a torch uint8 tensor (h, w, 4) of Rgba8UnormSrgb texels on CUDA or in pinned memory, any row stride.  The
+        engine keeps a reference to it until `remove_image`, `insert_image` or another `insert_dynamic_image` on the handle."""
+        s = _dynamic_source(surface)
+        h, w = int(surface.shape[0]), int(surface.shape[1])
+        self._check(self.lib.st_insert_dynamic_image(self._h, handle, s.ptr, s.pitch, w, h))
+        self._images[handle] = (w, h)
+        self._dynamic[handle] = surface
+
+    def remove_image(self, handle):
+        self._check(self.lib.st_remove_image(self._h, handle))
+        self._images.pop(handle, None)
+        self._dynamic.pop(handle, None)
+
+    def read_image(self, handle):
+        """The image's atlas rectangle as an (h, w, 4) uint8 array, after the work queued on the engine."""
+        w, h = self._images[handle]
+        out = np.empty((h, w, 4), dtype=np.uint8)
+        n = C.c_size_t()
+        self._check(self.lib.st_read_image(self._h, handle, out.ctypes.data, out.nbytes, C.byref(n)))
+        return out
 
     def set_material_textures(self, handle, base_color=None, emissive=None, metallic_roughness=None, normal_map=None):
         t = [base_color, emissive, metallic_roughness, normal_map]
@@ -355,6 +411,7 @@ class Engine:
 
     # ---- frame ------------------------------------------------------------------------------
     def tick(self):
+        _order_dynamic_sources(self._dynamic)
         self._check(self.lib.st_tick(self._h))
 
     def render_camera(self, cam, out=None, fmt=FORMAT_RGBA32F):
@@ -554,6 +611,7 @@ class MultiEngine:
         self._h = h
         self.n = len(devices)
         self._cams = {}
+        self._images, self._dynamic = {}, {}   # as Engine's
         if blue_noise is None:
             from . import scenes
             blue_noise = scenes.blue_noise()
@@ -582,6 +640,7 @@ class MultiEngine:
         """Borrowed `Engine` view of member `rank` (statistics, per-strip buffers); do not close it."""
         e = Engine.__new__(Engine)
         e.lib, e._h, e._cams = self.lib, C.c_void_p(self.lib.st_multi_engine(self._h, rank)), {}
+        e._images, e._dynamic = self._images, {}
         e.close = lambda: None
         return e
 
@@ -600,6 +659,25 @@ class MultiEngine:
     def insert_image(self, handle, rgba8):
         a = np.ascontiguousarray(rgba8, dtype=np.uint8)
         self._check(self.lib.st_multi_insert_image(self._h, handle, a.ctypes.data, a.shape[1], a.shape[0]))
+        self._images[handle] = (a.shape[1], a.shape[0])
+        self._dynamic.pop(handle, None)
+
+    def insert_dynamic_image(self, handle, surface):
+        """As `Engine.insert_dynamic_image`; every member refreshes its own atlas from `surface`, which every member's device must reach."""
+        s = _dynamic_source(surface)
+        h, w = int(surface.shape[0]), int(surface.shape[1])
+        self._check(self.lib.st_multi_insert_dynamic_image(self._h, handle, s.ptr, s.pitch, w, h))
+        self._images[handle] = (w, h)
+        self._dynamic[handle] = surface
+
+    def remove_image(self, handle):
+        self._check(self.lib.st_multi_remove_image(self._h, handle))
+        self._images.pop(handle, None)
+        self._dynamic.pop(handle, None)
+
+    def read_image(self, handle, rank=0):
+        """Member `rank`'s atlas rectangle of the image (every member holds the same texels)."""
+        return self.member(rank).read_image(handle)
 
     def set_material_textures(self, handle, base_color=None, emissive=None, metallic_roughness=None, normal_map=None):
         t = [base_color, emissive, metallic_roughness, normal_map]
@@ -638,6 +716,7 @@ class MultiEngine:
         self._cams[cam] = (w, h)
 
     def tick(self):
+        _order_dynamic_sources(self._dynamic)
         self._check(self.lib.st_multi_tick(self._h))
 
     def render_camera(self, cam, out=None, fmt=FORMAT_RGBA32F):
