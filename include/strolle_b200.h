@@ -389,6 +389,35 @@ int st_multi_set_blue_noise(st_multi* m, const uint8_t* rgba8_256x256);
 int st_multi_read_buffer(st_multi* m, st_camera_handle camera, const char* name, float* dst, size_t cap_floats, size_t* count);
 int st_multi_peer_errors(st_multi* m, st_camera_handle camera, uint32_t* count);
 
+/* ---- view-parallel groups: whole cameras placed on one member each (no reference counterpart) -------------------------------------
+ * Many independent views (split screen, camera walls, mirrors and monitors, probes) need no exchange between devices: each renders whole
+ * on one member.  Members tick in lockstep, so frame ids, seeds and the BVH are equal on every member, and a placed camera's frames are
+ * bit for bit what one st_engine with the same scene and seed base renders.  On a placed camera st_multi_update_camera (a resize
+ * re-creates its buffers there only), st_multi_delete_camera, st_multi_render_camera(_to) (the whole frame, as st_render_camera(_to)
+ * there), st_multi_read_buffer (the whole frame) and st_multi_peer_errors (always 0) act on its member only; st_multi_member_camera
+ * gives -1 on every other member, where it has no buffers at all.  In a group of one member a placed camera is a strip camera. */
+enum { ST_PLACE_STRIPS = -1, ST_PLACE_AUTO = -2 };
+/* A camera that lives on member `rank` only.  ST_PLACE_AUTO picks the member with the fewest pixels (width * height summed) of placed
+ * cameras, the lowest rank on a tie; the choice is made here, once.  ST_ERR_INVALID for another rank outside [0, size). */
+int st_multi_create_camera_on(st_multi* m, const st_camera* camera, int rank, st_camera_handle* out);
+/* The member a camera lives on, or ST_PLACE_STRIPS for a camera made by st_multi_create_camera.  ST_ERR_NOT_FOUND for an unknown or
+ * deleted camera. */
+int st_multi_camera_rank(st_multi* m, st_camera_handle camera, int* rank);
+/* Moves a placed camera, with all of its temporal state, to member `rank`: waits for the source member's queued work, allocates the
+ * camera there and copies its buffers device to device (a peer copy between devices), then frees the source.  The handle stays; the
+ * next frame is the one it would have rendered where it was.  Moving to its own member does nothing.  ST_ERR_NOT_FOUND for an unknown
+ * camera, ST_ERR_INVALID for a strip camera or a rank outside the group; a refused or failed move leaves the camera where it was. */
+int st_multi_move_camera(st_multi* m, st_camera_handle camera, int rank);
+/* st_render_cameras for the group: every member renders the listed cameras placed on it as batched groups, all members concurrently
+ * (every member's passes and device stores are enqueued before any host copy is issued, and nothing in between waits on the host).
+ * Camera for camera the result is what st_render_cameras gives for them on one engine.  A surface is resolved from its camera's member:
+ * device memory of any device that member reaches (a peer store otherwise), managed or host memory.  Host surfaces block unless
+ * ST_OPT_ASYNC_OUTPUT; device surfaces only enqueue (order with st_multi_synchronize).  In a group of one member this is st_render_cameras
+ * on it.  Everything is checked before any member renders: ST_ERR_NOT_FOUND for an unknown or deleted camera; ST_ERR_INVALID for n <= 0,
+ * a camera listed twice, a strip camera in a group of several members, a surface st_render_camera_to refuses on the camera's member,
+ * or a call before the first st_multi_tick. */
+int st_multi_render_cameras(st_multi* m, const st_camera_handle* cameras, int n, void* const* dsts, const size_t* pitch_bytes, int format);
+
 #ifdef __cplusplus
 }
 #endif

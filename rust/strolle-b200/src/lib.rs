@@ -5,7 +5,8 @@
 //! to the C ABI of `libstrolle_b200.so` (`strolle-b200-sys`).  What differs, and why:
 //!
 //! * `Engine::new` takes CUDA device ordinals instead of a `&wgpu::Device`; one ordinal = one GPU, several = the frame is partitioned
-//!   into row strips across them (`st_multi_*`).  `create_camera` / `update_camera` / `tick` lose their `device` / `queue` arguments.
+//!   into row strips across them (`st_multi_*`), or, with `create_camera_on`, each camera lives whole on one of them.
+//!   `create_camera` / `update_camera` / `tick` lose their `device` / `queue` arguments.
 //! * `render_camera` delivers the composed frame into a [`Frame`] (host pixels in the viewport's format) instead of recording into a
 //!   wgpu command encoder — the CUDA kernels run on the engine's own stream.  A wgpu host uploads it with `Queue::write_texture`
 //!   (what `bevy-strolle-b200` does); `render_camera_to_raw` composes straight into a caller-owned surface in device or host memory
@@ -335,6 +336,16 @@ impl Camera {
 #[derive(Clone, Copy, Debug, PartialEq, Eq, Hash)]
 pub struct CameraHandle(sys::st_camera_handle);
 
+/// Where [`Engine::create_camera_on`] puts a camera: whole on one device of the group (view parallelism), instead of split into row
+/// strips across all of them.
+#[derive(Clone, Copy, Debug, PartialEq, Eq)]
+pub enum Placement {
+    /// The device at this index of the list given to [`Engine::new`].
+    Device(usize),
+    /// The device with the fewest pixels of placed cameras, the lowest index on a tie; decided at creation only.
+    Auto,
+}
+
 /// Host pixels of one composed frame, `viewport.size.x * viewport.size.y` texels of `format`, row-major.  Allocate once per camera
 /// (page-locked memory makes the device-to-host copy asynchronous and full speed) and reuse.
 #[derive(Debug)]
@@ -565,6 +576,28 @@ impl<P: Params> Engine<P> {
         Ok(handle)
     }
 
+    /// Creates a camera that lives whole on one device of the group: its buffers exist there only, and it renders whole frames there
+    /// with no exchange between devices.  Many small independent views (split screen, monitors, mirrors) spread this way across the
+    /// devices and render concurrently through [`Self::render_cameras_to_raw`]; one large view is better split with [`Self::create_camera`].
+    pub fn create_camera_on(&mut self, camera: Camera, placement: Placement) -> Result<CameraHandle, Error> {
+        let rank = match placement {
+            Placement::Device(index) => c_int::try_from(index).map_err(|_| Error { code: sys::ST_ERR_INVALID, message: "device index out of range".into() })?,
+            Placement::Auto => sys::ST_PLACE_AUTO,
+        };
+        let mut out = 0;
+        check(unsafe { sys::st_multi_create_camera_on(self.raw, &camera.to_ffi(), rank, &mut out) })?;
+        let handle = CameraHandle(out);
+        self.viewports.insert(handle, camera.viewport);
+        Ok(handle)
+    }
+
+    /// Moves a camera made by [`Self::create_camera_on`], with all of its temporal state, to the device at `device` of the group; its
+    /// next frame is the one it would have rendered where it was.  Waits for the camera's queued work first.
+    pub fn move_camera(&mut self, handle: CameraHandle, device: usize) -> Result<(), Error> {
+        let rank = c_int::try_from(device).map_err(|_| Error { code: sys::ST_ERR_INVALID, message: "device index out of range".into() })?;
+        check(unsafe { sys::st_multi_move_camera(self.raw, handle.0, rank) })
+    }
+
     /// Updates camera, changing its mode, position, size etc. (`lib.rs:262-273`).
     pub fn update_camera(&mut self, handle: CameraHandle, camera: Camera) -> Result<(), Error> {
         check(unsafe { sys::st_multi_update_camera(self.raw, handle.0, &camera.to_ffi()) })?;
@@ -599,8 +632,9 @@ impl<P: Params> Engine<P> {
 
     /// Renders several cameras for this frame, each as [`Self::render_camera_to_raw`] with `dsts[i]` and `pitches[i]` would, bit for
     /// bit; cameras of one size and mode run as one launch per pass.  A null `dsts[i]` renders camera `i` without output; empty
-    /// `dsts` / `pitches` mean no outputs / packed rows.  Only a group of one device renders batches (the cameras of a strip group are
-    /// split across devices): with several devices this returns `ST_ERR_INVALID`.
+    /// `dsts` / `pitches` mean no outputs / packed rows.  In a group of several devices the cameras must have been made by
+    /// [`Self::create_camera_on`]: every device renders the listed cameras it holds, all devices at once, and a surface may be on any
+    /// device the camera's device reaches.
     ///
     /// # Safety
     /// Every non-null `dsts[i]` must satisfy the requirements of [`Self::render_camera_to_raw`] for camera `handles[i]`.
@@ -608,14 +642,11 @@ impl<P: Params> Engine<P> {
         if (!dsts.is_empty() && dsts.len() != handles.len()) || (!pitches.is_empty() && pitches.len() != handles.len()) {
             return Err(Error { code: sys::ST_ERR_INVALID, message: "one surface and one pitch per camera".into() });
         }
-        if sys::st_multi_size(self.raw) != 1 {
-            return Err(Error { code: sys::ST_ERR_INVALID, message: "batched rendering needs a group of one device".into() });
-        }
-        let members: Vec<sys::st_camera_handle> = handles.iter().map(|h| sys::st_multi_member_camera(self.raw, h.0, 0)).collect();
-        check(sys::st_render_cameras(
-            sys::st_multi_engine(self.raw, 0),
-            members.as_ptr(),
-            members.len() as c_int,
+        let cameras: Vec<sys::st_camera_handle> = handles.iter().map(|h| h.0).collect();
+        check(sys::st_multi_render_cameras(
+            self.raw,
+            cameras.as_ptr(),
+            cameras.len() as c_int,
             if dsts.is_empty() { std::ptr::null() } else { dsts.as_ptr() },
             if pitches.is_empty() { std::ptr::null() } else { pitches.as_ptr() },
             format.to_ffi(),

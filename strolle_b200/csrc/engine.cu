@@ -1614,24 +1614,31 @@ int st_render_camera_to(st_engine* e, st_camera_handle h, void* dst, size_t pitc
     return ST_OK;
 }
 // Several cameras of one frame.  Every camera rendered after the same tick has the same frame id, so cameras of one size and mode run
-// the same passes with the same seeds; such a group runs as one launch per pass, blockIdx.z selecting the camera.
-int st_render_cameras(st_engine* e, const st_camera_handle* cameras, int n, void* const* dsts, const size_t* pitch_bytes, int format) {
-    if (!e) return fail(ST_ERR_INVALID, "null engine");
-    if (n <= 0 || !cameras) return fail(ST_ERR_INVALID, "no cameras to render");
+// the same passes with the same seeds; such a group runs as one launch per pass, blockIdx.z selecting the camera.  Three steps, which
+// st_multi_render_cameras runs on every member of a group (each step on all members before the next): check, enqueue, copy out.
+struct CameraBatch { std::vector<CameraSlot*> cs; std::vector<OutputTarget> t; };
+// Everything is checked before any pass runs, so that a refused call changes nothing.
+static int batch_check(st_engine* e, const st_camera_handle* cameras, int n, void* const* dsts, const size_t* pitch_bytes, int format, CameraBatch* b) {
     CK(cudaSetDevice(e->device));
-    std::vector<CameraSlot*> cs(n);
-    std::vector<OutputTarget> t(n);
-    for (int i = 0; i < n; i++) {   // everything is checked before any pass runs: a refused call changes nothing
-        if (!(cs[i] = get_camera(e, cameras[i]))) return fail(ST_ERR_NOT_FOUND, "unknown camera " + std::to_string(cameras[i]));
+    b->cs.assign(n, nullptr); b->t.assign(n, OutputTarget{});
+    for (int i = 0; i < n; i++) {
+        if (!(b->cs[i] = get_camera(e, cameras[i]))) return fail(ST_ERR_NOT_FOUND, "unknown camera " + std::to_string(cameras[i]));
         if (std::find(cameras, cameras + i, cameras[i]) != cameras + i) return fail(ST_ERR_INVALID, "camera " + std::to_string(cameras[i]) + " is listed twice");
-        if (cs[i]->dev.y0 != 0 || cs[i]->dev.y1 != (int)cs[i]->desc.height || cs[i]->peer.ready)
+        const CameraSlot* c = b->cs[i];
+        if (c->dev.y0 != 0 || c->dev.y1 != (int)c->desc.height || c->peer.ready)
             return fail(ST_ERR_INVALID, "camera " + std::to_string(cameras[i]) + " renders a row strip; st_render_cameras takes whole-frame cameras only");
-        if (cs[i]->frame == 0) return fail(ST_ERR_INVALID, "st_tick must precede st_render_camera");
-        t[i].dst = nullptr;
-        if (dsts && dsts[i]) { int rc = resolve_target(e, cs[i]->desc.width, dsts[i], pitch_bytes ? pitch_bytes[i] : 0, format, &t[i]); if (rc) return rc; }
+        if (c->frame == 0) return fail(ST_ERR_INVALID, "st_tick must precede st_render_camera");
+        b->t[i].dst = nullptr;
+        if (dsts && dsts[i]) { int rc = resolve_target(e, c->desc.width, dsts[i], pitch_bytes ? pitch_bytes[i] : 0, format, &b->t[i]); if (rc) return rc; }
     }
-    int rc = ensure_luts(e); if (rc) return rc;
-    // groups by (width, height, mode, denoise, ref_depth), in the order of their first camera; list order within a group
+    return ST_OK;
+}
+// The passes and the device-surface stores, grouped by (width, height, mode, denoise, ref_depth) in the order of their first camera, list
+// order within a group, a group larger than one launch holds split into chunks.  Nothing here waits on the host.
+static int batch_enqueue(st_engine* e, const CameraBatch& b, int format) {
+    const std::vector<CameraSlot*>& cs = b.cs;
+    const int n = (int)cs.size();
+    CK(cudaSetDevice(e->device));
     std::vector<std::vector<int>> groups;
     for (int i = 0; i < n; i++) {
         const st_camera& d = cs[i]->desc;
@@ -1642,7 +1649,6 @@ int st_render_cameras(st_engine* e, const st_camera_handle* cameras, int n, void
         auto it = std::find_if(groups.begin(), groups.end(), same);
         if (it == groups.end()) groups.push_back({i}); else it->push_back(i);
     }
-    bool host_out = false;
     for (const std::vector<int>& g : groups) {
         for (size_t c0 = 0; c0 < g.size(); c0 += kBatchViews) {
             const std::vector<int> idx(g.begin() + c0, g.begin() + std::min(g.size(), c0 + kBatchViews));
@@ -1651,12 +1657,33 @@ int st_render_cameras(st_engine* e, const st_camera_handle* cameras, int n, void
             std::vector<Step> steps; build_schedule(e, chunk, &steps);
             for (const Step& s : steps) e->run_timed(s.pass, s.run, s.sub);
             ViewSet store;   // the device surfaces of the chunk: one store launch
-            for (int i : idx) if (t[i].dst && t[i].device) { store.push_back(view_of(cs[i], chunk[0], 0)); store.back().dst = t[i].dst; store.back().pitch = t[i].pitch; }
+            for (int i : idx) if (b.t[i].dst && b.t[i].device) { store.push_back(view_of(cs[i], chunk[0], 0)); store.back().dst = b.t[i].dst; store.back().pitch = b.t[i].pitch; }
             if (!store.empty()) { const SceneDev sc = e->scene(); e->run_timed(P_COMPOSITION, [&](cudaStream_t s) { launch_output_store(store, sc, format, s); }); }
-            for (int i : idx) if (t[i].dst && !t[i].device) { host_out = true; if ((rc = copy_rows_out(e, cs[i], t[i], 0, (int)cs[i]->desc.height))) return rc; }
         }
     }
     CK(cudaGetLastError());
+    return ST_OK;
+}
+// One copy per host surface (behind the passes on the engine's stream); *host_out = there was one.
+static int batch_copy_out(st_engine* e, const CameraBatch& b, bool* host_out) {
+    CK(cudaSetDevice(e->device));
+    *host_out = false;
+    for (size_t i = 0; i < b.cs.size(); i++) if (b.t[i].dst && !b.t[i].device) {
+        *host_out = true;
+        int rc = copy_rows_out(e, b.cs[i], b.t[i], 0, (int)b.cs[i]->desc.height); if (rc) return rc;
+    }
+    CK(cudaGetLastError());
+    return ST_OK;
+}
+int st_render_cameras(st_engine* e, const st_camera_handle* cameras, int n, void* const* dsts, const size_t* pitch_bytes, int format) {
+    if (!e) return fail(ST_ERR_INVALID, "null engine");
+    if (n <= 0 || !cameras) return fail(ST_ERR_INVALID, "no cameras to render");
+    CameraBatch b;
+    int rc = batch_check(e, cameras, n, dsts, pitch_bytes, format, &b); if (rc) return rc;
+    if ((rc = ensure_luts(e))) return rc;
+    if ((rc = batch_enqueue(e, b, format))) return rc;
+    bool host_out = false;
+    if ((rc = batch_copy_out(e, b, &host_out))) return rc;
     if (host_out && !e->async_output) CK(cudaStreamSynchronize(e->stream));
     return ST_OK;
 }
@@ -2201,7 +2228,9 @@ int st_wavelet_times(st_engine* e, float* ms5, uint32_t* launches5, int reset) {
 // every member and linked (st_link_local), st_multi_render_camera enqueues every rank's strip of the frame (fused transport) and then
 // lets every rank copy its own rows into the caller's frame.  What a single-process host (the Bevy plugin) binds instead of st_engine.
 // =================================================================================================
-struct st_multi { std::vector<st_engine*> e; std::vector<std::vector<st_camera_handle>> cams; };   // cams[c][rank]
+// cams[c][rank]: camera c's handle on member `rank` (-1 where it has none).  home[c]: ST_PLACE_STRIPS for a strip camera (one on every member,
+// linked), or the one member a placed camera lives on (st_multi_create_camera_on).
+struct st_multi { std::vector<st_engine*> e; std::vector<std::vector<st_camera_handle>> cams; std::vector<int> home; };
 #define ST_MULTI_ALL(call) do { if (!m) return fail(ST_ERR_INVALID, "null group"); for (st_engine* e : m->e) { int rc_ = (call); if (rc_) return rc_; } return ST_OK; } while (0)
 int st_multi_create(const int* devices, int n, st_multi** out) {
     if (!devices || !out || n < 1 || n > ST_PEER_MAX_RANKS) return fail(ST_ERR_LIMIT, "1..16 devices");
@@ -2265,12 +2294,78 @@ int st_multi_create_camera(st_multi* m, const st_camera* c, st_camera_handle* ou
     std::vector<st_camera_handle> hs(m->e.size());
     for (size_t i = 0; i < m->e.size(); i++) { int rc = st_create_camera(m->e[i], c, &hs[i]); if (rc) return rc; }
     if (m->e.size() > 1) { int rc = st_link_local(m->e.data(), hs.data(), (int)m->e.size()); if (rc) return rc; }
-    m->cams.push_back(hs);
+    m->cams.push_back(hs); m->home.push_back(ST_PLACE_STRIPS);
     *out = (st_camera_handle)m->cams.size() - 1;
     return ST_OK;
 }
+// camera `h` of the group, placed on one member: *rank = that member, *cs = its slot there.  ST_ERR_NOT_FOUND for an unknown or deleted
+// camera; nullptr in *cs and ST_OK for a strip camera.
+static int placed_camera(st_multi* m, st_camera_handle h, int* rank, CameraSlot** cs) {
+    if (!m || h < 0 || (size_t)h >= m->cams.size()) return fail(ST_ERR_NOT_FOUND, "unknown camera " + std::to_string(h));
+    *rank = m->home[h]; *cs = nullptr;
+    const int r = *rank >= 0 ? *rank : 0;
+    CameraSlot* c = get_camera(m->e[r], m->cams[h][r]);
+    if (!c) return fail(ST_ERR_NOT_FOUND, "camera " + std::to_string(h) + " was deleted");
+    if (*rank >= 0) *cs = c;
+    return ST_OK;
+}
+int st_multi_create_camera_on(st_multi* m, const st_camera* c, int rank, st_camera_handle* out) {
+    if (!m || !c || !out) return fail(ST_ERR_INVALID, "null argument");
+    const int n = (int)m->e.size();
+    if (rank == ST_PLACE_AUTO) {   // the member with the fewest pixels of placed cameras, the lowest rank on a tie
+        std::vector<uint64_t> pixels(n, 0);
+        for (size_t k = 0; k < m->cams.size(); k++) {
+            const int r = m->home[k];
+            const CameraSlot* cs = r >= 0 ? get_camera(m->e[r], m->cams[k][r]) : nullptr;
+            if (cs) pixels[r] += (uint64_t)cs->desc.width * cs->desc.height;
+        }
+        rank = (int)(std::min_element(pixels.begin(), pixels.end()) - pixels.begin());
+    }
+    if (rank < 0 || rank >= n) return fail(ST_ERR_INVALID, "rank " + std::to_string(rank) + " is not a member of this group of " + std::to_string(n));
+    st_camera_handle mh = -1;
+    int rc = st_create_camera(m->e[rank], c, &mh); if (rc) return rc;
+    std::vector<st_camera_handle> hs(n, -1); hs[rank] = mh;
+    m->cams.push_back(hs); m->home.push_back(rank);
+    *out = (st_camera_handle)m->cams.size() - 1;
+    return ST_OK;
+}
+int st_multi_camera_rank(st_multi* m, st_camera_handle h, int* rank) {
+    if (!rank) return fail(ST_ERR_INVALID, "null argument");
+    CameraSlot* cs = nullptr; int r = 0;
+    int rc = placed_camera(m, h, &r, &cs); if (rc) return rc;
+    *rank = r;
+    return ST_OK;
+}
+// The camera's complete state travels: the arena (every named buffer, history included), the paired à-trous scratch, the camera uniforms
+// of this and the last frame, and the frame it was ticked for.  The arenas of one size have one layout, so one copy each suffices.
+int st_multi_move_camera(st_multi* m, st_camera_handle h, int rank) {
+    CameraSlot* cs = nullptr; int from = 0;
+    int rc = placed_camera(m, h, &from, &cs); if (rc) return rc;
+    if (!cs) return fail(ST_ERR_INVALID, "camera " + std::to_string(h) + " is a strip camera; only placed cameras move");
+    if (rank < 0 || rank >= (int)m->e.size()) return fail(ST_ERR_INVALID, "rank " + std::to_string(rank) + " is not a member of this group of " + std::to_string(m->e.size()));
+    if (rank == from) return ST_OK;
+    st_engine *src = m->e[from], *dst = m->e[rank];
+    if ((rc = st_synchronize(src))) return rc;   // the source's queued passes and output copies are done with the arena
+    CK(cudaSetDevice(dst->device));
+    CameraSlot* ns = new CameraSlot();
+    ns->alive = true; ns->desc = cs->desc;
+    auto undo = [&](int code) { ns->arena.release(); ns->svgf_pairs.release(); delete ns; return code; };
+    if ((rc = allocate_camera(dst, ns))) return undo(rc);
+    if (ns->arena.cap != cs->arena.cap || ns->svgf_pairs.cap != cs->svgf_pairs.cap) return undo(fail(ST_ERR_INVALID, "arena layouts differ"));
+    // behind allocate_camera's fills on the target's stream; a peer copy when the devices differ
+    cudaError_t ce = cudaMemcpyPeerAsync(ns->arena.p, dst->device, cs->arena.p, src->device, cs->arena.cap, dst->stream);
+    if (ce == cudaSuccess && cs->svgf_pairs.p) ce = cudaMemcpyPeerAsync(ns->svgf_pairs.p, dst->device, cs->svgf_pairs.p, src->device, cs->svgf_pairs.cap, dst->stream);
+    if (ce == cudaSuccess) ce = cudaStreamSynchronize(dst->stream);
+    if (ce != cudaSuccess) { cudaGetLastError(); return undo(fail(ST_ERR_CUDA, std::string("camera move: ") + cudaGetErrorString(ce))); }
+    ns->dev.curr = cs->dev.curr; ns->dev.prev = cs->dev.prev; ns->frame = cs->frame;
+    dst->cameras.push_back(ns);
+    const st_camera_handle old = m->cams[h][from];
+    m->cams[h][from] = -1; m->cams[h][rank] = (st_camera_handle)dst->cameras.size() - 1; m->home[h] = rank;
+    return st_delete_camera(src, old);
+}
 int st_multi_update_camera(st_multi* m, st_camera_handle h, const st_camera* c) {
     if (!m || h < 0 || (size_t)h >= m->cams.size() || !c) return fail(ST_ERR_NOT_FOUND, "unknown camera");
+    if (m->home[h] >= 0) return st_update_camera(m->e[m->home[h]], m->cams[h][m->home[h]], c);   // a resize re-creates the buffers there only
     bool relink = false;
     for (size_t i = 0; i < m->e.size(); i++) {
         CameraSlot* cs = get_camera(m->e[i], m->cams[h][i]);
@@ -2284,6 +2379,7 @@ int st_multi_update_camera(st_multi* m, st_camera_handle h, const st_camera* c) 
 }
 int st_multi_delete_camera(st_multi* m, st_camera_handle h) {
     if (!m || h < 0 || (size_t)h >= m->cams.size()) return fail(ST_ERR_NOT_FOUND, "unknown camera");
+    if (m->home[h] >= 0) return st_delete_camera(m->e[m->home[h]], m->cams[h][m->home[h]]);
     for (st_engine* e : m->e) { cudaSetDevice(e->device); cudaStreamSynchronize(e->stream); }
     for (size_t i = 0; i < m->e.size(); i++) { int rc = st_delete_camera(m->e[i], m->cams[h][i]); if (rc) return rc; }
     return ST_OK;
@@ -2311,6 +2407,7 @@ static int multi_render(st_multi* m, st_camera_handle h, const OutputTarget* tar
 int st_multi_render_camera(st_multi* m, st_camera_handle h, void* host_out, int format) {
     if (!m || h < 0 || (size_t)h >= m->cams.size()) return fail(ST_ERR_NOT_FOUND, "unknown camera");
     if (m->e.size() == 1) return st_render_camera(m->e[0], m->cams[h][0], host_out, format);
+    if (m->home[h] >= 0) return st_render_camera(m->e[m->home[h]], m->cams[h][m->home[h]], host_out, format);   // a whole frame on its member
     std::vector<OutputTarget> t;
     for (size_t i = 0; host_out && i < m->e.size(); i++) {
         CameraSlot* cs = get_camera(m->e[i], m->cams[h][i]);
@@ -2322,6 +2419,7 @@ int st_multi_render_camera(st_multi* m, st_camera_handle h, void* host_out, int 
 int st_multi_render_camera_to(st_multi* m, st_camera_handle h, void* dst, size_t pitch, int format) {
     if (!m || h < 0 || (size_t)h >= m->cams.size()) return fail(ST_ERR_NOT_FOUND, "unknown camera");
     if (m->e.size() == 1) return st_render_camera_to(m->e[0], m->cams[h][0], dst, pitch, format);
+    if (m->home[h] >= 0) return st_render_camera_to(m->e[m->home[h]], m->cams[h][m->home[h]], dst, pitch, format);
     std::vector<OutputTarget> t(m->e.size());
     for (size_t i = 0; i < m->e.size(); i++) {   // every member must reach the surface before any of them renders
         CameraSlot* cs = get_camera(m->e[i], m->cams[h][i]);
@@ -2334,6 +2432,7 @@ int st_multi_render_camera_to(st_multi* m, st_camera_handle h, void* dst, size_t
 // per-camera buffer of the whole frame, assembled from the members' strips (test hook, cf. st_read_buffer)
 int st_multi_read_buffer(st_multi* m, st_camera_handle h, const char* name, float* dst, size_t cap, size_t* count) {
     if (!m || h < 0 || (size_t)h >= m->cams.size() || !name || !count) return fail(ST_ERR_NOT_FOUND, "unknown camera");
+    if (m->home[h] >= 0) return st_read_buffer(m->e[m->home[h]], m->cams[h][m->home[h]], name, dst, cap, count);
     const size_t n = m->e.size();
     int rc = st_read_buffer(m->e[0], m->cams[h][0], name, nullptr, 0, count); if (rc) return rc;
     if (!dst) return ST_OK;
@@ -2353,7 +2452,36 @@ int st_multi_read_buffer(st_multi* m, st_camera_handle h, const char* name, floa
 int st_multi_peer_errors(st_multi* m, st_camera_handle h, uint32_t* count) {
     if (!m || h < 0 || (size_t)h >= m->cams.size() || !count) return fail(ST_ERR_NOT_FOUND, "unknown camera");
     *count = 0;
+    if (m->home[h] >= 0) return get_camera(m->e[m->home[h]], m->cams[h][m->home[h]]) ? ST_OK : fail(ST_ERR_NOT_FOUND, "unknown camera");   // no peer link
     for (size_t i = 0; i < m->e.size(); i++) { uint32_t c = 0; int rc = st_peer_errors(m->e[i], m->cams[h][i], &c); if (rc) return rc; *count += c; }
+    return ST_OK;
+}
+// st_render_cameras for the group: every member renders the listed cameras that live on it as batched groups, all members at once.  Each
+// step runs on every member before the next one starts, so that no member's enqueue waits on the host: every check; the LUTs (which
+// synchronise their device); the passes and device-surface stores; the host-surface copies; the synchronisation of members that copied.
+int st_multi_render_cameras(st_multi* m, const st_camera_handle* cameras, int n, void* const* dsts, const size_t* pitch_bytes, int format) {
+    if (!m) return fail(ST_ERR_INVALID, "null group");
+    if (n <= 0 || !cameras) return fail(ST_ERR_INVALID, "no cameras to render");
+    const size_t world = m->e.size();
+    std::vector<std::vector<st_camera_handle>> hs(world);   // per member, in list order: member handles, surfaces, pitches
+    std::vector<std::vector<void*>> ds(world);
+    std::vector<std::vector<size_t>> ps(world);
+    for (int i = 0; i < n; i++) {
+        const st_camera_handle h = cameras[i];
+        if (h < 0 || (size_t)h >= m->cams.size()) return fail(ST_ERR_NOT_FOUND, "unknown camera " + std::to_string(h));
+        if (std::find(cameras, cameras + i, h) != cameras + i) return fail(ST_ERR_INVALID, "camera " + std::to_string(h) + " is listed twice");
+        if (m->home[h] < 0 && world > 1) return fail(ST_ERR_INVALID, "camera " + std::to_string(h) + " is a strip camera; st_multi_render_cameras takes placed cameras");
+        const int r = m->home[h] >= 0 ? m->home[h] : 0;
+        hs[r].push_back(m->cams[h][r]); ds[r].push_back(dsts ? dsts[i] : nullptr); ps[r].push_back(pitch_bytes ? pitch_bytes[i] : 0);
+    }
+    if (world == 1) return st_render_cameras(m->e[0], hs[0].data(), n, dsts, pitch_bytes, format);
+    std::vector<CameraBatch> b(world);
+    for (size_t r = 0; r < world; r++) if (!hs[r].empty()) { int rc = batch_check(m->e[r], hs[r].data(), (int)hs[r].size(), ds[r].data(), ps[r].data(), format, &b[r]); if (rc) return rc; }
+    for (size_t r = 0; r < world; r++) if (!hs[r].empty()) { CK(cudaSetDevice(m->e[r]->device)); int rc = ensure_luts(m->e[r]); if (rc) return rc; }
+    for (size_t r = 0; r < world; r++) if (!hs[r].empty()) { int rc = batch_enqueue(m->e[r], b[r], format); if (rc) return rc; }
+    std::vector<char> host_out(world, 0);
+    for (size_t r = 0; r < world; r++) if (!hs[r].empty()) { bool h = false; int rc = batch_copy_out(m->e[r], b[r], &h); if (rc) return rc; host_out[r] = h; }
+    for (size_t r = 0; r < world; r++) if (host_out[r] && !m->e[r]->async_output) { CK(cudaSetDevice(m->e[r]->device)); CK(cudaStreamSynchronize(m->e[r]->stream)); }
     return ST_OK;
 }
 

@@ -5,6 +5,7 @@ insert_light / update_sun / create_camera / update_camera / tick / render_camera
 hooks of include/strolle_b200.h (read_buffer, trace_closest, pass_times, ...).
 """
 import ctypes as C
+import numbers
 import os
 
 import numpy as np
@@ -33,6 +34,7 @@ STAT_VARIANCE_TILED_LAUNCHES = 4
 STAT_STRIP_PULLED_ROWS = 5
 STAT_LAST_FRAME_FUSED_STRIPS = 6
 STAT_STRIP_FIRST_TIMEOUT = 7
+PLACE_STRIPS, PLACE_AUTO = -1, -2   # st_multi_camera_rank of a strip camera; st_multi_create_camera_on's automatic placement
 
 
 class StrolleError(RuntimeError):
@@ -125,6 +127,9 @@ def load_library():
         "st_multi_set_option": [P, C.c_int, C.c_int], "st_multi_set_seed_base": [P, u32], "st_multi_set_blue_noise": [P, C.c_void_p],
         "st_multi_read_buffer": [P, i32, C.c_char_p, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)], "st_multi_peer_errors": [P, i32, C.POINTER(u32)],
         "st_multi_size": [P], "st_multi_member_camera": [P, i32, C.c_int],
+        "st_multi_create_camera_on": [P, C.POINTER(_Camera), C.c_int, C.POINTER(i32)], "st_multi_camera_rank": [P, i32, C.POINTER(C.c_int)],
+        "st_multi_move_camera": [P, i32, C.c_int],
+        "st_multi_render_cameras": [P, C.POINTER(i32), C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_int],
         "st_bvh_builder_create": [C.POINTER(P)], "st_bvh_builder_read": [P, C.c_void_p, C.c_size_t],
         "st_bvh_builder_build": [P, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t), C.POINTER(u32), C.POINTER(C.c_int)],
     }
@@ -257,6 +262,27 @@ class _Surface:
         fn_to(self.ptr, self.pitch)
         if self.cuda:
             synchronize()
+
+
+def _render_cameras(render, synchronize, sizes, cams, outs, fmt):
+    """The Python side of st_render_cameras / st_multi_render_cameras: checks every surface, orders the torch work queued on the CUDA ones
+    before the call `render(handles, n, dsts, pitches)`, and returns once they hold their frames."""
+    cams = [int(c) for c in cams]
+    n = len(cams)
+    if outs is not None and len(outs) != n:
+        raise ValueError(f"{n} cameras but {len(outs)} output surfaces")
+    surfaces = [None if o is None else _Surface(o, fmt, sizes.get(c)) for c, o in zip(cams, outs or [None] * n)]
+    handles = (C.c_int32 * max(n, 1))(*cams)
+    dsts = (C.c_void_p * max(n, 1))(*[s.ptr if s is not None else None for s in surfaces])
+    pitches = (C.c_size_t * max(n, 1))(*[s.pitch if s is not None else 0 for s in surfaces])
+    cuda = [s for s in surfaces if s is not None and s.cuda]
+    if cuda:
+        import torch
+        for d in {s.device for s in cuda}:
+            torch.cuda.current_stream(d).synchronize()
+    render(handles, n, dsts if outs is not None else None, pitches)
+    if cuda:
+        synchronize()
 
 
 def _dynamic_source(surface):
@@ -431,22 +457,7 @@ class Engine:
         camera's buffers and output are bit for bit what `render_camera` gives when called for the cameras one after another.  `outs`:
         None, or one entry per camera, each None (no output) or a surface as `render_camera`'s `out`, in format `fmt`.  CUDA surfaces
         hold their frames when this returns."""
-        cams = [int(c) for c in cams]
-        n = len(cams)
-        if outs is not None and len(outs) != n:
-            raise ValueError(f"{n} cameras but {len(outs)} output surfaces")
-        surfaces = [None if o is None else _Surface(o, fmt, self._cams.get(c)) for c, o in zip(cams, outs or [None] * n)]
-        handles = (C.c_int32 * max(n, 1))(*cams)
-        dsts = (C.c_void_p * max(n, 1))(*[s.ptr if s is not None else None for s in surfaces])
-        pitches = (C.c_size_t * max(n, 1))(*[s.pitch if s is not None else 0 for s in surfaces])
-        cuda = [s for s in surfaces if s is not None and s.cuda]
-        if cuda:
-            import torch
-            for d in {s.device for s in cuda}:
-                torch.cuda.current_stream(d).synchronize()
-        self._check(self.lib.st_render_cameras(self._h, handles, n, dsts if outs is not None else None, pitches, fmt))
-        if cuda:
-            self.synchronize()
+        _render_cameras(lambda *a: self._check(self.lib.st_render_cameras(self._h, *a, fmt)), self.synchronize, self._cams, cams, outs, fmt)
 
     def render_camera_to(self, cam, ptr, pitch_bytes, fmt):
         """st_render_camera_to on a raw address (pixel (0, 0) of the camera inside the surface); returns once enqueued for device memory."""
@@ -637,7 +648,8 @@ class MultiEngine:
             pass
 
     def member(self, rank):
-        """Borrowed `Engine` view of member `rank` (statistics, per-strip buffers); do not close it."""
+        """Borrowed `Engine` view of member `rank` (statistics, per-strip buffers, the buffers of the cameras placed there under their member
+        handles, `member_camera`); do not close it."""
         e = Engine.__new__(Engine)
         e.lib, e._h, e._cams = self.lib, C.c_void_p(self.lib.st_multi_engine(self._h, rank)), {}
         e._images, e._dynamic = self._images, {}
@@ -703,12 +715,37 @@ class MultiEngine:
     def update_sun(self, azimuth, altitude):
         self._check(self.lib.st_multi_update_sun(self._h, azimuth, altitude))
 
-    def create_camera(self, mode, denoise, ref_depth, w, h, transform16, projection16):
+    def _rank(self, rank, what):
+        if rank == "auto":
+            return PLACE_AUTO
+        if isinstance(rank, bool) or not isinstance(rank, numbers.Integral):
+            raise TypeError(f"{what}: rank must be a member index or \"auto\", got {rank!r}")
+        if not 0 <= rank < self.n:
+            raise ValueError(f"{what}: rank {rank} is not a member of this group of {self.n}")
+        return int(rank)
+
+    def create_camera(self, mode, denoise, ref_depth, w, h, transform16, projection16, rank=None):
+        """`rank=None`: a strip camera, rows split across every member.  An int or "auto": the camera lives whole on that member (view
+        parallelism; "auto" = the member with the fewest pixels of placed cameras, the lowest rank on a tie)."""
         c = Engine._cam(mode, denoise, ref_depth, w, h, transform16, projection16)
         out = C.c_int32()
-        self._check(self.lib.st_multi_create_camera(self._h, C.byref(c), C.byref(out)))
+        if rank is None:
+            self._check(self.lib.st_multi_create_camera(self._h, C.byref(c), C.byref(out)))
+        else:
+            self._check(self.lib.st_multi_create_camera_on(self._h, C.byref(c), self._rank(rank, "create_camera"), C.byref(out)))
         self._cams[out.value] = (w, h)
         return out.value
+
+    def camera_rank(self, cam):
+        """The member a placed camera lives on, or PLACE_STRIPS for a strip camera."""
+        r = C.c_int()
+        self._check(self.lib.st_multi_camera_rank(self._h, cam, C.byref(r)))
+        return r.value
+
+    def move_camera(self, cam, rank):
+        """Moves a placed camera with all of its temporal state to member `rank`; its next frame is the one it would have rendered where
+        it was."""
+        self._check(self.lib.st_multi_move_camera(self._h, cam, self._rank(rank, "move_camera")))
 
     def update_camera(self, cam, mode, denoise, ref_depth, w, h, transform16, projection16):
         c = Engine._cam(mode, denoise, ref_depth, w, h, transform16, projection16)
@@ -727,6 +764,12 @@ class MultiEngine:
         _Surface(out, fmt, self._cams.get(cam)).render(lambda p: self._check(self.lib.st_multi_render_camera(self._h, cam, p, fmt)),
                                                        lambda p, pitch: self._check(self.lib.st_multi_render_camera_to(self._h, cam, p, pitch, fmt)),
                                                        self.synchronize)
+
+    def render_cameras(self, cams, outs=None, fmt=FORMAT_RGBA32F):
+        """As `Engine.render_cameras`, for cameras placed on members of the group: every member renders its cameras of the list as batched
+        groups, all members at once.  Each camera's buffers and output are bit for bit what one `Engine` gives for it.  A CUDA surface may
+        be on any device the camera's member reaches; every one holds its frame when this returns."""
+        _render_cameras(lambda *a: self._check(self.lib.st_multi_render_cameras(self._h, *a, fmt)), self.synchronize, self._cams, cams, outs, fmt)
 
     def render_camera_to(self, cam, ptr, pitch_bytes, fmt):
         self._check(self.lib.st_multi_render_camera_to(self._h, cam, ptr, pitch_bytes, fmt))
